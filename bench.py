@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]                  this repo's B200 path
     python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]  the reference's CPU arithmetic (oracle port)
+    python bench.py ... --dump-outputs DIR                               also write the last timed step's results to DIR
 
 One "step" = one `sess.run([loss, global_step, train_op])` of the reference (model_combine.py:231-234): forward,
 losses, gradients, per-tensor clip and Adam over one length-bucketed batch of 512 sessions against the full
@@ -64,7 +65,14 @@ def parse():
     ap.add_argument("--profile_region", action="store_true",
                     help="for `ncu --profile-from-start off`: warm up, then ONE train step (T=20) and ONE eval step "
                          "between cudaProfilerStart/Stop; prints nothing")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed loops, write DIR/<name>.npy (float32 / float64): the loss and the updated "
+                         "parameters (dense tensors, a fixed sample of item rows) of the last timed train step, the "
+                         "top-20 ids, ranks and cross loss of the last timed eval step.  The inputs depend only on the "
+                         "arguments, so two builds can be compared output for output")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the results of the B200 path")
     if a.items <= 0:
         a.items = SHAPE[a.workload][1]
     if a.workload == "mind":
@@ -263,6 +271,42 @@ def workload_config(a, world):
 
 
 # ----------------------------------------------------------------------------------------------------- B200 arm
+DUMP_ITEM_ROWS = 4096      # item-table rows in the dump: a fixed sample keeps it at 4 MB instead of the 364 MB table
+DUMP_MAX_BYTES = 64 << 20
+
+
+def train_outputs(model, loss):
+    """What a caller of train_step holds after its last call, on the host: the returned per-session loss and the
+    updated parameters (every dense tensor, and the item-table rows of a fixed seeded sample with their ids)."""
+    import numpy as np
+    import torch
+    from tcar_b200.params import H
+    ps = model.ps
+    rows = np.sort(np.random.RandomState(7).choice(ps.N + 1, min(DUMP_ITEM_ROWS, ps.N + 1), replace=False))
+    out = {"train_loss": loss.float().cpu().numpy(), "item_row_ids": rows.astype(np.float64),
+           "item_rows": ps.item.index_select(0, torch.from_numpy(rows).to(ps.item.device))[:, :H].cpu().numpy()}
+    for name, t in ps.w.items():
+        out["param_" + name] = t.cpu().numpy()
+    return out
+
+
+def eval_outputs(top, ngt, ce):
+    """What eval_step / eval_round returned, on the host; the integer results as float64 (exact)."""
+    import numpy as np
+    return {"eval_top20_ids": top.cpu().numpy().astype(np.float64),
+            "eval_n_greater": ngt.cpu().numpy().astype(np.float64), "eval_cross_loss": ce.float().cpu().numpy()}
+
+
+def dump_outputs(path, arrays):
+    """DIR/<name>.npy per array, float32 or float64 only, at most DUMP_MAX_BYTES in all."""
+    import numpy as np
+    assert all(v.dtype in (np.float32, np.float64) for v in arrays.values())
+    assert sum(v.nbytes for v in arrays.values()) <= DUMP_MAX_BYTES
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), v)
+
+
 def time_kernel(torch, fn, iters, flush):
     """Average CUDA-event duration (ms) of fn() over `iters` launches on the current stream; `flush` (a >L2 buffer)
     is rewritten before every launch, outside the event pair."""
@@ -532,7 +576,7 @@ def run_b200(a):
     e0.record()
     marks = []
     for i in range(W, W + K):
-        model.train_step(dev[i % nbatch], nxt(dev, i))
+        loss_dev = model.train_step(dev[i % nbatch], nxt(dev, i))
         ev = torch.cuda.Event(enable_timing=True)      # per-step marks on the launching stream: spread of the K steps
         ev.record()
         marks.append(ev)
@@ -547,6 +591,11 @@ def run_b200(a):
                    "first_ms": [round(x, 3) for x in seq_ms[:12]], "last_ms": [round(x, 3) for x in seq_ms[-6:]],
                    "note": "rank 0, time between consecutive steps' last launches on the main stream"}
     loss_last = float(model.loss[:B].mean().item())
+    outputs = {}
+    if a.dump_outputs:
+        model.sync_item_table()    # catalog layout: rank 0 holds only its own item rows until this collective
+        if rank == 0:
+            outputs.update(train_outputs(model, loss_dev))
 
     # ---- end to end through the public API: pinned host batch -> H2D -> train_step -> D2H of the loss -------
     def e2e_loop(hosts, lens, n):
@@ -685,11 +734,13 @@ def run_b200(a):
     barrier()
     e0.record()
     for i in range(W, W + K):
-        estep(edev[i % nbatch], enxt(i))
+        eres = estep(edev[i % nbatch], enxt(i))
     model.sync_updates()
     e1.record()
     barrier()
     eval_ms = max_over_ranks(e0.elapsed_time(e1))
+    if a.dump_outputs and rank == 0:
+        outputs.update(eval_outputs(*eres))
     # share of the queries the certified selection handed to the widening pass, averaged over the batches
     unc = []
     for b_ in edev:
@@ -842,6 +893,8 @@ def run_b200(a):
         if dist is not None:
             dist.destroy_process_group()
         return
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, outputs)
     sessions = world * B * K
     value = sessions / (train_ms * 1e-3)
     # dominant kernel of the step = largest share of the isolated kernel times
