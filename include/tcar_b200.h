@@ -528,6 +528,23 @@ int tcar_eval_ce_combine(const float* sumexp, const float* rowmax, long long gst
 int tcar_eval_merge_flagged(const void* blocks, long long block_words, const int32_t* only_if, int32_t* out_ids,
                             float* out_scores, int32_t* out_ngt, int G, int B, void* stream);
 
+/* (6b) candidate re-ranking: session b's list is cand_ids[cand_off[b] .. cand_off[b+1]) (0-based item ids, at most
+ *      max_len <= TCAR_RERANK_MAXL entries; duplicates allowed).  a_ic / Tq are the session vectors of
+ *      tcar_build_query; item / content / mwdhm the fp32 tables of the full-catalog evaluation.
+ *        scores [nnz]   exact fp32 score of cand_ids[j], in input order: the arithmetic of tcar_eval_topk's re-scoring,
+ *                       so a candidate scores bit for bit what the full-catalog top-20 reports for it
+ *                       (model_combine.py:138);
+ *        ranked [nnz]   each list's ids ordered by (score desc, id asc, input position asc);
+ *      with label != NULL (label[b] = the positive, every other entry of the list is a negative):
+ *        label_rank [B] 1 + #(negatives scoring strictly above the label): the label wins ties (util.py:14);
+ *        auc [B]        (#(negatives below) + 1/2 #(negatives equal)) / #negatives, NaN without negatives.
+ *      An id outside [0, N) is not read and scores NaN; a label outside [0, N) gives label_rank 0 and auc NaN; a list
+ *      longer than max_len is not processed (outputs left as they are).  B = 0 launches nothing. */
+#define TCAR_RERANK_MAXL 2048
+int tcar_rerank(const float* a_ic, const float* Tq, const float* item, const float* content, const int32_t* mwdhm,
+                const int32_t* cand_off, const int32_t* cand_ids, const int32_t* label, int B, int N, int max_len,
+                float* scores, int32_t* ranked, int32_t* label_rank, float* auc, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

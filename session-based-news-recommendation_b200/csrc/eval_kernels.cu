@@ -945,6 +945,106 @@ topk_merge_kernel(const int32_t* ids, const float* scores, int32_t* out_ids, flo
     warp_merge_lists(ids, scores, G, B, gstride, b, lane, out_ids, out_scores);
 }
 
+// ------------------------------------------------------------------------------------------------ candidate re-ranking
+// One CTA per session.  Warp w scores the list entries w, w + 8, w + 16, w + 24, then the next 32, with exact_score_e
+// (the re-scoring arithmetic of the full-catalog top-20): four candidates per warp and iteration, branch-free, so that
+// a lane's 16 row loads are in flight before the first dot product, as in the widening pass.  Every candidate row is
+// used once per session, so this is a gather plus a GEMV: no tensor cores.  The order is found by counting -- entry i
+// goes to position #{j : key_j < key_i, or key_j == key_i and j < i} -- with no sort network and no atomics, so
+// repeated runs are bit-identical.
+constexpr int RMAXL = TCAR_RERANK_MAXL;
+
+// ascending key = (score desc, id asc).  +0 and -0 are equal scores and share a key; NaN gets a place in the order
+// (fkey is total on bit patterns), so the positions always form a permutation.
+__device__ __forceinline__ unsigned long long rerank_key(float s, int id) {
+    const uint32_t k = fkey(s == 0.f ? 0.f : s);
+    return ((unsigned long long)(~k) << 32) | (uint32_t)id;
+}
+
+__global__ void __launch_bounds__(256)
+rerank_kernel(const float* __restrict__ a_ic, const float* __restrict__ Tq, const float* __restrict__ item,
+              const float* __restrict__ content, const int32_t* __restrict__ mwdhm,
+              const int32_t* __restrict__ cand_off, const int32_t* __restrict__ cand_ids,
+              const int32_t* __restrict__ label, int N, int max_len, float* __restrict__ scores,
+              int32_t* __restrict__ ranked, int32_t* __restrict__ label_rank, float* __restrict__ auc) {
+    PDL_ENTER();
+    __shared__ float s_aic[XW], s_tq[NB + 1];
+    __shared__ float s_sc[RMAXL];
+    __shared__ unsigned long long s_key[RMAXL];
+    __shared__ float s_lab;
+    __shared__ int s_cnt[3][8];
+    const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    const int off = cand_off[b], L = cand_off[b + 1] - off;
+    if (L < 0 || L > max_len) return;               // block-uniform; the shared arrays hold max_len entries
+    for (int c = tid; c < XW; c += 256) s_aic[c] = a_ic[(size_t)b * XW + c];
+    for (int c = tid; c < NB; c += 256) s_tq[c] = Tq[(size_t)b * NB + c];
+    __syncthreads();
+    const int lab = label ? label[b] : -1;
+    const bool lab_ok = lab >= 0 && lab < N;
+    if (label && w == 0) {
+        const float ls = exact_score_e(s_aic, s_tq, item, content, mwdhm, lab_ok ? lab : 0, lane);
+        if (lane == 0) s_lab = lab_ok ? ls : NAN;
+    }
+    const int32_t* ids = cand_ids + off;
+    for (int c0 = w; c0 < L; c0 += 32) {
+        int raw[4];
+        bool ok[4];
+        float sc[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int c = c0 + 8 * u;
+            raw[u] = c < L ? ids[c] : -1;
+            ok[u] = raw[u] >= 0 && raw[u] < N;
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) sc[u] = exact_score_e(s_aic, s_tq, item, content, mwdhm, ok[u] ? raw[u] : 0, lane);
+        if (lane == 0) {
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const int c = c0 + 8 * u;
+                if (c < L) {
+                    const float s = ok[u] ? sc[u] : NAN;
+                    s_sc[c] = s;
+                    s_key[c] = rerank_key(s, raw[u]);
+                    scores[off + c] = s;
+                }
+            }
+        }
+    }
+    __syncthreads();
+    const float sl = label ? s_lab : 0.f;
+    int gt = 0, eq = 0, nneg = 0;
+    for (int i = tid; i < L; i += 256) {
+        const unsigned long long ki = s_key[i];
+        int pos = 0;
+#pragma unroll 4
+        for (int j = 0; j < L; ++j) {               // every lane reads the same s_key[j]: a broadcast
+            const unsigned long long kj = s_key[j];
+            pos += (kj < ki) | ((kj == ki) & (j < i));
+        }
+        const int id = (int)(uint32_t)ki;
+        ranked[off + pos] = id;
+        if (label && id != lab) {
+            const float s = s_sc[i];
+            ++nneg;
+            gt += s > sl;
+            eq += s == sl;
+        }
+    }
+    if (!label) return;
+    gt = __reduce_add_sync(0xffffffffu, gt);
+    eq = __reduce_add_sync(0xffffffffu, eq);
+    nneg = __reduce_add_sync(0xffffffffu, nneg);
+    if (lane == 0) { s_cnt[0][w] = gt; s_cnt[1][w] = eq; s_cnt[2][w] = nneg; }
+    __syncthreads();
+    if (tid == 0) {
+        int g = 0, e = 0, n = 0;
+        for (int k = 0; k < 8; ++k) { g += s_cnt[0][k]; e += s_cnt[1][k]; n += s_cnt[2][k]; }
+        label_rank[b] = lab_ok ? 1 + g : 0;                                               // util.py:14
+        auc[b] = lab_ok && n > 0 ? ((float)(n - g - e) + 0.5f * (float)e) / (float)n : NAN;
+    }
+}
+
 }  // namespace tcar
 
 using namespace tcar;
@@ -1143,6 +1243,19 @@ extern "C" int tcar_eval_merge_flagged(const void* blocks, long long block_words
     launch_pdl(topk_merge_kernel, dim3((B + 7) / 8), dim3(256), 0, STREAM, i + TCAR_EVAL_OFF_IDS, f + TCAR_EVAL_OFF_SCORES,
                out_ids, out_scores, G, B, block_words, i + TCAR_EVAL_OFF_NGT, static_cast<const float*>(nullptr),
                static_cast<const float*>(nullptr), out_ngt, static_cast<float*>(nullptr), only_if, WidenGroups{});
+    return (int)cudaGetLastError();
+}
+
+extern "C" int tcar_rerank(const float* a_ic, const float* Tq, const float* item, const float* content,
+                           const int32_t* mwdhm, const int32_t* cand_off, const int32_t* cand_ids, const int32_t* label,
+                           int B, int N, int max_len, float* scores, int32_t* ranked, int32_t* label_rank, float* auc,
+                           void* stream) {
+    if (B < 0 || B > TCAR_QROWS || N <= 0 || max_len < 0 || max_len > TCAR_RERANK_MAXL || !a_ic || !Tq || !item ||
+        !content || !mwdhm || !cand_off || (label && (!label_rank || !auc)))
+        return TCAR_ERR_ARG;
+    if (B == 0) return 0;
+    launch_pdl(rerank_kernel, dim3(B), dim3(256), 0, STREAM, a_ic, Tq, item, content, mwdhm, cand_off, cand_ids, label,
+               N, max_len, scores, ranked, label_rank, auc);
     return (int)cudaGetLastError();
 }
 

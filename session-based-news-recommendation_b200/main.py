@@ -60,6 +60,8 @@ def main(args):
         print("Begin Testing. Test data is %s data" % ("train" if input_data == "train" else "test"))
         restore_model(model, model_path)
         model.test(None, sent_data, args)
+    if args.get("impression_eval"):
+        model.test_impressions(None, test_data if is_train else sent_data, neighbor, item_dict, args)
     return model
 
 
@@ -103,6 +105,9 @@ def build_parser():
     # not a reference flag: the reference ships uniform negatives (sampler.py:98-99) and keeps the impression-list
     # sampler of the MIND experiments commented out (sampler.py:96,118-131); this switch selects it
     parser.add_argument("--negative_mode", default="uniform", choices=["uniform", "impression"], type=str)
+    # not a reference flag: after training / testing, also rank every session's impression list (the MIND protocol:
+    # AUC, MRR, nDCG@5, nDCG@10; Seq2SeqAttNN.test_impressions) with the impression file as the neighbour dict
+    parser.add_argument("--impression_eval", action="store_true")
     parser.add_argument("--inputdata", default="test", type=str)
     parser.add_argument("--threshold_acc", default=0.27, type=float)
     # additions

@@ -313,12 +313,17 @@ class Seq2SeqAttNN(CatalogShardedTraining):
 
     def stage_to_device(self, packed_np, B, T, Nn):
         """NumPy packed batch -> pinned ring slot -> device (the path of the train / test loops)."""
+        return Batch(self._stage_ints(packed_np), B, T, Nn)
+
+    def _stage_ints(self, arr_np):
+        """int32 NumPy array -> pinned ring slot -> new device tensor, without blocking the host."""
         if getattr(self, "_ring", None) is None:
             self._ring = PinnedRing()
-        view, ev = self._ring.stage(packed_np)
-        bt = self.to_device(view, B, T, Nn)
+        view, ev = self._ring.stage(arr_np)
+        buf = torch.empty(view.numel(), device=self.dev, dtype=torch.int32)
+        buf.copy_(view, non_blocking=True)
         ev.record()
-        return bt
+        return buf
 
     def fetch_async(self, t):
         """Start the device -> host copy of a result tensor into pinned memory; returns a handle whose .get() blocks
@@ -1264,6 +1269,100 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         [B,N] fp32 scores from the same bf16 operands with a library GEMM.  Not used on the hot path."""
         self._session_forward(bt)
         return self.Q[:bt.B].float() @ self.ps.iext[: self.ps.N].float().t()
+
+    # ------------------------------------------------------------------------------------------- candidate re-ranking
+    def rerank(self, bt, cand_off, cand_ids, metrics=True):
+        """Rank a given candidate list per session (tcar_rerank).  Session b's candidates are
+        cand_ids[cand_off[b]:cand_off[b + 1]]: 0-based item ids in host arrays (NumPy, lists or CPU tensors), duplicates
+        allowed, at most nv.RERANK_MAXL per session; cand_off has B + 1 entries from 0 to len(cand_ids).  The scores are
+        the exact fp32 scores of the full-catalog evaluation (bit for bit what eval_step reports for the same item), not
+        the bf16 products of softmax_input().
+
+        Returns device tensors (scores [nnz] in input order, ranked [nnz] = every list's ids ordered by (score desc,
+        id asc), label_rank [B], auc [B]).  bt.label is read for the metrics only: it is the positive of its session's
+        list and every other entry a negative; label_rank = 1 + #negatives scoring above it (the label wins ties),
+        auc counts a tied negative as 1/2 and is NaN for a list without negatives.  metrics=False returns None for
+        the last two, so a serving caller may fill bt.label with any valid item id."""
+        # validated in the callers' own integer type (min / max first: no int64 copy of a long list)
+        off, ids = np.asarray(cand_off).reshape(-1), np.asarray(cand_ids).reshape(-1)
+        if off.dtype.kind not in "iu" or (ids.size and ids.dtype.kind not in "iu"):
+            raise ValueError("cand_off and cand_ids must hold integers")
+        B, N = bt.B, self.N
+        if off.shape[0] != B + 1 or off[0] != 0 or off[-1] != ids.shape[0]:
+            raise ValueError(f"cand_off must hold B + 1 = {B + 1} offsets from 0 to len(cand_ids) = {ids.shape[0]}")
+        lens = np.diff(off.astype(np.int64))
+        for bad, what in ((lens < 0, "cand_off decreases"),
+                          (lens > nv.RERANK_MAXL, f"more than TCAR_RERANK_MAXL = {nv.RERANK_MAXL} candidates")):
+            if bad.any():
+                raise ValueError(f"session {int(np.argmax(bad))}: {what}")
+        if ids.size and (ids.min() < 0 or ids.max() >= N):
+            j = int(np.argmax((ids < 0) | (ids >= N)))
+            s = int(np.searchsorted(off, j, side="right")) - 1
+            raise ValueError(f"session {s}: candidate id {int(ids[j])} outside [0, {N})")
+        dev, p, ps = self.dev, nv.ptr, self.ps
+        scores = torch.empty(ids.shape[0], device=dev)
+        ranked = torch.empty(ids.shape[0], device=dev, dtype=torch.int32)
+        label_rank = torch.empty(B, device=dev, dtype=torch.int32) if metrics else None
+        auc = torch.empty(B, device=dev) if metrics else None
+        if B == 0:
+            return scores, ranked, label_rank, auc
+        if not self._item_table_synced:
+            self.sync_item_table()         # after catalog-sharded training every rank holds only its own rows
+        self._session_forward(bt)
+        host = np.empty(B + 1 + ids.shape[0], dtype=np.int32)
+        host[:B + 1], host[B + 1:] = off, ids
+        csr = self._stage_ints(host)
+        nv.counted_call("tcar_rerank", 1, p(self.a_ic), p(self.Tq), p(ps.item), p(ps.content), p(ps.mwdhm), p(csr),
+                        p(csr[B + 1:]), p(bt.label) if metrics else None, B, N, int(lens.max()), p(scores), p(ranked),
+                        p(label_rank), p(auc))
+        return scores, ranked, label_rank, auc
+
+    def test_impressions(self, sess, test_data, impressions, item_dict, args):
+        """Rank every session's impression list (the MIND protocol): the clicked article (the label) is the positive,
+        the listed articles known to item_dict the negatives (sampler.impression_candidates).  Prints and returns
+        {"auc", "mrr", "ndcg5", "ndcg10", "sessions", "skipped"}: averages over the sessions with at least one
+        negative (util.impression_sums); `skipped` counts the others.  Walks the split in the batches test() uses.
+        Under torchrun batch i goes to rank i mod world and the sums are all-reduced, so every rank returns the
+        metrics of the whole split."""
+        from .sampler import impression_candidates
+        from .util import impression_metrics, impression_sums
+        print("Ranking impression lists...")
+        self.sync_item_table()
+        (len_dict_test, session_dict_test, session_time_dict_test) = test_data
+        sampler = Sampler(len_dict_test, session_dict_test, session_time_dict_test, batch_size=self.batch_size)
+        # every batch's lists up front, so that the producer thread does no dictionary work per batch
+        cands = [impression_candidates(keys, [session_dict_test[k][-1] - 1 for k in keys], impressions, item_dict)
+                 for keys in sampler.session_id_batches]
+        dist_on = parallel.is_distributed(self.world)
+        if dist_on:
+            sampler.session_id_batches = sampler.session_id_batches[self.rank::self.world]
+            sampler.batch_num = len(sampler.session_id_batches)
+            cands = cands[self.rank::self.world]
+        sums = np.zeros(6)
+        # one batch of look-ahead (as in test()): batch i+1 is staged before batch i is ranked, and batch i's results
+        # are read from pinned memory while batch i+1 runs
+        it = zip((self.stage_to_device(packed, B, T, Nn) for packed, B, T, Nn in prefetch_packed(sampler)), cands)
+        cur, pending = next(it, None), None
+        while cur is not None:
+            nxt = next(it, None)
+            bt, (off, ids) = cur
+            _, _, rank, auc = self.rerank(bt, off, ids)
+            handles = (np.diff(off) - 1, self.fetch_async(rank), self.fetch_async(auc))
+            if pending is not None:
+                sums += impression_sums(pending[1].get().numpy(), pending[2].get().numpy(), pending[0])
+            pending, cur = handles, nxt
+        if pending is not None:
+            sums += impression_sums(pending[1].get().numpy(), pending[2].get().numpy(), pending[0])
+        if dist_on:
+            import torch.distributed as dist
+            t = torch.from_numpy(sums).to(self.dev)
+            dist.all_reduce(t, op=dist.ReduceOp.SUM)
+            sums = t.cpu().numpy()
+        m = impression_metrics(sums)
+        self.last_impression_metrics = m
+        print("Impressions: AUC: {}, MRR: {}, nDCG@5: {}, nDCG@10: {} ({} sessions, {} without a negative skipped)".format(
+            m["auc"], m["mrr"], m["ndcg5"], m["ndcg10"], m["sessions"], m["skipped"]))
+        return m
 
     # ------------------------------------------------------------------------------------------- metrics
     def _categories(self):

@@ -239,6 +239,27 @@ class Sampler(object):
         return neg
 
 
+def impression_candidates(keys, labels, impressions, item_dict):
+    """Candidate lists of a batch for ranking each session's impression list (the MIND protocol): session key k's list
+    is impressions[int(str(k).split("_")[0])] (the key rule of the impression negatives), its article ids mapped
+    through item_dict to 0-based ids.  Articles outside item_dict are dropped (the impression logs name more articles
+    than the clicked-item dictionary, mind_preprocess.py:275-280), repeats keep their first occurrence, and the label
+    is appended when absent, so every list holds it exactly once; a session without a list gets [label].
+    Returns (off int32 [B+1], ids int32 [nnz]) in CSR form."""
+    off = np.zeros(len(keys) + 1, dtype=np.int32)
+    ids = []
+    for b, (key, lab) in enumerate(zip(keys, labels)):
+        seen = {}
+        for art in impressions.get(int(str(key).split("_")[0]), ()):
+            i = item_dict.get(art)
+            if i is not None:
+                seen.setdefault(i - 1, None)
+        seen.setdefault(int(lab), None)
+        ids.extend(seen)
+        off[b + 1] = len(ids)
+    return off, np.asarray(ids, dtype=np.int32)
+
+
 def pack_batch(batch_in, batch_out, batch_pt, batch_ct, neg, gap):
     """Reference 6-tuple of lists -> (int32 array, B, T, Nn) in the model_combine.Batch layout."""
     B, T = len(batch_in), len(batch_in[0])

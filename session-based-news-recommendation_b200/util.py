@@ -20,6 +20,32 @@ def cau_metrics(preds, labels, cutoff=20):
     return recall, mrr, ndcg
 
 
+IMPRESSION_SUMS = ("auc", "mrr", "ndcg5", "ndcg10", "sessions", "skipped")
+
+
+def impression_sums(rank, auc, n_neg):
+    """Per-session results of ranking impression lists (one positive each: rank = 1 + #negatives scoring above it,
+    auc, n_neg = #negatives) -> float64 [6]: the sums of AUC, MRR = 1/rank (not truncated), nDCG@5 and nDCG@10
+    (1/log2(1 + rank) when rank <= k, else 0) over the sessions with at least one negative, their number, and the
+    number of sessions without a negative.  Sums add up across batches and ranks; impression_metrics averages them."""
+    rank = np.asarray(rank, dtype=np.float64)
+    auc = np.asarray(auc, dtype=np.float64)
+    used = np.asarray(n_neg) > 0
+    r, a = rank[used], auc[used]
+    gain = 1.0 / np.log2(1.0 + r)
+    return np.array([a.sum(), (1.0 / r).sum(), np.where(r <= 5, gain, 0.0).sum(), np.where(r <= 10, gain, 0.0).sum(),
+                     used.sum(), (~used).sum()], dtype=np.float64)
+
+
+def impression_metrics(sums):
+    """impression_sums (possibly added up) -> {"auc", "mrr", "ndcg5", "ndcg10", "sessions", "skipped"}."""
+    s = np.asarray(sums, dtype=np.float64)
+    n = s[4]
+    out = {k: float(s[i] / n) if n > 0 else float("nan") for i, k in enumerate(IMPRESSION_SUMS[:4])}
+    out["sessions"], out["skipped"] = int(s[4]), int(s[5])
+    return out
+
+
 def _load(path):
     with open(path, "rb") as f:
         return pickle.load(f)
