@@ -545,6 +545,28 @@ int tcar_rerank(const float* a_ic, const float* Tq, const float* item, const flo
                 const int32_t* cand_off, const int32_t* cand_ids, const int32_t* label, int B, int N, int max_len,
                 float* scores, int32_t* ranked, int32_t* label_rank, float* auc, void* stream);
 
+/* (6c) top-K recommendation: the exact top-K of the whole catalog per session, without the excluded ids.
+ *      chunkmax / tilemax: the eval-mode scoring GEMM (tcar_score_fwd mode 1) over the N items for these B queries;
+ *      a_ic / Tq / item / content / mwdhm as for tcar_eval_topk; cat_stats: tcar_catalog_stats over the N items.
+ *      Exclusions of session b (0-based ids; duplicates and ids outside [0, N) allowed): x_ids[x_off[b] .. x_off[b+1])
+ *      when x_off != NULL, and clicks[b*T .. b*T+T) - 1 when clicks != NULL (the 1-based click ids of the packed
+ *      batch, T clicks per session); at most TCAR_RECOMMEND_MAXX entries in all, a session with more is not processed
+ *      (outputs left as they are).
+ *        ids [B][K]       item ids ordered by (exact score desc, id asc); -1 past the end of a small catalog
+ *        scores [B][K]    their exact fp32 scores (the arithmetic of tcar_eval_topk's re-scoring, so bit for bit what
+ *                         eval_step and tcar_rerank report for the same item); -inf past the end
+ *        rescored [B]     (nullable) items re-scored exactly: the width of the band the error bound left open.
+ *      1 <= K <= TCAR_RECOMMEND_MAXK.  workspace: tcar_recommend_ws_bytes(B) bytes (a buffer sized for B serves every
+ *      smaller B), ZERO before the first call (it starts with TCAR_QROWS ticket counters that every call leaves at
+ *      zero again).  Two launches; B = 0 launches nothing. */
+#define TCAR_RECOMMEND_MAXK 256
+#define TCAR_RECOMMEND_MAXX 1024
+long long tcar_recommend_ws_bytes(int B);
+int tcar_recommend(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq, const float* item,
+                   const float* content, const int32_t* mwdhm, const float* cat_stats, const int32_t* x_off,
+                   const int32_t* x_ids, const int32_t* clicks, int T, int B, int N, int n_pad, int K, void* workspace,
+                   int32_t* ids, float* scores, int32_t* rescored, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

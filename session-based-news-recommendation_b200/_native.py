@@ -22,6 +22,8 @@ MAX_PEERS, PEER_HANDLE_BYTES = 16, 64      # TCAR_MAX_PEERS, TCAR_PEER_HANDLE_BY
 BIN_OFF = (0, 13, 45, 53, 78, 139)
 CLUSTER_PAIR = -2      # TCAR_CLUSTER_PAIR: tcar_score_fwd with tcgen05.mma.cta_group::2 CTA pairs
 RERANK_MAXL = 2048     # TCAR_RERANK_MAXL: longest candidate list of tcar_rerank
+RECOMMEND_MAXK = 256   # TCAR_RECOMMEND_MAXK: largest K of tcar_recommend
+RECOMMEND_MAXX = 1024  # TCAR_RECOMMEND_MAXX: exclusion entries per session of tcar_recommend, clicks included
 
 _P, _I, _F, _LL = C.c_void_p, C.c_int, C.c_float, C.c_longlong
 
@@ -102,6 +104,8 @@ SIGNATURES = {
     "tcar_eval_ce_combine": [_P, _P, _LL, _P, _I, _I, _P],
     "tcar_eval_merge_flagged": [_P, _LL, _P, _P, _P, _P, _I, _I, _P],
     "tcar_rerank": [_P] * 8 + [_I] * 3 + [_P] * 4 + [_P],
+    "tcar_recommend_ws_bytes": [_I],
+    "tcar_recommend": [_P] * 11 + [_I] * 5 + [_P] * 4 + [_P],
 }
 
 _lib = None

@@ -1045,6 +1045,309 @@ rerank_kernel(const float* __restrict__ a_ic, const float* __restrict__ Tq, cons
     }
 }
 
+// ------------------------------------------------------------------------------------------------ top-K recommendation
+// The exact top-K of the whole catalog per session, K <= 256, with up to 1024 excluded ids per session, in two launches
+// behind the eval-mode scoring GEMM (chunk / tile maxima of the bf16 scores):
+//   select  one CTA per query: K' = K + x_b (x_b = the session's exclusion entries, duplicates counted),
+//           tau_hi = the K'-th largest chunk maximum, tau_b = tau_hi - 2 eps_b (eps_b = score_error_bound);
+//           tau_b = -inf (a full exact scan) when K' >= the number of chunks.
+//   scan    TCAR_WIDEN_SPLITS CTAs per query over contiguous tile ranges: tiles whose maximum is below tau_b are
+//           skipped, chunks whose maximum reaches tau_b are re-scored exactly (exact_score_e) except for excluded
+//           ids (sorted list in shared memory, tested before the row loads) and ids >= N, and merged into a running
+//           top-K; the split CTA that finishes last (ticket counter) merges the partial lists.
+// Why the result is exact: the K' chunks with the largest maxima hold K' distinct valid items (chunk maxima mask items
+// >= N to -inf) whose bf16 scores are >= tau_hi.  At most x_b of them are excluded, so at least K eligible items score
+// >= tau_hi - eps_b exactly, i.e. the exact K-th best eligible score s_K >= tau_hi - eps_b.  Every member of the exact
+// top-K (ties included) scores >= s_K exactly, so its bf16 score is >= s_K - eps_b >= tau_b: its chunk is re-scored.
+// The order is the total order of rerank_key (score desc, id asc) and every item is re-scored by exactly one CTA, so
+// the order in which chunks are queued (shared-memory atomics) cannot change the result: reruns are bit-identical.
+constexpr int RK = TCAR_RECOMMEND_MAXK;
+constexpr int RX = TCAR_RECOMMEND_MAXX;
+constexpr int TL_CAP = 4096;                     // tiles listed for the chunk-level selection (more: scan every tile)
+constexpr unsigned long long KEY_NONE = ~0ull;   // empty slot: after every real key
+
+__device__ __forceinline__ float key_value(uint32_t k) {                     // inverse of fkey
+    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
+// fkey of the k-th largest of get(0 .. n) (1 <= k <= n) by four 8-bit radix passes.  256 threads, s_hist [256],
+// s_misc [2].  The values of one query sit in a narrow range, so lanes with equal bins are combined (match_any) before
+// the shared-memory atomic.
+template <class Get>
+__device__ __forceinline__ uint32_t block_kth_key(int n, int k, Get get, int* s_hist, int* s_misc) {
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    uint32_t prefix = 0, mask = 0;
+    for (int shift = 24; shift >= 0; shift -= 8) {
+        s_hist[tid] = 0;
+        __syncthreads();
+        for (int i0 = 0; i0 < n; i0 += 256) {                         // block-uniform trip count (match_any below)
+            const int i = i0 + tid;
+            const uint32_t key = i < n ? fkey(get(i)) : 0u;
+            const bool act = i < n && (key & mask) == prefix;
+            const uint32_t bin = act ? ((key >> shift) & 255u) : 256u;
+            const uint32_t peers = __match_any_sync(0xffffffffu, bin);
+            if (act && lane == __ffs(peers) - 1) atomicAdd(&s_hist[bin], __popc(peers));
+        }
+        __syncthreads();
+        if (w == 0) {                                                 // lane l owns bins 8l .. 8l+7
+            int cnt[8], tot = 0;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) { cnt[j] = s_hist[lane * 8 + j]; tot += cnt[j]; }
+            int suf = tot;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int v = __shfl_down_sync(0xffffffffu, suf, o);
+                if (lane + o < 32) suf += v;
+            }
+            const int above_lane = suf - tot;
+            const bool mine = above_lane < k && k <= suf;
+            if (mine) {
+                int a = above_lane;
+                for (int j = 7; j >= 0; --j) {
+                    if (a + cnt[j] >= k) { s_misc[0] = lane * 8 + j; s_misc[1] = a; break; }
+                    a += cnt[j];
+                }
+            }
+        }
+        __syncthreads();
+        prefix |= (uint32_t)s_misc[0] << shift;
+        mask |= 255u << shift;
+        k -= s_misc[1];
+    }
+    __syncthreads();
+    return prefix;
+}
+
+__global__ void __launch_bounds__(256)
+recommend_select_kernel(const float* chunkmax, const float* tilemax, const float* __restrict__ a_ic,
+                        const float* __restrict__ Tq, const float* __restrict__ cat_stats,
+                        const int32_t* __restrict__ x_off, int n_clicks, int K, int N, int n_pad,
+                        float* __restrict__ tau) {
+    PDL_ENTER();
+    __shared__ float s_aic[XW], s_tq[NB + 1];
+    __shared__ float s_red[32];
+    __shared__ int s_hist[256], s_misc[2];
+    __shared__ int s_tl[TL_CAP];
+    __shared__ int s_ntl;
+    const int b = blockIdx.x, tid = threadIdx.x;
+    const int nchunks = (N + CH - 1) / CH, ntiles = (N + 127) / 128;
+    const int kp = K + (x_off ? x_off[b + 1] - x_off[b] : 0) + n_clicks;
+    if (kp >= nchunks) {                                              // block-uniform
+        if (tid == 0) tau[b] = -INFINITY;
+        return;
+    }
+    const float* cm = chunkmax + (size_t)b * (n_pad / CH);
+    const float* tm = tilemax + (size_t)b * (n_pad / 128);
+    for (int c = tid; c < XW; c += 256) s_aic[c] = a_ic[(size_t)b * XW + c];
+    for (int c = tid; c < NB; c += 256) s_tq[c] = Tq[(size_t)b * NB + c];
+    if (tid == 0) s_ntl = 0;
+    __syncthreads();
+    // The K' largest tile maxima are K' distinct chunk values, so the K'-th largest chunk is >= the K'-th largest tile
+    // maximum: tiles below it cannot hold one of the K' best chunks.
+    float thr = -INFINITY;
+    if (ntiles > kp) thr = key_value(block_kth_key(ntiles, kp, [&](int i) { return tm[i]; }, s_hist, s_misc));
+    for (int i = tid; i < ntiles; i += 256)
+        if (tm[i] >= thr) {
+            const int at = atomicAdd(&s_ntl, 1);
+            if (at < TL_CAP) s_tl[at] = i;
+        }
+    __syncthreads();
+    const bool listed = s_ntl <= TL_CAP;                              // else ties: every tile
+    const int n = (listed ? s_ntl : ntiles) * TILE_CH;
+    const uint32_t kk = block_kth_key(n, kp, [&](int i) {
+        const int c = (listed ? s_tl[i / TILE_CH] : i / TILE_CH) * TILE_CH + i % TILE_CH;
+        return c < nchunks ? cm[c] : -INFINITY;
+    }, s_hist, s_misc);
+    const float eps = score_error_bound(s_aic, s_tq, cat_stats, s_red);
+    if (tid == 0) tau[b] = key_value(kk) - 2.f * eps;
+}
+
+// number of entries of a sorted list below x
+__device__ __forceinline__ int rank_in(const unsigned long long* a, int n, unsigned long long x) {
+    int lo = 0, hi = n;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (a[mid] < x) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+// out[0 .. K) = the K smallest keys of the ascending lists a[0 .. K) and c[0 .. nc), by merge path: an entry's place is
+// its index plus its rank in the other list (real keys are distinct; KEY_NONE slots write KEY_NONE wherever they
+// collide).  Ends with a barrier.
+__device__ __forceinline__ void merge_topk(const unsigned long long* a, int K, const unsigned long long* c, int nc,
+                                           unsigned long long* out) {
+    for (int i = threadIdx.x; i < K; i += 256) {
+        const unsigned long long v = a[i];
+        const int pos = i + rank_in(c, nc, v);
+        if (pos < K) out[pos] = v;
+    }
+    for (int j = threadIdx.x; j < nc && j < K; j += 256) {
+        const unsigned long long v = c[j];
+        const int pos = j + rank_in(a, K, v);
+        if (pos < K) out[pos] = v;
+    }
+    __syncthreads();
+}
+
+// workspace: tickets [512] (zero between calls; at fixed places, whatever B a call has) | tau [B] |
+// re-scored counts [S][B] | partial lists [S][B][256] keys
+__host__ __device__ constexpr size_t rec_keys_offset(int B) {
+    return ((size_t)(TCAR_QROWS + (1 + WSPLIT) * B) * 4 + 7) / 8 * 8;
+}
+
+__global__ void __launch_bounds__(256, 2)
+recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* __restrict__ a_ic,
+                      const float* __restrict__ Tq, const float* __restrict__ item, const float* __restrict__ content,
+                      const int32_t* __restrict__ mwdhm, const int32_t* __restrict__ x_off,
+                      const int32_t* __restrict__ x_ids, const int32_t* __restrict__ clicks, int n_clicks, int K, int N,
+                      int n_pad, int B, char* wspace, int32_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                      int32_t* __restrict__ rescored) {
+    PDL_ENTER();
+    __shared__ float s_aic[XW], s_tq[NB + 1];
+    __shared__ int s_x[RX];
+    __shared__ int s_q[WQ_CAP];
+    __shared__ unsigned long long s_top[2][RK];
+    __shared__ unsigned long long s_new[NCAND];
+    __shared__ int s_qn, s_cnt, s_last;
+    const int b = blockIdx.x, split = blockIdx.y, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    int32_t* ticket = reinterpret_cast<int32_t*>(wspace);
+    const float* tau = reinterpret_cast<const float*>(wspace) + TCAR_QROWS;
+    int32_t* part_cnt = reinterpret_cast<int32_t*>(wspace) + TCAR_QROWS + B;
+    unsigned long long* part = reinterpret_cast<unsigned long long*>(wspace + rec_keys_offset(B));
+    const int xo = x_off ? x_off[b] : 0;
+    const int nl = x_off ? x_off[b + 1] - xo : 0, nx = nl + n_clicks;
+    if (nl < 0 || nx > RX) return;                                   // block-uniform, and the same for every split
+    // the exclusion list, sorted ascending (padded with INT_MAX to a power of two)
+    int P = 1;
+    while (P < nx) P <<= 1;
+    for (int i = tid; i < P; i += 256)
+        s_x[i] = i < nl ? x_ids[xo + i] : i < nx ? clicks[(size_t)b * n_clicks + (i - nl)] - 1 : 0x7fffffff;
+    for (int c = tid; c < XW; c += 256) s_aic[c] = a_ic[(size_t)b * XW + c];
+    for (int c = tid; c < NB; c += 256) s_tq[c] = Tq[(size_t)b * NB + c];
+    for (int i = tid; i < RK; i += 256) s_top[0][i] = KEY_NONE;
+    if (tid == 0) { s_qn = 0; s_cnt = 0; }
+    __syncthreads();
+    for (int k = 2; k <= P; k <<= 1) {
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int i = tid; i < P; i += 256) {
+                const int ixj = i ^ j;
+                if (ixj > i) {
+                    const int a = s_x[i], c = s_x[ixj];
+                    if (((i & k) == 0) ? a > c : a < c) { s_x[i] = c; s_x[ixj] = a; }
+                }
+            }
+            __syncthreads();
+        }
+    }
+    auto excluded = [&](int n) {
+        int lo = 0, hi = nx;
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (s_x[mid] < n) lo = mid + 1; else hi = mid;
+        }
+        return lo < nx && s_x[lo] == n;
+    };
+    const int nchunks = (N + CH - 1) / CH, ntiles = (N + 127) / 128;
+    const float* cm = chunkmax + (size_t)b * (n_pad / CH);
+    const float* tm = tilemax + (size_t)b * (n_pad / 128);
+    const float bound = tau[b];
+    const int per = (ntiles + WSPLIT - 1) / WSPLIT;
+    const int t_lo = split * per, t_hi = min(t_lo + per, ntiles);
+    int cur = 0, my_cnt = 0;
+    for (int t0 = t_lo; t0 < t_hi; t0 += 256) {
+        const int tile = t0 + tid;
+        if (tile < t_hi && tm[tile] >= bound) {
+            float4 v[TILE_CH / 4];
+#pragma unroll
+            for (int c = 0; c < TILE_CH / 4; ++c) v[c] = reinterpret_cast<const float4*>(cm + (size_t)tile * TILE_CH)[c];
+#pragma unroll
+            for (int c = 0; c < TILE_CH; ++c) {
+                const int chunk = tile * TILE_CH + c;
+                const float cv = c % 4 == 0 ? v[c / 4].x : c % 4 == 1 ? v[c / 4].y : c % 4 == 2 ? v[c / 4].z : v[c / 4].w;
+                if (chunk < nchunks && cv >= bound) s_q[atomicAdd(&s_qn, 1)] = chunk;
+            }
+        }
+        __syncthreads();
+        const int qn = s_qn;
+        for (int q0 = 0; q0 < qn; q0 += NCH) {
+            const int ncand = min(qn - q0, NCH) * CH;
+            int P2 = 32;                                              // sort size: power of two >= ncand
+            while (P2 < ncand) P2 <<= 1;
+            if (tid < P2) s_new[tid] = KEY_NONE;
+            __syncthreads();
+            for (int ci = w; ci < ncand; ci += 32) {
+                // four candidates per warp and iteration, branch-free, as in the widening pass; an excluded id or one
+                // >= N reads row 0 instead of its own
+                int nn[4];
+                float sc[4];
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    const int cu = ci + 8 * u;
+                    const int n = cu < ncand ? s_q[q0 + cu / CH] * CH + (cu % CH) : N;
+                    nn[u] = n < N && !excluded(n) ? n : -1;
+                }
+#pragma unroll
+                for (int u = 0; u < 4; ++u)
+                    sc[u] = exact_score_e(s_aic, s_tq, item, content, mwdhm, nn[u] >= 0 ? nn[u] : 0, lane);
+                if (lane == 0) {
+#pragma unroll
+                    for (int u = 0; u < 4; ++u)
+                        if (nn[u] >= 0) { s_new[ci + 8 * u] = rerank_key(sc[u], nn[u]); ++my_cnt; }
+                }
+            }
+            for (int k = 2; k <= P2; k <<= 1) {
+                for (int j = k >> 1; j > 0; j >>= 1) {
+                    __syncthreads();
+                    const int ixj = tid ^ j;
+                    if (tid < P2 && ixj > tid) {
+                        const unsigned long long a = s_new[tid], c = s_new[ixj];
+                        if (((tid & k) == 0) ? a > c : a < c) { s_new[tid] = c; s_new[ixj] = a; }
+                    }
+                }
+            }
+            __syncthreads();
+            merge_topk(s_top[cur], K, s_new, P2, s_top[cur ^ 1]);
+            cur ^= 1;
+        }
+        if (tid == 0) s_qn = 0;
+        __syncthreads();
+    }
+    // partial list and count of this split, then the ticket: the last split CTA of the query merges all of them
+    if (lane == 0 && my_cnt) atomicAdd(&s_cnt, my_cnt);
+    unsigned long long* mine = part + ((size_t)split * B + b) * RK;
+    for (int i = tid; i < K; i += 256) mine[i] = s_top[cur][i];
+    __syncthreads();
+    if (tid == 0) part_cnt[(size_t)split * B + b] = s_cnt;
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) s_last = atomicAdd(&ticket[b], 1) == WSPLIT - 1;
+    __syncthreads();
+    if (!s_last) return;
+    __threadfence();
+    for (int s = 0; s < WSPLIT; ++s) {
+        if (s == split) continue;
+        const unsigned long long* other = part + ((size_t)s * B + b) * RK;
+        for (int i = tid; i < K; i += 256) s_new[i] = __ldcg(other + i);
+        __syncthreads();
+        merge_topk(s_top[cur], K, s_new, K, s_top[cur ^ 1]);
+        cur ^= 1;
+    }
+    for (int r = tid; r < K; r += 256) {
+        const unsigned long long key = s_top[cur][r];
+        out_ids[(size_t)b * K + r] = key == KEY_NONE ? -1 : (int)(uint32_t)key;
+        out_scores[(size_t)b * K + r] = key == KEY_NONE ? -INFINITY : key_value(~(uint32_t)(key >> 32));
+    }
+    if (tid == 0) {
+        if (rescored) {
+            int t = 0;
+            for (int s = 0; s < WSPLIT; ++s) t += __ldcg(part_cnt + (size_t)s * B + b);
+            rescored[b] = t;
+        }
+        ticket[b] = 0;
+    }
+}
+
 }  // namespace tcar
 
 using namespace tcar;
@@ -1256,6 +1559,31 @@ extern "C" int tcar_rerank(const float* a_ic, const float* Tq, const float* item
     if (B == 0) return 0;
     launch_pdl(rerank_kernel, dim3(B), dim3(256), 0, STREAM, a_ic, Tq, item, content, mwdhm, cand_off, cand_ids, label,
                N, max_len, scores, ranked, label_rank, auc);
+    return (int)cudaGetLastError();
+}
+
+extern "C" long long tcar_recommend_ws_bytes(int B) {
+    if (B < 0 || B > TCAR_QROWS) return TCAR_ERR_ARG;
+    return (long long)(rec_keys_offset(B) + (size_t)WSPLIT * B * RK * 8);
+}
+
+extern "C" int tcar_recommend(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
+                              const float* item, const float* content, const int32_t* mwdhm, const float* cat_stats,
+                              const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B, int N,
+                              int n_pad, int K, void* workspace, int32_t* ids, float* scores, int32_t* rescored,
+                              void* stream) {
+    if (B < 0 || B > TCAR_QROWS || N < 1 || n_pad < N || n_pad % 128 || K < 1 || K > RK ||
+        (clicks && (T < 1 || T > RX)) || !chunkmax || !tilemax || !a_ic || !Tq || !item || !content || !mwdhm ||
+        !cat_stats || (x_off && !x_ids) || !workspace || !ids || !scores)
+        return TCAR_ERR_ARG;
+    if (B == 0) return 0;
+    const int n_clicks = clicks ? T : 0;
+    char* ws = static_cast<char*>(workspace);
+    cudaError_t e = launch_pdl(recommend_select_kernel, dim3(B), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq,
+                               cat_stats, x_off, n_clicks, K, N, n_pad, reinterpret_cast<float*>(ws) + TCAR_QROWS);
+    if (e != cudaSuccess) return (int)e;
+    launch_pdl(recommend_scan_kernel, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq, item,
+               content, mwdhm, x_off, x_ids, clicks, n_clicks, K, N, n_pad, B, ws, ids, scores, rescored);
     return (int)cudaGetLastError();
 }
 

@@ -62,7 +62,18 @@ def main(args):
         model.test(None, sent_data, args)
     if args.get("impression_eval"):
         model.test_impressions(None, test_data if is_train else sent_data, neighbor, item_dict, args)
+    if args.get("recommend_k") is not None or args.get("recommend_exclude_clicked"):
+        model.recommend_split(None, test_data if is_train else sent_data, item_dict, args)
     return model
+
+
+def recommend_k(text):
+    """--recommend_k: an integer in [1, TCAR_RECOMMEND_MAXK], checked before any data is loaded."""
+    from ._native import RECOMMEND_MAXK
+    k = int(text)
+    if not 1 <= k <= RECOMMEND_MAXK:
+        raise argparse.ArgumentTypeError(f"must be in [1, {RECOMMEND_MAXK}]")
+    return k
 
 
 def build_parser():
@@ -108,6 +119,11 @@ def build_parser():
     # not a reference flag: after training / testing, also rank every session's impression list (the MIND protocol:
     # AUC, MRR, nDCG@5, nDCG@10; Seq2SeqAttNN.test_impressions) with the impression file as the neighbour dict
     parser.add_argument("--impression_eval", action="store_true")
+    # not a reference flag: after training / testing, also write every session's exact top-K of the whole catalog
+    # (Seq2SeqAttNN.recommend_split: saved/recommend_<foldnum>.txt, HR / MRR / nDCG@K); K defaults to 20, at most 256
+    parser.add_argument("--recommend_k", default=None, type=recommend_k)
+    # not a reference flag: leave a session's own clicked articles out of its recommendations
+    parser.add_argument("--recommend_exclude_clicked", action="store_true")
     parser.add_argument("--inputdata", default="test", type=str)
     parser.add_argument("--threshold_acc", default=0.27, type=float)
     # additions

@@ -1364,6 +1364,138 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             m["auc"], m["mrr"], m["ndcg5"], m["ndcg10"], m["sessions"], m["skipped"]))
         return m
 
+    # ------------------------------------------------------------------------------------------- top-K recommendation
+    def recommend(self, bt, k=20, exclude_off=None, exclude_ids=None, exclude_clicked=False):
+        """The exact top-k of the whole catalog for every session of bt (tcar_recommend), 1 <= k <= nv.RECOMMEND_MAXK,
+        ordered by (score desc, id asc).  Scores are the exact fp32 scores of the full-catalog evaluation: with k <= 20
+        and no exclusions the result is the prefix of eval_step's top-20, and an item scores bit for bit what eval_step
+        and rerank report for it.
+
+        Exclusions: session b never gets exclude_ids[exclude_off[b]:exclude_off[b + 1]] (0-based item ids in host
+        arrays, duplicates allowed; exclude_off has B + 1 entries from 0 to len(exclude_ids)) nor, with
+        exclude_clicked=True, the articles of its own clicks (read on the device from bt.seq).  A session's list
+        length plus T (with exclude_clicked) is at most nv.RECOMMEND_MAXX.
+
+        Returns device tensors (ids [B, k] int32, scores [B, k] fp32); a catalog of fewer than k eligible items pads
+        with -1 / -inf.  The number of items each session re-scored exactly is left in self.rec_rescored[:B].
+        bt.label plays no part in the result (the session forward reads it, so a serving caller fills it with any
+        valid item id)."""
+        if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= nv.RECOMMEND_MAXK:
+            raise ValueError(f"k must be an integer in [1, TCAR_RECOMMEND_MAXK = {nv.RECOMMEND_MAXK}], got {k!r}")
+        if (exclude_off is None) != (exclude_ids is None):
+            raise ValueError("exclude_off and exclude_ids are given together")
+        k, B, N = int(k), bt.B, self.N
+        extra = bt.T if exclude_clicked else 0
+        host = None
+        if exclude_off is not None:
+            # validated in the callers' own integer type (min / max first: no int64 copy of a long list)
+            off, ids = np.asarray(exclude_off).reshape(-1), np.asarray(exclude_ids).reshape(-1)
+            if off.dtype.kind not in "iu" or (ids.size and ids.dtype.kind not in "iu"):
+                raise ValueError("exclude_off and exclude_ids must hold integers")
+            if off.shape[0] != B + 1 or off[0] != 0 or off[-1] != ids.shape[0]:
+                raise ValueError(f"exclude_off must hold B + 1 = {B + 1} offsets from 0 to len(exclude_ids) = "
+                                 f"{ids.shape[0]}")
+            lens = np.diff(off.astype(np.int64))
+            for bad, what in ((lens < 0, "exclude_off decreases"),
+                              (lens + extra > nv.RECOMMEND_MAXX,
+                               f"more than TCAR_RECOMMEND_MAXX = {nv.RECOMMEND_MAXX} exclusions" +
+                               (f" with its {extra} clicks" if extra else ""))):
+                if bad.any():
+                    raise ValueError(f"session {int(np.argmax(bad))}: {what}")
+            if ids.size and (ids.min() < 0 or ids.max() >= N):
+                j = int(np.argmax((ids < 0) | (ids >= N)))
+                s = int(np.searchsorted(off, j, side="right")) - 1
+                raise ValueError(f"session {s}: excluded id {int(ids[j])} outside [0, {N})")
+            host = np.empty(B + 1 + ids.shape[0], dtype=np.int32)
+            host[:B + 1], host[B + 1:] = off, ids
+        elif extra > nv.RECOMMEND_MAXX:
+            raise ValueError(f"session 0: more than TCAR_RECOMMEND_MAXX = {nv.RECOMMEND_MAXX} clicks")
+        dev, p, ps = self.dev, nv.ptr, self.ps
+        out_ids = torch.empty(B, k, device=dev, dtype=torch.int32)
+        out_sc = torch.empty(B, k, device=dev)
+        if B == 0:
+            return out_ids, out_sc
+        if getattr(self, "_rec_ws", None) is None:
+            # ticket counters first: zero once, every call leaves them at zero
+            self._rec_ws = torch.zeros(int(nv.lib().tcar_recommend_ws_bytes(QROWS)), device=dev, dtype=torch.uint8)
+            self.rec_rescored = torch.zeros(QROWS, device=dev, dtype=torch.int32)
+        if not self._item_table_synced:
+            self.sync_item_table()         # after catalog-sharded training every rank holds only its own rows
+        self._session_forward(bt)
+        self._ensure_cat_stats()
+        ws = self._score_buffers(ps.n_pad, False)
+        # one unguarded eval-mode GEMM for the chunk / tile maxima; its softmax partial sums (which may overflow without
+        # the guard) are not read
+        nv.counted_call("tcar_score_fwd", 1, p(self.Q), p(ps.iext), p(self.c_ref), None, p(ws["part"]), p(ws["cmax"]),
+                        p(ws["tmax"]), B, N, ps.n_pad, 1, self._cluster_for(B))
+        csr = self._stage_ints(host) if host is not None else None
+        nv.counted_call("tcar_recommend", 2, p(ws["cmax"]), p(ws["tmax"]), p(self.a_ic), p(self.Tq), p(ps.item),
+                        p(ps.content), p(ps.mwdhm), p(self.cat_stats), p(csr),
+                        p(csr[B + 1:]) if csr is not None else None, p(bt.seq) if exclude_clicked else None, bt.T, B,
+                        N, ps.n_pad, k, p(self._rec_ws), p(out_ids), p(out_sc), p(self.rec_rescored))
+        return out_ids, out_sc
+
+    def recommend_split(self, sess, test_data, item_dict, args):
+        """Recommend the top-K articles (args["recommend_k"], default 20) for every session of a split, optionally
+        without the session's own clicks (args["recommend_exclude_clicked"]), in the batches test() uses.  Writes one
+        line per session to saved/recommend_<foldnum>[_rank<r>].txt (util.recommend_line: the session key, then K
+        `article:score` pairs with the original article ids) and prints and returns {"hr", "mrr", "ndcg", "sessions"}
+        @K, where a session's rank is its label's 1-based position in the returned list (ties go to the lower id).
+        Under torchrun batch i goes to rank i mod world (each rank writes its own file) and the sums are all-reduced,
+        so every rank returns the metrics of the whole split."""
+        from .util import label_positions, recommend_line, topk_metrics, topk_sums
+        k = int(args.get("recommend_k") or 20)
+        clicked = bool(args.get("recommend_exclude_clicked"))
+        print("Recommending the top-{} articles{}...".format(k, " without the clicked ones" if clicked else ""))
+        self.sync_item_table()
+        (len_dict_test, session_dict_test, session_time_dict_test) = test_data
+        reverse = self.reverse_item if self.reverse_item is not None else \
+            {cnt - 1: art for art, cnt in item_dict.items()}
+        sampler = Sampler(len_dict_test, session_dict_test, session_time_dict_test, batch_size=self.batch_size)
+        keys = list(sampler.session_id_batches)
+        dist_on = parallel.is_distributed(self.world)
+        if dist_on:
+            sampler.session_id_batches = sampler.session_id_batches[self.rank::self.world]
+            sampler.batch_num = len(sampler.session_id_batches)
+            keys = keys[self.rank::self.world]
+        os.makedirs("saved", exist_ok=True)
+        path = "saved/recommend_{}{}.txt".format(args.get("foldnum", 0), "_rank{}".format(self.rank) if dist_on else "")
+        sums = np.zeros(4)
+
+        def consume(kb, ids_h, sc_h):
+            nonlocal sums
+            ids, sc = ids_h.get().numpy(), sc_h.get().numpy()
+            labels = [session_dict_test[key][-1] - 1 for key in kb]
+            sums += topk_sums(label_positions(ids, labels))
+            f.writelines(recommend_line(key, ids[b], sc[b], reverse) for b, key in enumerate(kb))
+
+        with open(path, "w") as f:
+            # one batch of look-ahead (as in test()): batch i+1 is staged before batch i is scored, and batch i's lists
+            # are read from pinned memory while batch i+1 runs
+            it = zip((self.stage_to_device(packed, B, T, Nn) for packed, B, T, Nn in prefetch_packed(sampler)), keys)
+            cur, pending = next(it, None), None
+            while cur is not None:
+                nxt = next(it, None)
+                bt, kb = cur
+                ids, sc = self.recommend(bt, k, exclude_clicked=clicked)
+                handles = (kb, self.fetch_async(ids), self.fetch_async(sc))
+                if pending is not None:
+                    consume(*pending)
+                pending, cur = handles, nxt
+            if pending is not None:
+                consume(*pending)
+        if dist_on:
+            import torch.distributed as dist
+            t = torch.from_numpy(sums).to(self.dev)
+            dist.all_reduce(t, op=dist.ReduceOp.SUM)
+            sums = t.cpu().numpy()
+        m = topk_metrics(sums)
+        self.last_recommend_metrics = m
+        self.last_recommend_path = path
+        print("Recommend: HR@{k}: {}, MRR@{k}: {}, nDCG@{k}: {} ({} sessions, written to {})".format(
+            m["hr"], m["mrr"], m["ndcg"], m["sessions"], path, k=k))
+        return m
+
     # ------------------------------------------------------------------------------------------- metrics
     def _categories(self):
         if self._cat_array is None:

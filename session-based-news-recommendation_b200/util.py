@@ -46,6 +46,41 @@ def impression_metrics(sums):
     return out
 
 
+def label_positions(ids, labels):
+    """1-based position of each session's label in its recommended list ids [B, K] (0 when absent)."""
+    ids = np.asarray(ids)
+    hit = ids == np.asarray(labels).reshape(-1, 1)
+    return np.where(hit.any(1), hit.argmax(1) + 1, 0)
+
+
+def topk_sums(rank):
+    """Label positions in top-K lists (label_positions; 0 = not in the list) -> float64 [4]: the sums of HR@K (hit),
+    MRR@K (1/rank) and nDCG@K (1/log2(1 + rank)), misses counting 0, and the number of sessions.  Sums add up across
+    batches and ranks; topk_metrics averages them."""
+    r = np.asarray(rank, dtype=np.float64)
+    hit = r > 0
+    rr = np.where(hit, r, 1.0)
+    return np.array([hit.sum(), np.where(hit, 1.0 / rr, 0.0).sum(), np.where(hit, 1.0 / np.log2(1.0 + rr), 0.0).sum(),
+                     len(r)], dtype=np.float64)
+
+
+def topk_metrics(sums):
+    """topk_sums (possibly added up) -> {"hr", "mrr", "ndcg", "sessions"}."""
+    s = np.asarray(sums, dtype=np.float64)
+    n = s[3]
+    out = {k: float(s[i] / n) if n > 0 else float("nan") for i, k in enumerate(("hr", "mrr", "ndcg"))}
+    out["sessions"] = int(n)
+    return out
+
+
+def recommend_line(key, ids, scores, reverse_item):
+    """One line of a recommendation file: the session key, then `article:score` for every returned item (original
+    article ids through reverse_item, 0-based item id -> article; the -1 padding of a small catalog is left out).
+    Scores are printed with 9 significant digits, enough to read back the fp32 value exactly."""
+    pairs = ["{}:{:.9g}".format(reverse_item[int(i)], float(s)) for i, s in zip(ids, scores) if i >= 0]
+    return " ".join([str(key)] + pairs) + "\n"
+
+
 def _load(path):
     with open(path, "rb") as f:
         return pickle.load(f)
