@@ -20,6 +20,7 @@ from . import parallel
 from .catalog_parallel import CatalogShardedTraining
 from .params import ParamStore, SMALL
 from .sampler import Sampler, pack_batch
+from .util import check_id_lists
 
 H, TH, XW, PW, NB, KEXT, QROWS, TOPK = nv.H, nv.TH, nv.XW, nv.PW, nv.NBINS, nv.KEXT, nv.QROWS, nv.TOPK
 
@@ -73,6 +74,23 @@ def prefetch_packed(sampler, depth=4):
             yield item
     finally:
         sys.setswitchinterval(old_interval)
+
+
+def pipelined(items, launch, consume):
+    """One item of look-ahead, the loop of test() / test_impressions() / recommend_split(): launch(cur, nxt) enqueues
+    item i (nxt = item i + 1, None for the last; items are never None) and returns the handles of its results, or
+    None when there is nothing to read back; consume(*handles) of item i runs after item i + 1 has been launched, so
+    the host reads item i's results from pinned memory while item i + 1 runs on the device."""
+    it = iter(items)
+    cur, pending = next(it, None), None
+    while cur is not None:
+        nxt = next(it, None)
+        handles = launch(cur, nxt)
+        if pending is not None:
+            consume(*pending)
+        pending, cur = handles, nxt
+    if pending is not None:
+        consume(*pending)
 
 
 class PinnedRing:
@@ -1283,25 +1301,14 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         list and every other entry a negative; label_rank = 1 + #negatives scoring above it (the label wins ties),
         auc counts a tied negative as 1/2 and is NaN for a list without negatives.  metrics=False returns None for
         the last two, so a serving caller may fill bt.label with any valid item id."""
-        # validated in the callers' own integer type (min / max first: no int64 copy of a long list)
-        off, ids = np.asarray(cand_off).reshape(-1), np.asarray(cand_ids).reshape(-1)
-        if off.dtype.kind not in "iu" or (ids.size and ids.dtype.kind not in "iu"):
-            raise ValueError("cand_off and cand_ids must hold integers")
         B, N = bt.B, self.N
-        if off.shape[0] != B + 1 or off[0] != 0 or off[-1] != ids.shape[0]:
-            raise ValueError(f"cand_off must hold B + 1 = {B + 1} offsets from 0 to len(cand_ids) = {ids.shape[0]}")
-        lens = np.diff(off.astype(np.int64))
-        for bad, what in ((lens < 0, "cand_off decreases"),
-                          (lens > nv.RERANK_MAXL, f"more than TCAR_RERANK_MAXL = {nv.RERANK_MAXL} candidates")):
-            if bad.any():
-                raise ValueError(f"session {int(np.argmax(bad))}: {what}")
-        if ids.size and (ids.min() < 0 or ids.max() >= N):
-            j = int(np.argmax((ids < 0) | (ids >= N)))
-            s = int(np.searchsorted(off, j, side="right")) - 1
-            raise ValueError(f"session {s}: candidate id {int(ids[j])} outside [0, {N})")
+        host, max_len = check_id_lists(cand_off, cand_ids, B, N, names=("cand_off", "cand_ids"),
+                                       nouns=("candidate id", "candidates"), limit=nv.RERANK_MAXL,
+                                       limit_name="TCAR_RERANK_MAXL")
+        nnz = host.shape[0] - (B + 1)
         dev, p, ps = self.dev, nv.ptr, self.ps
-        scores = torch.empty(ids.shape[0], device=dev)
-        ranked = torch.empty(ids.shape[0], device=dev, dtype=torch.int32)
+        scores = torch.empty(nnz, device=dev)
+        ranked = torch.empty(nnz, device=dev, dtype=torch.int32)
         label_rank = torch.empty(B, device=dev, dtype=torch.int32) if metrics else None
         auc = torch.empty(B, device=dev) if metrics else None
         if B == 0:
@@ -1309,13 +1316,26 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         if not self._item_table_synced:
             self.sync_item_table()         # after catalog-sharded training every rank holds only its own rows
         self._session_forward(bt)
-        host = np.empty(B + 1 + ids.shape[0], dtype=np.int32)
-        host[:B + 1], host[B + 1:] = off, ids
         csr = self._stage_ints(host)
         nv.counted_call("tcar_rerank", 1, p(self.a_ic), p(self.Tq), p(ps.item), p(ps.content), p(ps.mwdhm), p(csr),
-                        p(csr[B + 1:]), p(bt.label) if metrics else None, B, N, int(lens.max()), p(scores), p(ranked),
+                        p(csr[B + 1:]), p(bt.label) if metrics else None, B, N, max_len, p(scores), p(ranked),
                         p(label_rank), p(auc))
         return scores, ranked, label_rank, auc
+
+    def _eval_sampler(self, test_data):
+        """The batches of a split as test() walks them; under torchrun only this rank's (Sampler.keep_rank_batches)."""
+        sampler = Sampler(*test_data, batch_size=self.batch_size)
+        if parallel.is_distributed(self.world):
+            sampler.keep_rank_batches(self.rank, self.world)
+        return sampler
+
+    def _sum_over_ranks(self, sums):
+        """This rank's float64 metric sums -> their sum over all ranks (unchanged on one GPU)."""
+        if not parallel.is_distributed(self.world):
+            return sums
+        t = torch.as_tensor(sums, device=self.dev)
+        parallel.allreduce_sum((t,), self.world)
+        return t.cpu().numpy()
 
     def test_impressions(self, sess, test_data, impressions, item_dict, args):
         """Rank every session's impression list (the MIND protocol): the clicked article (the label) is the positive,
@@ -1328,37 +1348,24 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         from .util import impression_metrics, impression_sums
         print("Ranking impression lists...")
         self.sync_item_table()
-        (len_dict_test, session_dict_test, session_time_dict_test) = test_data
-        sampler = Sampler(len_dict_test, session_dict_test, session_time_dict_test, batch_size=self.batch_size)
-        # every batch's lists up front, so that the producer thread does no dictionary work per batch
+        session_dict_test = test_data[1]
+        sampler = self._eval_sampler(test_data)
+        # this rank's lists up front, so that the producer thread does no dictionary work per batch
         cands = [impression_candidates(keys, [session_dict_test[k][-1] - 1 for k in keys], impressions, item_dict)
                  for keys in sampler.session_id_batches]
-        dist_on = parallel.is_distributed(self.world)
-        if dist_on:
-            sampler.session_id_batches = sampler.session_id_batches[self.rank::self.world]
-            sampler.batch_num = len(sampler.session_id_batches)
-            cands = cands[self.rank::self.world]
         sums = np.zeros(6)
-        # one batch of look-ahead (as in test()): batch i+1 is staged before batch i is ranked, and batch i's results
-        # are read from pinned memory while batch i+1 runs
-        it = zip((self.stage_to_device(packed, B, T, Nn) for packed, B, T, Nn in prefetch_packed(sampler)), cands)
-        cur, pending = next(it, None), None
-        while cur is not None:
-            nxt = next(it, None)
+
+        def launch(cur, nxt):
             bt, (off, ids) = cur
             _, _, rank, auc = self.rerank(bt, off, ids)
-            handles = (np.diff(off) - 1, self.fetch_async(rank), self.fetch_async(auc))
-            if pending is not None:
-                sums += impression_sums(pending[1].get().numpy(), pending[2].get().numpy(), pending[0])
-            pending, cur = handles, nxt
-        if pending is not None:
-            sums += impression_sums(pending[1].get().numpy(), pending[2].get().numpy(), pending[0])
-        if dist_on:
-            import torch.distributed as dist
-            t = torch.from_numpy(sums).to(self.dev)
-            dist.all_reduce(t, op=dist.ReduceOp.SUM)
-            sums = t.cpu().numpy()
-        m = impression_metrics(sums)
+            return np.diff(off) - 1, self.fetch_async(rank), self.fetch_async(auc)
+
+        def consume(n_neg, rank, auc):
+            sums[:] += impression_sums(rank.get().numpy(), auc.get().numpy(), n_neg)
+
+        pipelined(zip((self.stage_to_device(packed, B, T, Nn) for packed, B, T, Nn in prefetch_packed(sampler)), cands),
+                  launch, consume)
+        m = impression_metrics(self._sum_over_ranks(sums))
         self.last_impression_metrics = m
         print("Impressions: AUC: {}, MRR: {}, nDCG@5: {}, nDCG@10: {} ({} sessions, {} without a negative skipped)".format(
             m["auc"], m["mrr"], m["ndcg5"], m["ndcg10"], m["sessions"], m["skipped"]))
@@ -1388,26 +1395,9 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         extra = bt.T if exclude_clicked else 0
         host = None
         if exclude_off is not None:
-            # validated in the callers' own integer type (min / max first: no int64 copy of a long list)
-            off, ids = np.asarray(exclude_off).reshape(-1), np.asarray(exclude_ids).reshape(-1)
-            if off.dtype.kind not in "iu" or (ids.size and ids.dtype.kind not in "iu"):
-                raise ValueError("exclude_off and exclude_ids must hold integers")
-            if off.shape[0] != B + 1 or off[0] != 0 or off[-1] != ids.shape[0]:
-                raise ValueError(f"exclude_off must hold B + 1 = {B + 1} offsets from 0 to len(exclude_ids) = "
-                                 f"{ids.shape[0]}")
-            lens = np.diff(off.astype(np.int64))
-            for bad, what in ((lens < 0, "exclude_off decreases"),
-                              (lens + extra > nv.RECOMMEND_MAXX,
-                               f"more than TCAR_RECOMMEND_MAXX = {nv.RECOMMEND_MAXX} exclusions" +
-                               (f" with its {extra} clicks" if extra else ""))):
-                if bad.any():
-                    raise ValueError(f"session {int(np.argmax(bad))}: {what}")
-            if ids.size and (ids.min() < 0 or ids.max() >= N):
-                j = int(np.argmax((ids < 0) | (ids >= N)))
-                s = int(np.searchsorted(off, j, side="right")) - 1
-                raise ValueError(f"session {s}: excluded id {int(ids[j])} outside [0, {N})")
-            host = np.empty(B + 1 + ids.shape[0], dtype=np.int32)
-            host[:B + 1], host[B + 1:] = off, ids
+            host, _ = check_id_lists(exclude_off, exclude_ids, B, N, names=("exclude_off", "exclude_ids"),
+                                     nouns=("excluded id", "exclusions"), limit=nv.RECOMMEND_MAXX,
+                                     limit_name="TCAR_RECOMMEND_MAXX", extra=extra)
         elif extra > nv.RECOMMEND_MAXX:
             raise ValueError(f"session 0: more than TCAR_RECOMMEND_MAXX = {nv.RECOMMEND_MAXX} clicks")
         dev, p, ps = self.dev, nv.ptr, self.ps
@@ -1448,48 +1438,31 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         clicked = bool(args.get("recommend_exclude_clicked"))
         print("Recommending the top-{} articles{}...".format(k, " without the clicked ones" if clicked else ""))
         self.sync_item_table()
-        (len_dict_test, session_dict_test, session_time_dict_test) = test_data
+        session_dict_test = test_data[1]
         reverse = self.reverse_item if self.reverse_item is not None else \
             {cnt - 1: art for art, cnt in item_dict.items()}
-        sampler = Sampler(len_dict_test, session_dict_test, session_time_dict_test, batch_size=self.batch_size)
+        sampler = self._eval_sampler(test_data)
         keys = list(sampler.session_id_batches)
-        dist_on = parallel.is_distributed(self.world)
-        if dist_on:
-            sampler.session_id_batches = sampler.session_id_batches[self.rank::self.world]
-            sampler.batch_num = len(sampler.session_id_batches)
-            keys = keys[self.rank::self.world]
         os.makedirs("saved", exist_ok=True)
+        dist_on = parallel.is_distributed(self.world)
         path = "saved/recommend_{}{}.txt".format(args.get("foldnum", 0), "_rank{}".format(self.rank) if dist_on else "")
         sums = np.zeros(4)
 
+        def launch(cur, nxt):
+            bt, kb = cur
+            ids, sc = self.recommend(bt, k, exclude_clicked=clicked)
+            return kb, self.fetch_async(ids), self.fetch_async(sc)
+
         def consume(kb, ids_h, sc_h):
-            nonlocal sums
             ids, sc = ids_h.get().numpy(), sc_h.get().numpy()
             labels = [session_dict_test[key][-1] - 1 for key in kb]
-            sums += topk_sums(label_positions(ids, labels))
+            sums[:] += topk_sums(label_positions(ids, labels))
             f.writelines(recommend_line(key, ids[b], sc[b], reverse) for b, key in enumerate(kb))
 
         with open(path, "w") as f:
-            # one batch of look-ahead (as in test()): batch i+1 is staged before batch i is scored, and batch i's lists
-            # are read from pinned memory while batch i+1 runs
-            it = zip((self.stage_to_device(packed, B, T, Nn) for packed, B, T, Nn in prefetch_packed(sampler)), keys)
-            cur, pending = next(it, None), None
-            while cur is not None:
-                nxt = next(it, None)
-                bt, kb = cur
-                ids, sc = self.recommend(bt, k, exclude_clicked=clicked)
-                handles = (kb, self.fetch_async(ids), self.fetch_async(sc))
-                if pending is not None:
-                    consume(*pending)
-                pending, cur = handles, nxt
-            if pending is not None:
-                consume(*pending)
-        if dist_on:
-            import torch.distributed as dist
-            t = torch.from_numpy(sums).to(self.dev)
-            dist.all_reduce(t, op=dist.ReduceOp.SUM)
-            sums = t.cpu().numpy()
-        m = topk_metrics(sums)
+            pipelined(zip((self.stage_to_device(packed, B, T, Nn) for packed, B, T, Nn in prefetch_packed(sampler)),
+                          keys), launch, consume)
+        m = topk_metrics(self._sum_over_ranks(sums))
         self.last_recommend_metrics = m
         self.last_recommend_path = path
         print("Recommend: HR@{k}: {}, MRR@{k}: {}, nDCG@{k}: {} ({} sessions, written to {})".format(
@@ -1615,18 +1588,9 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         ranks, so every rank prints / returns the metrics of the whole test set."""
         print("Measuring...")
         self.sync_item_table()
-        (len_dict_test, session_dict_test, session_time_dict_test) = test_data
         acc = {"mrr": [], "recall": [], "ndcg": [], "ild": [], "unexp": [], "loss": [], "items": {}}
-        sampler = Sampler(len_dict_test, session_dict_test, session_time_dict_test, batch_size=self.batch_size)
+        sampler = self._eval_sampler(test_data)         # the producer thread packs only this rank's batches
         dist_on = parallel.is_distributed(self.world)
-        R, me = (self.world, self.rank) if dist_on else (1, 0)
-        sizes = [len(b) for b in sampler.session_id_batches]
-        lens = [len(sampler.session_dict[b[0]]) - 1 for b in sampler.session_id_batches]
-        rounds = (len(sizes) + R - 1) // R
-        if dist_on:
-            # this rank's batches: me, me + R, ... (the producer thread packs only those)
-            sampler.session_id_batches = sampler.session_id_batches[me::R]
-            sampler.batch_num = len(sampler.session_id_batches)
         batch = 0
 
         def consume(packed, B, T, top, ngt, ce):
@@ -1655,44 +1619,40 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             if args.get("is_print"):
                 self.printData(str(args["foldnum"]) + "_" + str(self.curEpoch), batch_in, batch_out, batch_pred)
 
-        # one batch of look-ahead (as in train): batch i+1 is staged before batch i is evaluated, and batch i's results
-        # are read from pinned memory while batch i+1 runs
         staged = ((packed, B, T, self.stage_to_device(packed, B, T, Nn)) for packed, B, T, Nn in prefetch_packed(sampler))
-        pending = None
         if dist_on:
-            for r in range(rounds):
-                counts = [sizes[r * R + g] if r * R + g < len(sizes) else 0 for g in range(R)]
-                if counts[me]:
-                    packed, B, T, bt = next(staged)
-                else:
-                    packed, B, T = None, 0, lens[0]
-                    bt = Batch(torch.zeros(0, device=self.dev, dtype=torch.int32), 0, T, 0)
+            # round r evaluates batches r * R ... r * R + R - 1, one per rank; a rank without a batch in the last round
+            # still takes part in its collectives with B = 0
+            R, me, sizes = self.world, self.rank, sampler.global_sizes
+
+            def rounds():
+                for r in range(0, len(sizes), R):
+                    counts = [sizes[r + g] if r + g < len(sizes) else 0 for g in range(R)]
+                    if counts[me]:
+                        yield counts, next(staged)
+                    else:
+                        T = sampler.batch_T[0]
+                        yield counts, (None, 0, T, Batch(torch.zeros(0, device=self.dev, dtype=torch.int32), 0, T, 0))
+
+            def launch(cur, nxt):
+                counts, (packed, B, T, bt) = cur
                 top, ngt, ce = self.eval_round(bt, counts)
-                handles = [self.fetch_async(x) for x in (top, ngt, ce)] if B else None
-                if pending is not None:
-                    consume(*pending)
-                pending = (packed, B, T, *handles) if B else None
+                return (packed, B, T, *[self.fetch_async(x) for x in (top, ngt, ce)]) if B else None
+
+            pipelined(rounds(), launch, consume)
         else:
-            cur = next(staged, None)
-            while cur is not None:
-                nxt = next(staged, None)
+            def launch(cur, nxt):
                 packed, B, T, bt = cur
-                cur = nxt
                 top, ngt, ce = self.eval_step(bt, next_bt=nxt[3] if nxt is not None else None)
-                handles = [self.fetch_async(x) for x in (top, ngt, ce)]
-                if pending is not None:
-                    consume(*pending)
-                pending = (packed, B, T, *handles)
-        if pending is not None:
-            consume(*pending)
+                return (packed, B, T, *[self.fetch_async(x) for x in (top, ngt, ce)])
+
+            pipelined(staged, launch, consume)
         sums = np.array([np.sum(acc["loss"]), len(acc["loss"]), np.sum(acc["ild"]), len(acc["ild"]), np.sum(acc["unexp"]),
                          np.sum(acc["mrr"]), np.sum(acc["recall"]), np.sum(acc["ndcg"])], dtype=np.float64)
+        sums = self._sum_over_ranks(sums)
         coverage = len(acc["items"])
         if dist_on:
             import torch.distributed as dist
-            t = torch.from_numpy(sums).to(self.dev)
-            dist.all_reduce(t, op=dist.ReduceOp.SUM)
-            sums = t.cpu().numpy()
             seen = torch.zeros(self.N, device=self.dev, dtype=torch.int32)
             if acc["items"]:
                 seen[torch.tensor(list(acc["items"].keys()), device=self.dev, dtype=torch.long)] = 1

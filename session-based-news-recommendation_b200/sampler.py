@@ -124,8 +124,7 @@ class Sampler(object):
         so that the global `random` stream -- which shuffles the next epoch's batches -- stays identical on all ranks;
         the NumPy stream of the uniform negatives is per process anyway (reseed it per rank for distinct draws)."""
         from .parallel import shard_sessions
-        self.global_sizes = [len(b) for b in self.session_id_batches]
-        self.batch_T = [len(self.session_dict[b[0]]) - 1 for b in self.session_id_batches]
+        self._record_global_batches()
         out = []
         for b in self.session_id_batches:
             lo, hi = shard_sessions(len(b), rank, world)
@@ -133,6 +132,19 @@ class Sampler(object):
         self.session_id_batches = out
         self._choice = random.Random(2020 + 7919 * rank).choice
         return self
+
+    def keep_rank_batches(self, rank, world):
+        """Evaluation under torchrun: batch i of the split goes to rank i mod world, so keep this rank's whole batches
+        rank, rank + world, ...  `global_sizes` / `batch_T` keep the size and session length of every batch of the
+        split (as restrict_to_rank does), from which all ranks derive the same rounds."""
+        self._record_global_batches()
+        self.session_id_batches = self.session_id_batches[rank::world]
+        self.batch_num = len(self.session_id_batches)
+        return self
+
+    def _record_global_batches(self):
+        self.global_sizes = [len(b) for b in self.session_id_batches]
+        self.batch_T = [len(self.session_dict[b[0]]) - 1 for b in self.session_id_batches]
 
     def _features(self, sid):
         f = self._cache.get(sid)
@@ -178,7 +190,8 @@ class Sampler(object):
         yields exactly the values of the reference's B consecutive calls of size Nn (sampler.py:98-99)."""
         ids = self.session_id_batches[self.batch_i]
         B = len(ids)
-        T = self.batch_T[self.batch_i] if getattr(self, "batch_T", None) else len(self.session_dict[ids[0]]) - 1
+        # an empty share of restrict_to_rank takes its global batch's length (batch_T is indexed by global batch)
+        T = len(self.session_dict[ids[0]]) - 1 if B else self.batch_T[self.batch_i]
         Nn = self.neg_num if (self.neighbor_dict and self.neg_num) else 0
         M = B * T
         col = _columnar(self.session_dict, self.session_time_dict)

@@ -81,6 +81,34 @@ def recommend_line(key, ids, scores, reverse_item):
     return " ".join([str(key)] + pairs) + "\n"
 
 
+def check_id_lists(off, ids, B, N, *, names, nouns, limit, limit_name, extra=0):
+    """Validate B per-session id lists in CSR form (session b's ids are ids[off[b]:off[b + 1]]) before anything is
+    launched: off holds B + 1 integer offsets from 0 to len(ids), never decreasing; a list's length plus `extra` (the
+    session's clicks counted against the same limit) is at most `limit`; every id lies in [0, N).  The checks run in
+    the caller's own integer type (min / max first: no int64 copy of a long list) and raise a ValueError that names the
+    first offending session.  names = (offsets, ids) and nouns = (one id, the list's entries) word the messages, e.g.
+    ("cand_off", "cand_ids") and ("candidate id", "candidates").
+    Returns (the int32 host array [off | ids] the kernels read, the longest list's length; 0 when B = 0)."""
+    off, ids = np.asarray(off).reshape(-1), np.asarray(ids).reshape(-1)
+    if off.dtype.kind not in "iu" or (ids.size and ids.dtype.kind not in "iu"):
+        raise ValueError(f"{names[0]} and {names[1]} must hold integers")
+    if off.shape[0] != B + 1 or off[0] != 0 or off[-1] != ids.shape[0]:
+        raise ValueError(f"{names[0]} must hold B + 1 = {B + 1} offsets from 0 to len({names[1]}) = {ids.shape[0]}")
+    lens = np.diff(off.astype(np.int64))
+    for bad, what in ((lens < 0, f"{names[0]} decreases"),
+                      (lens + extra > limit, f"more than {limit_name} = {limit} {nouns[1]}" +
+                       (f" with its {extra} clicks" if extra else ""))):
+        if bad.any():
+            raise ValueError(f"session {int(np.argmax(bad))}: {what}")
+    if ids.size and (ids.min() < 0 or ids.max() >= N):
+        j = int(np.argmax((ids < 0) | (ids >= N)))
+        s = int(np.searchsorted(off, j, side="right")) - 1
+        raise ValueError(f"session {s}: {nouns[0]} {int(ids[j])} outside [0, {N})")
+    host = np.empty(B + 1 + ids.shape[0], dtype=np.int32)
+    host[:B + 1], host[B + 1:] = off, ids
+    return host, int(lens.max()) if B else 0
+
+
 def _load(path):
     with open(path, "rb") as f:
         return pickle.load(f)

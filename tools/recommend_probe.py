@@ -2,11 +2,9 @@
 shape (364 047 items) and the MIND shape (103 630 items), 512 sessions per batch, T in {1, 20}, K in {20, 100, 256},
 with and without the session's own clicks excluded.
 
-    python tools/recommend_probe.py          every workload
-    python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29514 \\
-        tools/recommend_probe.py --check     recommend_split at world 2 == world 1 on a synthetic split, file for file
-                                             and metric for metric (NCCL with a GPU per rank; ranks sharing a GPU use
-                                             gloo)
+    python tools/recommend_probe.py [--shapes globo,mind]
+
+recommend_split across ranks is checked by tools/split_check.py.
 
 Per workload:
   select_us_cold / scan_us_cold   recommend_select_kernel / recommend_scan_kernel alone (torch.profiler, CUDA
@@ -19,43 +17,15 @@ Per workload:
   rescored_mean / rescored_max    items re-scored exactly per query (the width of the error band)
 """
 import argparse
-import copy
 import json
-import os
-import random
-import subprocess
-import sys
-import tempfile
 
 import numpy as np
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-import __graft_entry__ as ge  # noqa: E402
-
-ge.load_package()
-from tcar_b200 import _native as nv, synth  # noqa: E402
-from tcar_b200.model_combine import Seq2SeqAttNN  # noqa: E402
+from probe_common import B, gpu_info, make_model
+from tcar_b200 import _native as nv, synth
 
 SHAPES = {"globo": 364047, "mind": 103630}
-B = 512
-
-
-def make_model(N, rank=0, world=1, seed=2020):
-    content, mwdhm, _ = synth.make_catalog(N, seed=seed)
-    np.random.seed(2020)
-    return Seq2SeqAttNN(dict(publish_time_MWDHM=mwdhm, itemnum=N, category_id=None, item_freq_dict_norm={},
-                             reverse_item=None, content_emb=content, emb_stddev=0.04, stddev=0.05, hidden_size=250,
-                             time_hidden_size=64, l2_emb=0.0, batch_size=B, epoch=1, neg_num=20, lr=0.001,
-                             max_grad=150, rank=rank, world_size=world, train_parallel="dp")), mwdhm
-
-
-def gpu_info():
-    idx = torch.cuda.current_device()
-    out = subprocess.run(["nvidia-smi", "-i", str(idx), "--query-gpu=power.limit", "--format=csv,noheader,nounits"],
-                         capture_output=True, text=True).stdout.strip()
-    return {"gpu": torch.cuda.get_device_name(idx), "power_limit_w": float(out) if out else None}
 
 
 def kernel_times(model, bt, K, clicked, flush):
@@ -121,54 +91,10 @@ def workload(model, mwdhm, shape, T, K, clicked, info, flush):
     print("recommend_probe " + json.dumps(res), flush=True)
 
 
-def check():
-    """recommend_split under torchrun (batch i on rank i mod world, sums all-reduced) == the same split on one GPU: the
-    ranks' files together hold exactly the lines of the single-GPU file, and the metrics agree."""
-    import torch.distributed as dist
-    rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
-    gpus = torch.cuda.device_count()
-    torch.cuda.set_device(local % gpus)
-    if gpus >= world:
-        dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    else:                                                # ranks share a GPU: NCCL needs one GPU per rank, gloo does not
-        dist.init_process_group("gloo")
-    N = 20000
-    len_dict, sdict, tdict, item_dict, _ = synth.make_sessions(N, 3000, train=False)
-    base = os.path.join(tempfile.gettempdir(), "recommend_check")
-    out, files = {}, {}
-    for w in (world, 1):
-        d = os.path.join(base, f"world{w}" + (f"_rank{rank}" if w == 1 else ""))
-        os.makedirs(d, exist_ok=True)
-        os.chdir(d)
-        model, _ = make_model(N, rank if w > 1 else 0, w, seed=3)
-        random.seed(7)                                   # same batches for both runs
-        args = {"recommend_k": 100, "recommend_exclude_clicked": True, "foldnum": 0}
-        out[w] = model.recommend_split(None, (copy.deepcopy(len_dict), sdict, tdict), item_dict, args)
-        files[w] = model.last_recommend_path if w == 1 else None
-        dist.barrier()
-    a, b = out[world], out[1]
-    lines_n = []
-    for r in range(world):
-        lines_n += open(os.path.join(base, f"world{world}", f"saved/recommend_0_rank{r}.txt")).read().splitlines()
-    lines_1 = open(os.path.join(base, f"world1_rank{rank}", files[1])).read().splitlines()
-    same_files = sorted(lines_n) == sorted(lines_1) and len(lines_1) == b["sessions"]
-    same = same_files and a["sessions"] == b["sessions"] and all(abs(a[k] - b[k]) <= 1e-12 for k in ("hr", "mrr", "ndcg"))
-    print(f"rank {rank} recommend_check " + json.dumps(dict(gpu_info(), world=world, gpus=min(gpus, world),
-                                                            backend=dist.get_backend(), K=100, exclude_clicked=True,
-                                                            world_n=a, world_1=b, lines=len(lines_1),
-                                                            files_equal=same_files, equal=same)), flush=True)
-    dist.destroy_process_group()
-    if not same:
-        sys.exit(1)
-
-
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--check", action="store_true")
     ap.add_argument("--shapes", default="globo,mind")
     a = ap.parse_args()
-    if a.check:
-        return check()
     torch.cuda.set_device(0)
     info = gpu_info()
     flush = torch.empty(256 << 20, device="cuda", dtype=torch.uint8)

@@ -2,9 +2,8 @@
 (catalog of 103 630 items, 512 sessions per batch).
 
     python tools/rerank_probe.py             T in {1, 20} x MIND-like list lengths (LogNormal, mean 37); T = 20 x 300
-    python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29513 \
-        tools/rerank_probe.py --check        test_impressions at world 2 == world 1 on a synthetic split
-                                             (NCCL with a GPU per rank; ranks sharing a GPU use gloo)
+
+test_impressions across ranks is checked by tools/split_check.py.
 
 Per workload:
   kernel_us_cold  tcar_rerank alone, CUDA events around every launch, L2 overwritten (256 MB memset) before each one:
@@ -16,43 +15,16 @@ Per workload:
                   session plus the session vectors (500 + 139 floats) and the list itself
   hbm_share       bytes / 7.7 TB/s (B200 data sheet HBM3e bandwidth) over kernel_us_cold
 """
-import argparse
-import copy
 import json
-import os
-import random
-import subprocess
-import sys
 
 import numpy as np
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-import __graft_entry__ as ge  # noqa: E402
+from probe_common import B, gpu_info, make_model
+from tcar_b200 import _native as nv, synth
 
-ge.load_package()
-from tcar_b200 import _native as nv, synth  # noqa: E402
-from tcar_b200.model_combine import Seq2SeqAttNN  # noqa: E402
-
-N_MIND, B = 103630, 512
+N_MIND = 103630
 HBM_BPS = 7.7e12
-
-
-def make_model(N, rank=0, world=1, seed=2020):
-    content, mwdhm, _ = synth.make_catalog(N, seed=seed)
-    np.random.seed(2020)
-    return Seq2SeqAttNN(dict(publish_time_MWDHM=mwdhm, itemnum=N, category_id=None, item_freq_dict_norm={},
-                             reverse_item=None, content_emb=content, emb_stddev=0.04, stddev=0.05, hidden_size=250,
-                             time_hidden_size=64, l2_emb=0.0, batch_size=B, epoch=1, neg_num=20, lr=0.001,
-                             max_grad=150, rank=rank, world_size=world, train_parallel="dp")), mwdhm
-
-
-def gpu_info():
-    idx = torch.cuda.current_device()
-    out = subprocess.run(["nvidia-smi", "-i", str(idx), "--query-gpu=power.limit", "--format=csv,noheader,nounits"],
-                         capture_output=True, text=True).stdout.strip()
-    return {"gpu": torch.cuda.get_device_name(idx), "power_limit_w": float(out) if out else None}
 
 
 def lists_for(rs, labels, lens):
@@ -131,40 +103,7 @@ def workload(model, mwdhm, T, fixed_len, info):
     print("rerank_probe " + json.dumps(res), flush=True)
 
 
-def check():
-    """test_impressions under torchrun (batch i on rank i mod world, sums all-reduced) == the same split on one GPU."""
-    import torch.distributed as dist
-    rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
-    gpus = torch.cuda.device_count()
-    torch.cuda.set_device(local % gpus)
-    if gpus >= world:
-        dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    else:                                                # ranks share a GPU: NCCL needs one GPU per rank, gloo does not
-        dist.init_process_group("gloo")
-    N = 20000
-    len_dict, sdict, tdict, item_dict, impr = synth.make_sessions(N, 3000, train=False, impressions="mind")
-    impr[0] = ["x1"]                                     # one session without a known negative: skipped
-    out = {}
-    for w in (world, 1):
-        model, _ = make_model(N, rank if w > 1 else 0, w, seed=3)
-        random.seed(7)                                   # same batches for both runs
-        out[w] = model.test_impressions(None, (copy.deepcopy(len_dict), sdict, tdict), impr, item_dict, {})
-    a, b = out[world], out[1]
-    same = a["sessions"] == b["sessions"] and a["skipped"] == b["skipped"] and \
-        all(abs(a[k] - b[k]) <= 1e-12 for k in ("auc", "mrr", "ndcg5", "ndcg10"))
-    print(f"rank {rank} rerank_check " + json.dumps(dict(gpu_info(), world=world, gpus=min(gpus, world),
-                                                         backend=dist.get_backend(), world_n=a, world_1=b, equal=same)),
-          flush=True)
-    dist.destroy_process_group()
-    if not same:
-        sys.exit(1)
-
-
 def main():
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--check", action="store_true")
-    if ap.parse_args().check:
-        return check()
     torch.cuda.set_device(0)
     info = gpu_info()
     model, mwdhm = make_model(N_MIND)
