@@ -146,6 +146,16 @@ int tcar_score_fwd_guarded(const void* q_bf16, const void* iext_bf16, const floa
                            float* rowsum_part, float* chunkmax, float* tilemax, float* rowmax_part, const float* rowmax,
                            int n_rows, int n_items, int n_pad, int mode, int cluster, void* stream);
 int tcar_score_fwd_tiles(int n_pad);
+/* Eval mode with a publish-time window per session row: item n is in the window of row b when
+ * win_lo[b] <= item_time[n] <= win_hi[b] (int32, any clock unit the caller uses for both; win_lo[b] > win_hi[b] is an
+ * empty window).  chunkmax / tilemax / rowsum_part as mode 1, except that an item outside the row's window counts as
+ * -inf, exactly as items >= n_items do: a chunk or tile without an in-window item has the maximum -inf, and an
+ * in-window chunk keeps the bit-exact mode-1 value.  item_time holds n_pad entries (those past n_items are not read as
+ * scores).  Always the CTA-pair kernel (score_fwd_pair_kernel<2>); tilemax is nullable.  The inputs of
+ * tcar_recommend_window. */
+int tcar_score_fwd_window(const void* q_bf16, const void* iext_bf16, const float* c_ref, float* rowsum_part,
+                          float* chunkmax, float* tilemax, const int32_t* item_time, const int32_t* win_lo,
+                          const int32_t* win_hi, int n_rows, int n_items, int n_pad, void* stream);
 
 /* (4a) softmax cross-entropy from the partial sums (model_combine.py:145): sumexp[b] = sum_tiles part,
  *      ce[b] = log(sumexp[b]) (because c_ref is the label score). Fixed summation order. */
@@ -566,6 +576,16 @@ int tcar_recommend(const float* chunkmax, const float* tilemax, const float* a_i
                    const float* content, const int32_t* mwdhm, const float* cat_stats, const int32_t* x_off,
                    const int32_t* x_ids, const int32_t* clicks, int T, int B, int N, int n_pad, int K, void* workspace,
                    int32_t* ids, float* scores, int32_t* rescored, void* stream);
+/* The same restricted to a publish-time window per session: the exact top-K, by (score desc, id asc), of the items
+ * with win_lo[b] <= item_time[n] <= win_hi[b] that are not excluded.  chunkmax / tilemax must come from
+ * tcar_score_fwd_window with the same item_time / win_lo / win_hi (the masked maxima keep the selection exact); the
+ * scores are the same exact fp32 scores as tcar_recommend's.  A window with fewer than K eligible items pads with
+ * -1 / -inf; rescored counts in-window items only.  Same workspace, limits and launches as tcar_recommend. */
+int tcar_recommend_window(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
+                          const float* item, const float* content, const int32_t* mwdhm, const float* cat_stats,
+                          const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B, int N,
+                          int n_pad, int K, void* workspace, int32_t* ids, float* scores, int32_t* rescored,
+                          const int32_t* item_time, const int32_t* win_lo, const int32_t* win_hi, void* stream);
 
 #ifdef __cplusplus
 }

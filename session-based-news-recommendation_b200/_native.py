@@ -40,6 +40,7 @@ SIGNATURES = {
     "tcar_score_fwd": [_P] * 7 + [_I] * 5 + [_P],
     "tcar_score_fwd_guarded": [_P] * 9 + [_I] * 5 + [_P],
     "tcar_score_fwd_tiles": [_I],
+    "tcar_score_fwd_window": [_P] * 9 + [_I] * 3 + [_P],
     "tcar_ce_finish": [_P] * 3 + [_I, _I, _P],
     "tcar_ce_finish_guarded": [_P] * 5 + [_I, _I, _I, _P],
     "tcar_neg_loss": [_P] * 9 + [_I, _I, _P],
@@ -106,6 +107,7 @@ SIGNATURES = {
     "tcar_rerank": [_P] * 8 + [_I] * 3 + [_P] * 4 + [_P],
     "tcar_recommend_ws_bytes": [_I],
     "tcar_recommend": [_P] * 11 + [_I] * 5 + [_P] * 4 + [_P],
+    "tcar_recommend_window": [_P] * 11 + [_I] * 5 + [_P] * 7 + [_P],
 }
 
 _lib = None

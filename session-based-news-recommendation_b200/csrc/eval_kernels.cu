@@ -1061,6 +1061,17 @@ rerank_kernel(const float* __restrict__ a_ic, const float* __restrict__ Tq, cons
 // top-K (ties included) scores >= s_K exactly, so its bf16 score is >= s_K - eps_b >= tau_b: its chunk is re-scored.
 // The order is the total order of rerank_key (score desc, id asc) and every item is re-scored by exactly one CTA, so
 // the order in which chunks are queued (shared-memory atomics) cannot change the result: reruns are bit-identical.
+//
+// With a publish-time window (tcar_recommend_window, behind tcar_score_fwd_window): item n is eligible for session b
+// only when win_lo[b] <= item_time[n] <= win_hi[b].  The GEMM epilogue gives out-of-window items the score -inf before
+// the chunk and tile maxima see them, exactly as it does for items >= N, so a finite chunk maximum is the bf16 score
+// of an in-window item of that chunk.  The argument above then carries over word for word with "valid" read as "< N
+// and in the window": the K' chunks with the largest masked maxima hold K' distinct in-window items scoring >= tau_hi.
+// When fewer than K' chunks hold an in-window item, the K'-th largest maximum is -inf: key_value(fkey(-inf)) = -inf,
+// so tau_b = -inf - 2 eps_b = -inf (never NaN or finite) and the scan visits every chunk that holds an in-window item.
+// The scan drops an out-of-window candidate beside excluded ids and ids >= N, before its rows are loaded, and skips
+// chunks and tiles whose masked maximum is -inf (they hold no in-window item).  An empty window therefore re-scores
+// nothing and returns -1 / -inf throughout.
 constexpr int RK = TCAR_RECOMMEND_MAXK;
 constexpr int RX = TCAR_RECOMMEND_MAXX;
 constexpr int TL_CAP = 4096;                     // tiles listed for the chunk-level selection (more: scan every tile)
@@ -1196,13 +1207,15 @@ __host__ __device__ constexpr size_t rec_keys_offset(int B) {
     return ((size_t)(TCAR_QROWS + (1 + WSPLIT) * B) * 4 + 7) / 8 * 8;
 }
 
+template <bool WINDOW>
 __global__ void __launch_bounds__(256, 2)
 recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* __restrict__ a_ic,
                       const float* __restrict__ Tq, const float* __restrict__ item, const float* __restrict__ content,
                       const int32_t* __restrict__ mwdhm, const int32_t* __restrict__ x_off,
                       const int32_t* __restrict__ x_ids, const int32_t* __restrict__ clicks, int n_clicks, int K, int N,
                       int n_pad, int B, char* wspace, int32_t* __restrict__ out_ids, float* __restrict__ out_scores,
-                      int32_t* __restrict__ rescored) {
+                      int32_t* __restrict__ rescored, const int32_t* __restrict__ item_time,
+                      const int32_t* __restrict__ win_lo, const int32_t* __restrict__ win_hi) {
     PDL_ENTER();
     __shared__ float s_aic[XW], s_tq[NB + 1];
     __shared__ int s_x[RX];
@@ -1248,6 +1261,7 @@ recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* 
         }
         return lo < nx && s_x[lo] == n;
     };
+    const int32_t w_lo = WINDOW ? win_lo[b] : 0, w_hi = WINDOW ? win_hi[b] : 0;
     const int nchunks = (N + CH - 1) / CH, ntiles = (N + 127) / 128;
     const float* cm = chunkmax + (size_t)b * (n_pad / CH);
     const float* tm = tilemax + (size_t)b * (n_pad / 128);
@@ -1257,7 +1271,8 @@ recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* 
     int cur = 0, my_cnt = 0;
     for (int t0 = t_lo; t0 < t_hi; t0 += 256) {
         const int tile = t0 + tid;
-        if (tile < t_hi && tm[tile] >= bound) {
+        // WINDOW: a chunk (tile) whose masked maximum is -inf holds no in-window item -- skipped even when bound = -inf
+        if (tile < t_hi && tm[tile] >= bound && (!WINDOW || tm[tile] > -INFINITY)) {
             float4 v[TILE_CH / 4];
 #pragma unroll
             for (int c = 0; c < TILE_CH / 4; ++c) v[c] = reinterpret_cast<const float4*>(cm + (size_t)tile * TILE_CH)[c];
@@ -1265,7 +1280,7 @@ recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* 
             for (int c = 0; c < TILE_CH; ++c) {
                 const int chunk = tile * TILE_CH + c;
                 const float cv = c % 4 == 0 ? v[c / 4].x : c % 4 == 1 ? v[c / 4].y : c % 4 == 2 ? v[c / 4].z : v[c / 4].w;
-                if (chunk < nchunks && cv >= bound) s_q[atomicAdd(&s_qn, 1)] = chunk;
+                if (chunk < nchunks && cv >= bound && (!WINDOW || cv > -INFINITY)) s_q[atomicAdd(&s_qn, 1)] = chunk;
             }
         }
         __syncthreads();
@@ -1277,15 +1292,20 @@ recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* 
             if (tid < P2) s_new[tid] = KEY_NONE;
             __syncthreads();
             for (int ci = w; ci < ncand; ci += 32) {
-                // four candidates per warp and iteration, branch-free, as in the widening pass; an excluded id or one
-                // >= N reads row 0 instead of its own
+                // four candidates per warp and iteration, branch-free, as in the widening pass; an excluded id, one
+                // >= N or (WINDOW) one outside the session's window reads row 0 instead of its own
                 int nn[4];
                 float sc[4];
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
                     const int cu = ci + 8 * u;
                     const int n = cu < ncand ? s_q[q0 + cu / CH] * CH + (cu % CH) : N;
-                    nn[u] = n < N && !excluded(n) ? n : -1;
+                    bool ok = n < N;
+                    if (WINDOW && ok) {
+                        const int32_t t = item_time[n];
+                        ok = w_lo <= t && t <= w_hi;
+                    }
+                    nn[u] = ok && !excluded(n) ? n : -1;
                 }
 #pragma unroll
                 for (int u = 0; u < 4; ++u)
@@ -1582,8 +1602,32 @@ extern "C" int tcar_recommend(const float* chunkmax, const float* tilemax, const
     cudaError_t e = launch_pdl(recommend_select_kernel, dim3(B), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq,
                                cat_stats, x_off, n_clicks, K, N, n_pad, reinterpret_cast<float*>(ws) + TCAR_QROWS);
     if (e != cudaSuccess) return (int)e;
-    launch_pdl(recommend_scan_kernel, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq, item,
-               content, mwdhm, x_off, x_ids, clicks, n_clicks, K, N, n_pad, B, ws, ids, scores, rescored);
+    launch_pdl(recommend_scan_kernel<false>, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq, item,
+               content, mwdhm, x_off, x_ids, clicks, n_clicks, K, N, n_pad, B, ws, ids, scores, rescored,
+               static_cast<const int32_t*>(nullptr), static_cast<const int32_t*>(nullptr),
+               static_cast<const int32_t*>(nullptr));
+    return (int)cudaGetLastError();
+}
+
+extern "C" int tcar_recommend_window(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
+                                     const float* item, const float* content, const int32_t* mwdhm,
+                                     const float* cat_stats, const int32_t* x_off, const int32_t* x_ids,
+                                     const int32_t* clicks, int T, int B, int N, int n_pad, int K, void* workspace,
+                                     int32_t* ids, float* scores, int32_t* rescored, const int32_t* item_time,
+                                     const int32_t* win_lo, const int32_t* win_hi, void* stream) {
+    if (B < 0 || B > TCAR_QROWS || N < 1 || n_pad < N || n_pad % 128 || K < 1 || K > RK ||
+        (clicks && (T < 1 || T > RX)) || !chunkmax || !tilemax || !a_ic || !Tq || !item || !content || !mwdhm ||
+        !cat_stats || (x_off && !x_ids) || !workspace || !ids || !scores || !item_time || !win_lo || !win_hi)
+        return TCAR_ERR_ARG;
+    if (B == 0) return 0;
+    const int n_clicks = clicks ? T : 0;
+    char* ws = static_cast<char*>(workspace);
+    cudaError_t e = launch_pdl(recommend_select_kernel, dim3(B), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq,
+                               cat_stats, x_off, n_clicks, K, N, n_pad, reinterpret_cast<float*>(ws) + TCAR_QROWS);
+    if (e != cudaSuccess) return (int)e;
+    launch_pdl(recommend_scan_kernel<true>, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq, item,
+               content, mwdhm, x_off, x_ids, clicks, n_clicks, K, N, n_pad, B, ws, ids, scores, rescored, item_time,
+               win_lo, win_hi);
     return (int)cudaGetLastError();
 }
 

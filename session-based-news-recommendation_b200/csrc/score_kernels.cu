@@ -58,8 +58,11 @@ struct FwdParams {
     int n_rows;             // valid sessions B
     int e_pitch;            // Npad
     int groups;             // number of session groups (ceil(ceil(B/128)/CL))
-    int mode;               // 0 = train, 1 = eval
+    int mode;               // 0 = train, 1 = eval, 2 = eval with a publish-time window per row (pair kernel only)
     int prefetch;           // pair kernel: L2 prefetch distance of the streamed item operand in stages (0 = off)
+    const int32_t* item_time;   // MODE 2: [e_pitch] time of every item
+    const int32_t* win_lo;      // MODE 2: [512] window of every row: item n is in row b's window when
+    const int32_t* win_hi;      //         win_lo[b] <= item_time[n] <= win_hi[b]; the others count as -inf
 };
 
 // exponent shift of one session row in log2 units: the label score, plus -- in pass 2 of the overflow guard -- the
@@ -285,15 +288,34 @@ constexpr int P_SMEM = F_A_BYTES + P_STAGES * P_B_STAGE + 1024 /*align*/ + 256 /
 
 // TAIL = false: every item of the chunk exists (all tiles but the last one or two) -- no per-element bounds logic, which
 // was half of the epilogue's instructions (2 ISETP + 2 PLOP3 + FSEL per element beside FFMA / MUFU / FMNMX / FADD).
+// MODE 2 (eval with a window): an item outside the row's window gets the score -inf before anything reads it, so it adds
+// exp(-inf) = 0 to the partial sum and nothing to the chunk / tile maxima, exactly like an item >= N.  The row's window
+// arrives as wlo = win_lo and wspan = win_hi - win_lo (uint32: t is inside iff t - wlo <= wspan, one IADD + one ISETP),
+// wempty = win_lo > win_hi.  The chunk's 32 item times are the same for every lane: eight warp-uniform 16-byte loads.
 template <int MODE, bool TAIL>
 __device__ __forceinline__ void fwd_epilogue_chunk_t(const uint32_t (&v)[32], const FwdParams& p, float cshift,
                                                      bool row_ok, bool store_ok, uint32_t row, int nb,
-                                                     float& psum, float& tmax, float& amax) {
+                                                     float& psum, float& tmax, float& amax, uint32_t wlo = 0,
+                                                     uint32_t wspan = 0, bool wempty = false) {
     constexpr bool tail = TAIL;
     float e[32];
+    float sm[32];                                            // MODE 2: the masked scores
+    if (MODE == 2) {
+        const int4* tp = reinterpret_cast<const int4*>(p.item_time + nb);
+#pragma unroll
+        for (int g = 0; g < 8; ++g) {
+            const int4 t = __ldg(tp + g);
+            const int tv[4] = {t.x, t.y, t.z, t.w};
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {
+                const bool out = wempty || (uint32_t)tv[c] - wlo > wspan;
+                sm[g * 4 + c] = out ? -INFINITY : __uint_as_float(v[g * 4 + c]);
+            }
+        }
+    }
 #pragma unroll
     for (int j = 0; j < 32; ++j) {
-        const float arg = fmaf(__uint_as_float(v[j]), kLog2e, -cshift);
+        const float arg = fmaf(MODE == 2 ? sm[j] : __uint_as_float(v[j]), kLog2e, -cshift);
         float ex = ex2_approx(arg);
         if (TAIL) {
             if (!row_ok || nb + j >= p.n_items) ex = 0.f;
@@ -327,7 +349,7 @@ __device__ __forceinline__ void fwd_epilogue_chunk_t(const uint32_t (&v)[32], co
             float mx = -INFINITY;
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
-                const float sv = __uint_as_float(v[g * 8 + j]);
+                const float sv = MODE == 2 ? sm[g * 8 + j] : __uint_as_float(v[g * 8 + j]);
                 const bool ok = !(tail && nb + g * 8 + j >= p.n_items);
                 mx = ok ? fmaxf(mx, sv) : mx;
             }
@@ -341,9 +363,12 @@ __device__ __forceinline__ void fwd_epilogue_chunk_t(const uint32_t (&v)[32], co
 template <int MODE>
 __device__ __forceinline__ void fwd_epilogue_chunk(const uint32_t (&v)[32], const FwdParams& p, float cshift,
                                                    bool row_ok, bool store_ok, bool tail, uint32_t row, int nb,
-                                                   float& psum, float& tmax, float& amax) {
-    if (tail) fwd_epilogue_chunk_t<MODE, true>(v, p, cshift, row_ok, store_ok, row, nb, psum, tmax, amax);
-    else fwd_epilogue_chunk_t<MODE, false>(v, p, cshift, row_ok, store_ok, row, nb, psum, tmax, amax);
+                                                   float& psum, float& tmax, float& amax, uint32_t wlo = 0,
+                                                   uint32_t wspan = 0, bool wempty = false) {
+    if (tail)
+        fwd_epilogue_chunk_t<MODE, true>(v, p, cshift, row_ok, store_ok, row, nb, psum, tmax, amax, wlo, wspan, wempty);
+    else
+        fwd_epilogue_chunk_t<MODE, false>(v, p, cshift, row_ok, store_ok, row, nb, psum, tmax, amax, wlo, wspan, wempty);
 }
 
 template <int MODE>
@@ -465,6 +490,14 @@ score_fwd_pair_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
         const bool row_ok = row < (uint32_t)p.n_rows;
         const bool store_ok = row < (((uint32_t)p.n_rows + 63u) & ~63u);
         const float cshift = row_ok ? exp_shift(p, row) : 0.f;
+        uint32_t wlo = 0, wspan = 0;
+        bool wempty = false;
+        if (MODE == 2 && row_ok) {                  // the row's window, loaded once
+            const int32_t lo = p.win_lo[row], hi = p.win_hi[row];
+            wlo = (uint32_t)lo;
+            wspan = (uint32_t)hi - (uint32_t)lo;
+            wempty = lo > hi;
+        }
         const uint32_t acc_empty_l = mapa_u32(acc_empty, 0);
         for (uint32_t it = 0; it < my_tiles; ++it) {
             const uint32_t acc = it % P_NACC;
@@ -480,23 +513,27 @@ score_fwd_pair_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
             tmem_ld32(taddr, va);
             tmem_ld_wait();
             tmem_ld32(taddr + 32, vb);
-            fwd_epilogue_chunk<MODE>(va, p, cshift, row_ok, store_ok, tail, row, n0, psum, tmax, amax);
+            fwd_epilogue_chunk<MODE>(va, p, cshift, row_ok, store_ok, tail, row, n0, psum, tmax, amax, wlo, wspan,
+                                     wempty);
             tmem_ld_wait();
             tmem_ld32(taddr + 64, va);
-            fwd_epilogue_chunk<MODE>(vb, p, cshift, row_ok, store_ok, tail, row, n0 + 32, psum, tmax, amax);
+            fwd_epilogue_chunk<MODE>(vb, p, cshift, row_ok, store_ok, tail, row, n0 + 32, psum, tmax, amax, wlo, wspan,
+                                     wempty);
             tmem_ld_wait();
             tmem_ld32(taddr + 96, vb);
-            fwd_epilogue_chunk<MODE>(va, p, cshift, row_ok, store_ok, tail, row, n0 + 64, psum, tmax, amax);
+            fwd_epilogue_chunk<MODE>(va, p, cshift, row_ok, store_ok, tail, row, n0 + 64, psum, tmax, amax, wlo, wspan,
+                                     wempty);
             tmem_ld_wait();
             // every TMEM read of this accumulator half is in registers -> hand it back to the MMA warp
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive_cluster(acc_empty_l + acc * 8);
-            fwd_epilogue_chunk<MODE>(vb, p, cshift, row_ok, store_ok, tail, row, n0 + 96, psum, tmax, amax);
+            fwd_epilogue_chunk<MODE>(vb, p, cshift, row_ok, store_ok, tail, row, n0 + 96, psum, tmax, amax, wlo, wspan,
+                                     wempty);
             if (row_ok) p.rowsum_part[(size_t)(tile * 2 + h) * QROWS + row] = psum;
             if (row_ok && p.rowmax_part)
-                p.rowmax_part[(size_t)(tile * 2 + h) * QROWS + row] = MODE == 1 ? fmaf(tmax, kLog2e, -cshift) : amax;
-            if (MODE == 1 && row_ok && p.tilemax) p.tilemax[(size_t)row * (p.e_pitch / 128) + tile * 2 + h] = tmax;
+                p.rowmax_part[(size_t)(tile * 2 + h) * QROWS + row] = MODE != 0 ? fmaf(tmax, kLog2e, -cshift) : amax;
+            if (MODE != 0 && row_ok && p.tilemax) p.tilemax[(size_t)row * (p.e_pitch / 128) + tile * 2 + h] = tmax;
         }
     }
 
@@ -1541,6 +1578,42 @@ extern "C" int tcar_score_fwd_guarded(const void* q_bf16, const void* iext_bf16,
     if (cluster == 1) return launch_fwd<1>(mq, mi, p, n_clusters, stream);
     if (cluster == 2) return launch_fwd<2>(mq, mi, p, n_clusters, stream);
     return launch_fwd<4>(mq, mi, p, n_clusters, stream);
+}
+
+// Eval mode with a publish-time window per row: score_fwd_pair_kernel<2>, whatever cluster setting the caller's model
+// uses for tcar_score_fwd (the pair kernel only needs n_pad % 256 == 0).
+extern "C" int tcar_score_fwd_window(const void* q_bf16, const void* iext_bf16, const float* c_ref, float* rowsum_part,
+                                     float* chunkmax, float* tilemax, const int32_t* item_time, const int32_t* win_lo,
+                                     const int32_t* win_hi, int n_rows, int n_items, int n_pad, void* stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    if (n_rows < 1 || n_rows > QROWS || n_items < 1 || n_pad % 256 != 0 || n_items > n_pad || !q_bf16 || !iext_bf16 ||
+        !c_ref || !rowsum_part || !chunkmax || !item_time || !win_lo || !win_hi)
+        return TCAR_ERR_ARG;
+    CUtensorMap mq, mi;
+    int rc = make_map_bf16(&mq, q_bf16, QROWS, KEXT, KEXT, BK, BM);
+    if (rc) return rc;
+    rc = make_map_bf16(&mi, iext_bf16, n_pad, KEXT, KEXT, BK, P_HALF);
+    if (rc) return rc;
+    FwdParams p = {};
+    p.rowsum_part = rowsum_part;
+    p.chunkmax = chunkmax;
+    p.tilemax = tilemax;
+    p.c_ref = c_ref;
+    p.n_items = n_items;
+    p.n_tiles = n_pad / P_BN;
+    p.n_rows = n_rows;
+    p.e_pitch = n_pad;
+    const int mtiles = (n_rows + BM - 1) / BM;
+    p.groups = (mtiles + 1) / 2;
+    p.mode = 2;
+    p.prefetch = tma_prefetch_depth(12, "TCAR_TMA_PREFETCH_FWD");
+    p.item_time = item_time;
+    p.win_lo = win_lo;
+    p.win_hi = win_hi;
+    int n_pairs = ((sm_count() / 2) / p.groups) * p.groups;
+    if (n_pairs < p.groups) n_pairs = p.groups;
+    if (n_pairs / p.groups > p.n_tiles) n_pairs = p.n_tiles * p.groups;
+    return launch_fwd_pair<2>(mq, mi, p, n_pairs, stream);
 }
 
 extern "C" int tcar_score_fwd_tiles(int n_pad) { return n_pad / F_BN; }

@@ -76,8 +76,26 @@ def recommend_k(text):
     return k
 
 
+def max_age_hours(text):
+    """--recommend_max_age_h: a float number of hours > 0."""
+    h = float(text)
+    if not h > 0:
+        raise argparse.ArgumentTypeError("must be > 0 hours")
+    return h
+
+
+class _Parser(argparse.ArgumentParser):
+    """Checks the flags that depend on one another right after parsing, before any data is loaded."""
+
+    def parse_args(self, args=None, namespace=None):
+        ns = super().parse_args(args, namespace)
+        if getattr(ns, "recommend_max_age_h", None) is not None and ns.recommend_k is None:
+            self.error("--recommend_max_age_h requires --recommend_k")
+        return ns
+
+
 def build_parser():
-    parser = argparse.ArgumentParser()
+    parser = _Parser()
     # DATASET PARAMETERS
     parser.add_argument("--datapath", default="./data/", type=str, help="Location of pre-processed dataset")
     parser.add_argument("--dataset", default="mind/TCAR-mid/", type=str, help="Dataset")
@@ -124,6 +142,9 @@ def build_parser():
     parser.add_argument("--recommend_k", default=None, type=recommend_k)
     # not a reference flag: leave a session's own clicked articles out of its recommendations
     parser.add_argument("--recommend_exclude_clicked", action="store_true")
+    # not a reference flag: recommend only articles published at most H hours before the session's last input click
+    # (the time-aware protocol: publish-time windows applied exactly on the device, Seq2SeqAttNN.recommend_split)
+    parser.add_argument("--recommend_max_age_h", default=None, type=max_age_hours)
     parser.add_argument("--inputdata", default="test", type=str)
     parser.add_argument("--threshold_acc", default=0.27, type=float)
     # additions

@@ -20,7 +20,7 @@ from . import parallel
 from .catalog_parallel import CatalogShardedTraining
 from .params import ParamStore, SMALL
 from .sampler import Sampler, pack_batch
-from .util import check_id_lists
+from .util import check_id_lists, check_item_times, check_windows
 
 H, TH, XW, PW, NB, KEXT, QROWS, TOPK = nv.H, nv.TH, nv.XW, nv.PW, nv.NBINS, nv.KEXT, nv.QROWS, nv.TOPK
 
@@ -1372,7 +1372,17 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         return m
 
     # ------------------------------------------------------------------------------------------- top-K recommendation
-    def recommend(self, bt, k=20, exclude_off=None, exclude_ids=None, exclude_clicked=False):
+    def set_item_times(self, times):
+        """One time per item for recommend(window=...): N integers of any integer type, each within int32, in whatever
+        clock unit the windows use (recommend_split: minutes since the epoch).  Checked on the host (ValueError, nothing
+        uploaded), then copied once to an int32 [n_pad] device buffer; may be called again at any time, e.g. to
+        withdraw an article by giving it a time no window reaches."""
+        t = check_item_times(times, self.N)
+        if getattr(self, "_item_time", None) is None:
+            self._item_time = torch.zeros(self.ps.n_pad, device=self.dev, dtype=torch.int32)
+        self._item_time[:self.N].copy_(torch.from_numpy(t))
+
+    def recommend(self, bt, k=20, exclude_off=None, exclude_ids=None, exclude_clicked=False, window=None):
         """The exact top-k of the whole catalog for every session of bt (tcar_recommend), 1 <= k <= nv.RECOMMEND_MAXK,
         ordered by (score desc, id asc).  Scores are the exact fp32 scores of the full-catalog evaluation: with k <= 20
         and no exclusions the result is the prefix of eval_step's top-20, and an item scores bit for bit what eval_step
@@ -1386,7 +1396,13 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         Returns device tensors (ids [B, k] int32, scores [B, k] fp32); a catalog of fewer than k eligible items pads
         with -1 / -inf.  The number of items each session re-scored exactly is left in self.rec_rescored[:B].
         bt.label plays no part in the result (the session forward reads it, so a serving caller fills it with any
-        valid item id)."""
+        valid item id).
+
+        Publish-time window: window = (lo, hi), host arrays of B integers within int32, lo[b] <= hi[b], restricts
+        session b to the items with lo[b] <= t[n] <= hi[b], t = the times of set_item_times (same clock unit).  The
+        result is the exact top-k of the in-window, non-excluded items, with the same exact scores; a window with fewer
+        than k of them pads with -1 / -inf.  The mask sits in the scoring GEMM's epilogue (tcar_score_fwd_window,
+        tcar_recommend_window), so the selection stays exact however few items a window holds."""
         if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= nv.RECOMMEND_MAXK:
             raise ValueError(f"k must be an integer in [1, TCAR_RECOMMEND_MAXK = {nv.RECOMMEND_MAXK}], got {k!r}")
         if (exclude_off is None) != (exclude_ids is None):
@@ -1400,6 +1416,11 @@ class Seq2SeqAttNN(CatalogShardedTraining):
                                      limit_name="TCAR_RECOMMEND_MAXX", extra=extra)
         elif extra > nv.RECOMMEND_MAXX:
             raise ValueError(f"session 0: more than TCAR_RECOMMEND_MAXX = {nv.RECOMMEND_MAXX} clicks")
+        win = None
+        if window is not None:
+            if getattr(self, "_item_time", None) is None:
+                raise ValueError("window needs item times: call set_item_times first")
+            win = check_windows(window, B)
         dev, p, ps = self.dev, nv.ptr, self.ps
         out_ids = torch.empty(B, k, device=dev, dtype=torch.int32)
         out_sc = torch.empty(B, k, device=dev)
@@ -1414,6 +1435,8 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         self._session_forward(bt)
         self._ensure_cat_stats()
         ws = self._score_buffers(ps.n_pad, False)
+        if win is not None:
+            return self._recommend_window(bt, k, host, exclude_clicked, win, out_ids, out_sc)
         # one unguarded eval-mode GEMM for the chunk / tile maxima; its softmax partial sums (which may overflow without
         # the guard) are not read
         nv.counted_call("tcar_score_fwd", 1, p(self.Q), p(ps.iext), p(self.c_ref), None, p(ws["part"]), p(ws["cmax"]),
@@ -1425,6 +1448,22 @@ class Seq2SeqAttNN(CatalogShardedTraining):
                         N, ps.n_pad, k, p(self._rec_ws), p(out_ids), p(out_sc), p(self.rec_rescored))
         return out_ids, out_sc
 
+    def _recommend_window(self, bt, k, host, exclude_clicked, win, out_ids, out_sc):
+        """recommend() with checked windows win = int32 [lo | hi]: the windowed GEMM (masked chunk / tile maxima), then
+        the windowed selection and scan.  The windows go up through the pinned ring like the exclusion lists."""
+        B, N, p, ps = bt.B, self.N, nv.ptr, self.ps
+        ws = self._score_buffers(ps.n_pad, False)
+        wv = self._stage_ints(win)
+        nv.counted_call("tcar_score_fwd_window", 1, p(self.Q), p(ps.iext), p(self.c_ref), p(ws["part"]), p(ws["cmax"]),
+                        p(ws["tmax"]), p(self._item_time), p(wv), p(wv[B:]), B, N, ps.n_pad)
+        csr = self._stage_ints(host) if host is not None else None
+        nv.counted_call("tcar_recommend_window", 2, p(ws["cmax"]), p(ws["tmax"]), p(self.a_ic), p(self.Tq),
+                        p(ps.item), p(ps.content), p(ps.mwdhm), p(self.cat_stats), p(csr),
+                        p(csr[B + 1:]) if csr is not None else None, p(bt.seq) if exclude_clicked else None, bt.T, B,
+                        N, ps.n_pad, k, p(self._rec_ws), p(out_ids), p(out_sc), p(self.rec_rescored),
+                        p(self._item_time), p(wv), p(wv[B:]))
+        return out_ids, out_sc
+
     def recommend_split(self, sess, test_data, item_dict, args):
         """Recommend the top-K articles (args["recommend_k"], default 20) for every session of a split, optionally
         without the session's own clicks (args["recommend_exclude_clicked"]), in the batches test() uses.  Writes one
@@ -1432,41 +1471,68 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         `article:score` pairs with the original article ids) and prints and returns {"hr", "mrr", "ndcg", "sessions"}
         @K, where a session's rank is its label's 1-based position in the returned list (ties go to the lower id).
         Under torchrun batch i goes to rank i mod world (each rank writes its own file) and the sums are all-reduced,
-        so every rank returns the metrics of the whole split."""
-        from .util import label_positions, recommend_line, topk_metrics, topk_sums
+        so every rank returns the metrics of the whole split.
+
+        args["recommend_max_age_h"] = H > 0 (hours) restricts every session to the articles published in
+        [t_req - round(60 H) min, t_req], t_req = the click time of its last input click (util.session_windows): the
+        time-aware protocol, which never recommends an article published after the request.  Article times are
+        args["publish_time"] (one datetime per item, main.load_datas) in minutes since the epoch.  Then the result
+        also holds "label_outside": the sessions whose label was published outside their window (never a hit)."""
+        from .util import (count_outside, epoch_minutes, label_positions, recommend_line, session_windows, topk_metrics,
+                           topk_sums)
         k = int(args.get("recommend_k") or 20)
         clicked = bool(args.get("recommend_exclude_clicked"))
-        print("Recommending the top-{} articles{}...".format(k, " without the clicked ones" if clicked else ""))
+        max_age = args.get("recommend_max_age_h")
+        windowed = max_age is not None
+        if windowed:
+            if not float(max_age) > 0:
+                raise ValueError(f"recommend_max_age_h must be > 0 hours, got {max_age!r}")
+            if args.get("publish_time") is None:
+                raise ValueError("recommend_max_age_h needs every article's publish time in args['publish_time']")
+            item_time = epoch_minutes(args["publish_time"])
+            self.set_item_times(item_time)
+            max_age_min = int(round(60 * float(max_age)))
+        print("Recommending the top-{} articles{}{}...".format(
+            k, " without the clicked ones" if clicked else "",
+            " published at most {} h before the request".format(max_age) if windowed else ""))
         self.sync_item_table()
         session_dict_test = test_data[1]
         reverse = self.reverse_item if self.reverse_item is not None else \
             {cnt - 1: art for art, cnt in item_dict.items()}
         sampler = self._eval_sampler(test_data)
         keys = list(sampler.session_id_batches)
+        # this rank's windows up front, so that the producer thread does no dictionary work per batch
+        wins = [session_windows(kb, test_data[2], max_age_min) for kb in keys] if windowed else [None] * len(keys)
         os.makedirs("saved", exist_ok=True)
         dist_on = parallel.is_distributed(self.world)
         path = "saved/recommend_{}{}.txt".format(args.get("foldnum", 0), "_rank{}".format(self.rank) if dist_on else "")
-        sums = np.zeros(4)
+        sums = np.zeros(5 if windowed else 4)
 
         def launch(cur, nxt):
-            bt, kb = cur
-            ids, sc = self.recommend(bt, k, exclude_clicked=clicked)
-            return kb, self.fetch_async(ids), self.fetch_async(sc)
+            bt, (kb, win) = cur
+            ids, sc = self.recommend(bt, k, exclude_clicked=clicked, window=win)
+            return kb, win, self.fetch_async(ids), self.fetch_async(sc)
 
-        def consume(kb, ids_h, sc_h):
+        def consume(kb, win, ids_h, sc_h):
             ids, sc = ids_h.get().numpy(), sc_h.get().numpy()
             labels = [session_dict_test[key][-1] - 1 for key in kb]
-            sums[:] += topk_sums(label_positions(ids, labels))
+            sums[:4] += topk_sums(label_positions(ids, labels))
+            if windowed:
+                sums[4] += count_outside(item_time[labels], *win)
             f.writelines(recommend_line(key, ids[b], sc[b], reverse) for b, key in enumerate(kb))
 
         with open(path, "w") as f:
             pipelined(zip((self.stage_to_device(packed, B, T, Nn) for packed, B, T, Nn in prefetch_packed(sampler)),
-                          keys), launch, consume)
-        m = topk_metrics(self._sum_over_ranks(sums))
+                          zip(keys, wins)), launch, consume)
+        total = self._sum_over_ranks(sums)
+        m = topk_metrics(total[:4])
+        if windowed:
+            m["label_outside"] = int(total[4])
         self.last_recommend_metrics = m
         self.last_recommend_path = path
-        print("Recommend: HR@{k}: {}, MRR@{k}: {}, nDCG@{k}: {} ({} sessions, written to {})".format(
-            m["hr"], m["mrr"], m["ndcg"], m["sessions"], path, k=k))
+        print("Recommend: HR@{k}: {}, MRR@{k}: {}, nDCG@{k}: {} ({} sessions{}, written to {})".format(
+            m["hr"], m["mrr"], m["ndcg"], m["sessions"],
+            ", {} labels published outside their window".format(m["label_outside"]) if windowed else "", path, k=k))
         return m
 
     # ------------------------------------------------------------------------------------------- metrics

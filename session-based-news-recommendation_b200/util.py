@@ -1,5 +1,6 @@
 """Host utilities mirroring the reference's util.py: data_partition (pickle loader, util.py:20-57), cau_metrics
 (util.py:8-18), save_model (util.py:102-106; the reference version is broken -- stray `self`, wrong key)."""
+import datetime
 import os
 import pickle
 import time
@@ -107,6 +108,70 @@ def check_id_lists(off, ids, B, N, *, names, nouns, limit, limit_name, extra=0):
     host = np.empty(B + 1 + ids.shape[0], dtype=np.int32)
     host[:B + 1], host[B + 1:] = off, ids
     return host, int(lens.max()) if B else 0
+
+
+INT32_MIN, INT32_MAX = -2 ** 31, 2 ** 31 - 1
+_EPOCH = datetime.datetime(1970, 1, 1)
+_EPOCH_UTC = _EPOCH.replace(tzinfo=datetime.timezone.utc)
+_MINUTE = datetime.timedelta(minutes=1)
+
+
+def epoch_minutes(datetimes):
+    """datetime objects -> int64 whole minutes since 1970-01-01 00:00 (floor: seconds are dropped, so a click and an
+    article of the same minute compare equal).  Naive datetimes are read as UTC, aware ones converted."""
+    return np.array([(d - (_EPOCH if d.tzinfo is None else _EPOCH_UTC)) // _MINUTE for d in datetimes],
+                    dtype=np.int64)
+
+
+def check_item_times(times, N):
+    """Validate one time per item before anything is uploaded: N integers of any integer type, each within int32.
+    Returns them as an int32 host array; raises ValueError naming the first bad item."""
+    t = np.asarray(times).reshape(-1)
+    if t.size and t.dtype.kind not in "iu":
+        raise ValueError("item times must be integers")
+    if t.shape[0] != N:
+        raise ValueError(f"item times must hold N = {N} values, got {t.shape[0]}")
+    if N and (t.min() < INT32_MIN or t.max() > INT32_MAX):
+        n = int(np.argmax((t < INT32_MIN) | (t > INT32_MAX)))
+        raise ValueError(f"item {n}: time {int(t[n])} outside int32")
+    return t.astype(np.int32)
+
+
+def check_windows(window, B):
+    """Validate the publish-time windows (lo, hi) of B sessions before anything is launched: two host arrays of B
+    integers each within int32, lo[b] <= hi[b].  Returns the int32 host array [lo | hi] the kernels read; raises
+    ValueError naming the first bad session."""
+    if not isinstance(window, (tuple, list)) or len(window) != 2:
+        raise ValueError("window must be a pair (lo, hi) of arrays of B integers")
+    lo, hi = (np.asarray(w).reshape(-1) for w in window)
+    for name, w in (("lo", lo), ("hi", hi)):
+        if w.size and w.dtype.kind not in "iu":
+            raise ValueError(f"window {name} must hold integers")
+        if w.shape[0] != B:
+            raise ValueError(f"window {name} must hold B = {B} values, got {w.shape[0]}")
+        if B and (w.min() < INT32_MIN or w.max() > INT32_MAX):
+            b = int(np.argmax((w < INT32_MIN) | (w > INT32_MAX)))
+            raise ValueError(f"session {b}: window {name} {int(w[b])} outside int32")
+    if B and (lo.astype(np.int64) > hi.astype(np.int64)).any():
+        b = int(np.argmax(lo.astype(np.int64) > hi.astype(np.int64)))
+        raise ValueError(f"session {b}: window lo {int(lo[b])} > hi {int(hi[b])}")
+    out = np.empty(2 * B, dtype=np.int32)
+    out[:B], out[B:] = lo, hi
+    return out
+
+
+def session_windows(keys, session_time_dict, max_age_min):
+    """Publish-time windows of a batch's sessions (keys in batch order) for recommend(window=...): [t_req - max_age_min,
+    t_req] in epoch minutes, t_req = the click_t of the session's last input click (session_time_dict[key][-2], the
+    click the sampler takes the request context from).  Returns int64 arrays (lo, hi)."""
+    hi = epoch_minutes([session_time_dict[k][-2]["click_t"] for k in keys])
+    return hi - int(max_age_min), hi
+
+
+def count_outside(times, lo, hi):
+    """Number of sessions whose time (e.g. their label's publish time) lies outside their window [lo, hi]."""
+    t = np.asarray(times, dtype=np.int64)
+    return int(((t < np.asarray(lo)) | (t > np.asarray(hi))).sum())
 
 
 def _load(path):

@@ -3,6 +3,7 @@ shape (364 047 items) and the MIND shape (103 630 items), 512 sessions per batch
 with and without the session's own clicks excluded.
 
     python tools/recommend_probe.py [--shapes globo,mind]
+    python tools/recommend_probe.py --window [--shapes globo,mind]
 
 recommend_split across ranks is checked by tools/split_check.py.
 
@@ -15,6 +16,16 @@ Per workload:
   eval_step_us                    Seq2SeqAttNN.eval_step per batch on the same batches (the certified top-20)
   ratio                           recommend_us / eval_step_us
   rescored_mean / rescored_max    items re-scored exactly per query (the width of the error band)
+
+--window: publish-time windows (tcar_score_fwd_window / tcar_recommend_window) instead, one JSON line per shape,
+window width (100 %, 10 %, 1 %, 0.05 % of the catalog: item times are a random permutation of 0 .. N-1, every session
+its own window of that many consecutive times) and K in {20, 100}, T = 1, no exclusions:
+  gemm_mode1_us_cold / gemm_window_us_cold   score_fwd_pair_kernel<1> / <2> alone (torch.profiler), the L2
+                                             overwritten before each call; gemm_ratio = window / mode 1
+  recommend_us / recommend_window_us         Seq2SeqAttNN.recommend without / with the window per batch (CUDA events
+                                             over 32 batches); ratio = window / none
+  rescored_mean / rescored_max               items re-scored exactly per query with the window (rescored_nowin_mean:
+                                             without)
 """
 import argparse
 import json
@@ -91,15 +102,91 @@ def workload(model, mwdhm, shape, T, K, clicked, info, flush):
     print("recommend_probe " + json.dumps(res), flush=True)
 
 
+def gemm_times(model, bt, wins, flush):
+    """Mean device time of score_fwd_pair_kernel<1> and <2> over 20 calls each on bt's queries, cold L2."""
+    from torch.profiler import ProfilerActivity, profile
+    model.recommend(bt, 20)                                 # leaves bt's session vectors in place
+    ps, p = model.ps, nv.ptr
+    ws = model._score_buffers(ps.n_pad, False)
+    wv = torch.from_numpy(np.concatenate(wins).astype(np.int32)).cuda()
+    calls = (("tcar_score_fwd", p(model.Q), p(ps.iext), p(model.c_ref), None, p(ws["part"]), p(ws["cmax"]),
+              p(ws["tmax"]), B, ps.N, ps.n_pad, 1, nv.CLUSTER_PAIR),
+             ("tcar_score_fwd_window", p(model.Q), p(ps.iext), p(model.c_ref), p(ws["part"]), p(ws["cmax"]),
+              p(ws["tmax"]), p(model._item_time), p(wv), p(wv[B:]), B, ps.N, ps.n_pad))
+    for c in calls:
+        nv.call(*c)
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(20):
+            for c in calls:
+                flush.zero_()
+                nv.call(*c)
+        torch.cuda.synchronize()
+    out = {}
+    for e in prof.key_averages():
+        for mode in (1, 2):
+            if f"score_fwd_pair_kernel<{mode}>" in e.key:
+                out[mode] = e.device_time_total / e.count
+    return out[1], out[2]
+
+
+def window_workloads(model, mwdhm, shape, info, flush):
+    N = model.N
+    rs = np.random.RandomState(5)
+    model.set_item_times(rs.permutation(N))
+    bts = []
+    for i in range(4):
+        packed = synth.make_index_batch(N, B, 1, 0, mwdhm, seed=100 + i)
+        bts.append(model.to_device(torch.from_numpy(packed).pin_memory(), B, 1, 0))
+    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    KB = 32
+    for frac in (1.0, 0.1, 0.01, 0.0005):
+        width = max(1, int(round(frac * N)))
+        wins = []
+        for _ in range(4):
+            lo = rs.randint(0, N - width + 1, B)
+            wins.append((lo, lo + width - 1))
+        g1, g2 = gemm_times(model, bts[0], wins[0], flush)
+        for K in (20, 100):
+            resc, resc0 = [], []
+            for bt, w in zip(bts, wins):
+                model.recommend(bt, K)
+                resc0.append(model.rec_rescored[:B].cpu().numpy())
+                model.recommend(bt, K, window=w)
+                resc.append(model.rec_rescored[:B].cpu().numpy())
+            resc, resc0 = np.concatenate(resc), np.concatenate(resc0)
+            times = {}
+            for name, kw in (("none", lambda i: {}), ("window", lambda i: {"window": wins[i % 4]})):
+                t0.record()
+                for i in range(KB):
+                    model.recommend(bts[i % 4], K, **kw(i))
+                t1.record()
+                torch.cuda.synchronize()
+                times[name] = t0.elapsed_time(t1) / KB * 1e3
+            res = dict(info, workload=f"{shape} N={N} B={B} T=1 K={K} window={frac:g}", N=N, B=B, T=1, K=K,
+                       window_frac=frac, window_items=width, gemm_mode1_us_cold=round(g1, 2),
+                       gemm_window_us_cold=round(g2, 2), gemm_ratio=round(g2 / g1, 3),
+                       recommend_us=round(times["none"], 1), recommend_window_us=round(times["window"], 1),
+                       ratio=round(times["window"] / times["none"], 3), rescored_mean=round(float(resc.mean()), 1),
+                       rescored_max=int(resc.max()), rescored_nowin_mean=round(float(resc0.mean()), 1))
+            print("recommend_probe_window " + json.dumps(res), flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--shapes", default="globo,mind")
+    ap.add_argument("--window", action="store_true", help="publish-time windows (see the module docstring)")
     a = ap.parse_args()
     torch.cuda.set_device(0)
     info = gpu_info()
     flush = torch.empty(256 << 20, device="cuda", dtype=torch.uint8)
     for shape in a.shapes.split(","):
         model, mwdhm = make_model(SHAPES[shape])
+        if a.window:
+            window_workloads(model, mwdhm, shape, info, flush)
+            del model
+            torch.cuda.empty_cache()
+            continue
         for T in (1, 20):
             for K in (20, 100, 256):
                 for clicked in (False, True):

@@ -1,6 +1,6 @@
 """Run under torchrun: the split walkers of Seq2SeqAttNN -- test() (catalog-sharded eval_round, one round per `world`
-batches), test_impressions() and recommend_split() (batch i on rank i mod world) -- on one synthetic split at world N
-equal the same walkers at world 1.
+batches), test_impressions() and recommend_split() (batch i on rank i mod world; once more with 24 h publish-time
+windows) -- on one synthetic split at world N equal the same walkers at world 1.
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29513 \\
         tools/split_check.py
@@ -11,12 +11,14 @@ equal, and the ranks' recommend_split files together hold line for line the sing
 per rank and exits with status 1 on a mismatch.
 """
 import copy
+import datetime
 import json
 import os
 import random
 import sys
 import tempfile
 
+import numpy as np
 import torch.distributed as dist
 
 from probe_common import gpu_info, init_torchrun, make_model
@@ -25,14 +27,27 @@ from tcar_b200 import synth
 N, SESSIONS, K = 20000, 3000, 100
 
 
+def publish_times(n):
+    """Article publish times over the sessions' two weeks (synth.make_sessions: clicks from day 31 to 45 after
+    2017-10-01), so that a 24 h window holds a few percent of the catalog."""
+    rs = np.random.RandomState(11)
+    t0 = datetime.datetime(2017, 10, 1) + datetime.timedelta(days=30)
+    return [t0 + datetime.timedelta(minutes=int(m)) for m in rs.randint(0, 60 * 24 * 16, n)]
+
+
 def run_walkers(model, split, impressions, item_dict):
-    """The three walkers on the same batches (Sampler shuffles len_dict in place and draws from `random`)."""
+    """The walkers on the same batches (Sampler shuffles len_dict in place and draws from `random`); recommend_split
+    also with 24 h publish-time windows (written to recommend_1*.txt)."""
     def fresh():
         random.seed(7)
         return (copy.deepcopy(split[0]), *split[1:])
     out = {"impressions": model.test_impressions(None, fresh(), impressions, item_dict, {}),
            "recommend": model.recommend_split(None, fresh(), item_dict,
-                                              {"recommend_k": K, "recommend_exclude_clicked": True, "foldnum": 0})}
+                                              {"recommend_k": K, "recommend_exclude_clicked": True, "foldnum": 0}),
+           "recommend_window": model.recommend_split(None, fresh(), item_dict,
+                                                     {"recommend_k": K, "recommend_exclude_clicked": True,
+                                                      "recommend_max_age_h": 24.0, "publish_time": publish_times(N),
+                                                      "foldnum": 1})}
     model.test(None, fresh(), {})
     out["test"] = model.last_metrics
     return out
@@ -59,16 +74,24 @@ def main():
         res[w] = run_walkers(model, (len_dict, sdict, tdict), impr, item_dict)
         dist.barrier()
     a, b = res[world], res[1]
-    lines_n = []
-    for r in range(world):
-        with open(os.path.join(base, f"world{world}", f"saved/recommend_0_rank{r}.txt")) as f:
-            lines_n += f.read().splitlines()
-    with open(os.path.join(base, f"world1_rank{rank}", "saved/recommend_0.txt")) as f:
-        lines_1 = f.read().splitlines()
+
+    def lines(fold):
+        n = []
+        for r in range(world):
+            with open(os.path.join(base, f"world{world}", f"saved/recommend_{fold}_rank{r}.txt")) as f:
+                n += f.read().splitlines()
+        with open(os.path.join(base, f"world1_rank{rank}", f"saved/recommend_{fold}.txt")) as f:
+            return n, f.read().splitlines()
+    lines_n, lines_1 = lines(0)
+    win_n, win_1 = lines(1)
     equal = {"test": close(a["test"], b["test"], exact=("coverage",), rel=("loss",)),
              "impressions": close(a["impressions"], b["impressions"], exact=("sessions", "skipped")),
              "recommend": close(a["recommend"], b["recommend"], exact=("sessions",)),
-             "recommend_files": sorted(lines_n) == sorted(lines_1) and len(lines_1) == b["recommend"]["sessions"]}
+             "recommend_files": sorted(lines_n) == sorted(lines_1) and len(lines_1) == b["recommend"]["sessions"],
+             "recommend_window": close(a["recommend_window"], b["recommend_window"],
+                                       exact=("sessions", "label_outside")),
+             "recommend_window_files": sorted(win_n) == sorted(win_1) and
+             len(win_1) == b["recommend_window"]["sessions"]}
     ok = all(equal.values())
     print(f"rank {rank} split_check " + json.dumps(dict(gpu_info(), world=world, gpus=gpus, backend=dist.get_backend(),
                                                         sessions=SESSIONS, K=K, exclude_clicked=True, world_n=a,
