@@ -586,6 +586,26 @@ int tcar_recommend_window(const float* chunkmax, const float* tilemax, const flo
                           const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B, int N,
                           int n_pad, int K, void* workspace, int32_t* ids, float* scores, int32_t* rescored,
                           const int32_t* item_time, const int32_t* win_lo, const int32_t* win_hi, void* stream);
+/* The same with at most C items of one category and a per-session set of allowed categories: the exact top-K, by
+ * (score desc, id asc), of the non-excluded items of the allowed categories, in which an item that has C better items
+ * of its category in the list is left out (C >= K: no cap).  G <= TCAR_RECOMMEND_MAXG categories, item_cat [N] the
+ * code in [0, G) of every (original) item id.  The catalog in category order: perm [N'] the original id at position p
+ * (-1 on a pad), every category padded to whole TCAR_CHUNK chunks by repeating its last item; category g owns the
+ * chunks cat_chunk_off[g] .. cat_chunk_off[g + 1] (cat_chunk_off [G + 1], cat_chunk_off[G] = N' / TCAR_CHUNK).
+ * chunkmax: tcar_score_fwd mode 1 over iext_cat (row p = the iext row of perm[p], a pad's that of the item it repeats)
+ * with n_items = N' and this n_pad.  Allowed codes of session b: a_codes[a_off[b] .. a_off[b + 1]) (in [0, G),
+ * duplicates allowed; an empty list returns -1 / -inf throughout); a_off == NULL allows every category.  Exclusions,
+ * outputs and limits as tcar_recommend (ids are original ids; rescored counts items scored exactly).  workspace:
+ * tcar_recommend_category_ws_bytes(B) bytes, ZERO before the first call (tcar_recommend's layout, then per-category
+ * thresholds).  Two launches; B = 0 launches nothing. */
+#define TCAR_RECOMMEND_MAXG 1024
+long long tcar_recommend_category_ws_bytes(int B);
+int tcar_recommend_category(const float* chunkmax, const float* a_ic, const float* Tq, const float* item,
+                            const float* content, const int32_t* mwdhm, const float* cat_stats, const int32_t* x_off,
+                            const int32_t* x_ids, const int32_t* clicks, int T, int B, int n_pad, int K,
+                            const int32_t* perm, const int32_t* item_cat, const int32_t* cat_chunk_off, int G,
+                            const int32_t* a_off, const int32_t* a_codes, int C, void* workspace, int32_t* ids,
+                            float* scores, int32_t* rescored, void* stream);
 
 #ifdef __cplusplus
 }

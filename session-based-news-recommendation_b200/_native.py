@@ -24,6 +24,7 @@ CLUSTER_PAIR = -2      # TCAR_CLUSTER_PAIR: tcar_score_fwd with tcgen05.mma.cta_
 RERANK_MAXL = 2048     # TCAR_RERANK_MAXL: longest candidate list of tcar_rerank
 RECOMMEND_MAXK = 256   # TCAR_RECOMMEND_MAXK: largest K of tcar_recommend
 RECOMMEND_MAXX = 1024  # TCAR_RECOMMEND_MAXX: exclusion entries per session of tcar_recommend, clicks included
+RECOMMEND_MAXG = 1024  # TCAR_RECOMMEND_MAXG: most categories of tcar_recommend_category
 
 _P, _I, _F, _LL = C.c_void_p, C.c_int, C.c_float, C.c_longlong
 
@@ -108,6 +109,8 @@ SIGNATURES = {
     "tcar_recommend_ws_bytes": [_I],
     "tcar_recommend": [_P] * 11 + [_I] * 5 + [_P] * 4 + [_P],
     "tcar_recommend_window": [_P] * 11 + [_I] * 5 + [_P] * 7 + [_P],
+    "tcar_recommend_category_ws_bytes": [_I],
+    "tcar_recommend_category": [_P] * 10 + [_I] * 4 + [_P] * 3 + [_I] + [_P] * 2 + [_I] + [_P] * 4 + [_P],
 }
 
 _lib = None

@@ -1368,6 +1368,429 @@ recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* 
     }
 }
 
+// ------------------------------------------------------------------------- top-K recommendation by category (§4.9)
+// The exact top-K per session with at most C items of one category and only the session's allowed categories, behind
+// the unchanged eval-mode scoring GEMM run on iext_cat: the scoring operand with its rows ordered by (category, id) and
+// every category padded to whole chunks by repeating its last row (perm[p] = the original id at position p, -1 on a
+// pad; category g owns the chunks cat_chunk_off[g] .. cat_chunk_off[g + 1]).  Every chunk maximum is then the bf16
+// score of a real item of exactly one category, and distinct chunks hold distinct items.
+//   select  one CTA per query: K' = K + x_b; M = from each allowed category g the min(C, .) largest chunk maxima of g;
+//           v = the K'-th largest of M, tau_b = v - 2 eps_b.  When |M| <= K' (few categories times a small C) there is
+//           no such v: tau_b = -inf, and with a cap every allowed category g gets its own threshold tau_g = its
+//           (C + x_b)-th largest chunk maximum - 2 eps_b (-inf when it has no more chunks): those chunks hold C + x_b
+//           distinct items of g scoring >= tau_g + eps_b exactly, at most x_b are excluded, so g's eligible top-C (which
+//           holds every member of the answer from g) scores >= tau_g + eps_b and lies in chunks >= tau_g.  Without a cap
+//           (C >= K) v is the
+//           K'-th largest allowed chunk maximum (block_kth_key).  With a cap, count(x) = sum_g min(C, #{chunks of g
+//           >= x}) is monotone in x and v = the largest x with count(x) >= K', found bit by bit over the 32-bit fkey;
+//           count runs over the allowed chunks at or above the CL_CAP-th largest when those are listed in shared memory
+//           and already give count >= K' (the usual case), else over every allowed chunk.
+//   scan    TCAR_WIDEN_SPLITS CTAs per query over the allowed chunks, balanced by chunk count: chunks below
+//           max(tau_b, tau_g) are skipped, a position's original id is read from perm and pads and excluded ids are dropped before any row
+//           is loaded, the rest are scored exactly on their ORIGINAL rows (exact_score_e: bit for bit the scores of
+//           tcar_recommend and eval_step) and merged into a running capped top-K: after each sorted merge an entry
+//           with C earlier entries of its category is dropped, then the first K are kept.  The last split CTA merges
+//           the partial lists the same way (a category may span two splits, so the cap is applied there too).
+// Why the result is exact: the K' largest entries of M are K' distinct items, at most C per category, each scoring
+// >= v - eps_b exactly.  At most x_b are excluded, so at least K eligible items remain, still <= C per category.  A
+// category holding k_g of them has an eligible top-C holding >= k_g items >= v - eps_b, so the union U of the
+// per-category top-C has >= K items >= v - eps_b; the capped answer is the top-K of U, so its K-th score s* >= v - eps_b
+// and every member has a bf16 score >= tau_b: its chunk is scanned.  A scanned item that is in the scanned top-C of its
+// category but not in the true top-C scores below s* (an unscanned item of its category beats it), so it cannot enter
+// the result.  Capping is decomposable -- the capped top-K of A u B is the capped top-K of capped-top-K(A) u
+// capped-top-K(B) -- so the per-CTA lists give the exact result.  The order is the total order of rerank_key, so reruns
+// are bit-identical.
+constexpr int RG = TCAR_RECOMMEND_MAXG;
+constexpr int CL_CAP = 4096;                     // chunks listed for the capped count (more, or too few: every chunk)
+
+__device__ __forceinline__ int warp_scan_incl(int v, int lane) {
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, v, o);
+        if (lane >= o) v += t;
+    }
+    return v;
+}
+
+// block-wide sum; s_w [8]; ends with a barrier
+__device__ __forceinline__ int block_sum_i(int v, int* s_w) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = v;
+    __syncthreads();
+    int t = 0;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) t += s_w[j];
+    __syncthreads();
+    return t;
+}
+
+struct CatRanges {
+    int A;        // allowed non-empty categories
+    int total;    // their chunks
+    int capped;   // sum of min(cap, chunks) over them
+};
+
+// The allowed categories of session b as ranges of the category-ordered chunks: s_cst[a] = the first chunk of the a-th
+// allowed non-empty category, s_pre[a] = the allowed chunks before it (s_pre[A] = total).  a_off == NULL allows every
+// category; codes may repeat.  s_bits [RG / 32], s_w [3][8].  256 threads (4 categories each), ends with a barrier.
+__device__ CatRanges category_ranges(const int32_t* __restrict__ cat_chunk_off, int G,
+                                     const int32_t* __restrict__ a_off, const int32_t* __restrict__ a_codes, int b,
+                                     int cap, uint32_t* s_bits, int* s_cst, int* s_pre, int (*s_w)[8]) {
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    for (int i = tid; i < RG / 32; i += 256) s_bits[i] = a_off ? 0u : ~0u;
+    __syncthreads();
+    if (a_off)
+        for (int i = a_off[b] + tid; i < a_off[b + 1]; i += 256) {
+            const int g = a_codes[i];
+            atomicOr(&s_bits[g >> 5], 1u << (g & 31));
+        }
+    __syncthreads();
+    int len[4], na = 0, nc = 0, ncap = 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        const int g = tid * 4 + j;
+        len[j] = g < G && ((s_bits[g >> 5] >> (g & 31)) & 1u) ? cat_chunk_off[g + 1] - cat_chunk_off[g] : 0;
+        na += len[j] > 0;
+        nc += len[j];
+        ncap += min(len[j], cap);
+    }
+    const int ia = warp_scan_incl(na, lane), ic = warp_scan_incl(nc, lane), ik = warp_scan_incl(ncap, lane);
+    if (lane == 31) { s_w[0][w] = ia; s_w[1][w] = ic; s_w[2][w] = ik; }
+    __syncthreads();
+    CatRanges r = {0, 0, 0};
+    int a = ia - na, c = ic - nc;
+    for (int j = 0; j < 8; ++j) {
+        if (j < w) { a += s_w[0][j]; c += s_w[1][j]; }
+        r.A += s_w[0][j];
+        r.total += s_w[1][j];
+        r.capped += s_w[2][j];
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+        if (len[j] > 0) {
+            s_cst[a] = cat_chunk_off[tid * 4 + j];
+            s_pre[a] = c;
+            ++a;
+            c += len[j];
+        }
+    if (tid == 0) s_pre[r.A] = r.total;
+    __syncthreads();
+    return r;
+}
+
+// the allowed category a that holds the i-th allowed chunk (0 <= i < s_pre[A]); that chunk is s_cst[a] + i - s_pre[a]
+__device__ __forceinline__ int allowed_index(const int* s_pre, int A, int i) {
+    int lo = 0, hi = A - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (s_pre[mid] <= i) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+__device__ __forceinline__ int allowed_chunk(const int* s_cst, const int* s_pre, int A, int i) {
+    const int a = allowed_index(s_pre, A, i);
+    return s_cst[a] + i - s_pre[a];
+}
+
+__global__ void __launch_bounds__(256)
+recommend_category_select_kernel(const float* chunkmax, const float* __restrict__ a_ic, const float* __restrict__ Tq,
+                                 const float* __restrict__ cat_stats, const int32_t* __restrict__ x_off, int n_clicks,
+                                 const int32_t* __restrict__ cat_chunk_off, int G, const int32_t* __restrict__ a_off,
+                                 const int32_t* __restrict__ a_codes, int C, int K, int n_pad,
+                                 float* __restrict__ tau, float* __restrict__ cat_tau) {
+    PDL_ENTER();
+    __shared__ float s_aic[XW], s_tq[NB + 1];
+    __shared__ float s_red[32];
+    __shared__ int s_hist[256], s_misc[2], s_w[3][8];
+    __shared__ uint32_t s_bits[RG / 32];
+    __shared__ int s_cst[RG], s_pre[RG + 1], s_cnt[RG];
+    __shared__ uint32_t s_lkey[CL_CAP];
+    __shared__ short s_lcat[CL_CAP];
+    __shared__ int s_nl;
+    const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    const int kp = K + (x_off ? x_off[b + 1] - x_off[b] : 0) + n_clicks;
+    const int cap = C < K ? C : 0x7fffffff;                           // C >= K: the list cannot exceed the cap
+    const CatRanges r = category_ranges(cat_chunk_off, G, a_off, a_codes, b, cap, s_bits, s_cst, s_pre, s_w);
+    float* ctau = cat_tau + (size_t)b * RG;
+    const float* cm = chunkmax + (size_t)b * (n_pad / CH);
+    if (r.capped <= kp && cap > kp) {                                 // block-uniform: no cap, scan every allowed chunk
+        for (int a = tid; a < r.A; a += 256) ctau[a] = -INFINITY;
+        if (tid == 0) tau[b] = -INFINITY;
+        return;
+    }
+    for (int c = tid; c < XW; c += 256) s_aic[c] = a_ic[(size_t)b * XW + c];
+    for (int c = tid; c < NB; c += 256) s_tq[c] = Tq[(size_t)b * NB + c];
+    if (r.capped <= kp) {
+        // |M| <= K': no global threshold, but a category's eligible top-C all score >= its (C + x_b)-th largest chunk
+        // maximum - eps_b (those chunks hold C + x_b distinct items of it, at most x_b excluded), so category a is
+        // scanned down to tau_a = that maximum - 2 eps_b (-inf when it has no more than C + x_b chunks)
+        __syncthreads();
+        const float eps = score_error_bound(s_aic, s_tq, cat_stats, s_red);
+        const int j = C + kp - K;
+        for (int a = 0; a < r.A; ++a) {                               // block-uniform loop
+            const int c0 = s_cst[a], len = s_pre[a + 1] - s_pre[a];
+            float t = -INFINITY;
+            if (len > j) t = key_value(block_kth_key(len, j, [&](int i) { return cm[c0 + i]; }, s_hist, s_misc)) - 2.f * eps;
+            if (tid == 0) ctau[a] = t;
+        }
+        if (tid == 0) tau[b] = -INFINITY;
+        return;
+    }
+    for (int a = tid; a < r.A; a += 256) ctau[a] = -INFINITY;
+    for (int a = tid; a < r.A; a += 256) s_cnt[a] = 0;
+    if (tid == 0) s_nl = 0;
+    __syncthreads();
+    auto chunk_val = [&](int i) { return cm[allowed_chunk(s_cst, s_pre, r.A, i)]; };
+    uint32_t v;
+    if (cap > kp) {
+        v = block_kth_key(r.total, kp, chunk_val, s_hist, s_misc);
+    } else {
+        // list the allowed chunks at or above the R-th largest (R = min(CL_CAP, total)) with their category
+        const uint32_t x0 = block_kth_key(r.total, min(CL_CAP, r.total), chunk_val, s_hist, s_misc);
+        for (int i = tid; i < r.total; i += 256) {
+            const int a = allowed_index(s_pre, r.A, i);
+            const uint32_t key = fkey(cm[s_cst[a] + i - s_pre[a]]);
+            if (key >= x0) {
+                const int at = atomicAdd(&s_nl, 1);
+                if (at < CL_CAP) { s_lkey[at] = key; s_lcat[at] = (short)a; }
+            }
+        }
+        __syncthreads();
+        const int nl = s_nl;
+        // count(x) over the list: exact for x >= x0 when every chunk >= x0 is listed
+        auto count_list = [&](uint32_t x) {
+            for (int i = tid; i < nl; i += 256)
+                if (s_lkey[i] >= x) atomicAdd(&s_cnt[s_lcat[i]], 1);
+            __syncthreads();
+            int s = 0;
+            for (int a = tid; a < r.A; a += 256) { s += min(s_cnt[a], cap); s_cnt[a] = 0; }
+            return block_sum_i(s, s_w[0]);
+        };
+        // count(x) over every allowed chunk: one warp per category, stopping at cap chunks >= x
+        auto count_all = [&](uint32_t x) {
+            int s = 0;
+            for (int a = w; a < r.A; a += 8) {
+                const int c0 = s_cst[a], len = s_pre[a + 1] - s_pre[a];
+                int n = 0;
+                for (int j0 = 0; j0 < len && n < cap; j0 += 32) {
+                    const int j = j0 + lane;
+                    n += __popc(__ballot_sync(0xffffffffu, j < len && fkey(cm[c0 + j]) >= x));
+                }
+                s += min(n, cap);
+            }
+            return block_sum_i(lane == 0 ? s : 0, s_w[0]);
+        };
+        const bool listed = nl <= CL_CAP && count_list(x0) >= kp;     // block-uniform
+        v = 0;
+        for (int bit = 31; bit >= 0; --bit) {
+            const uint32_t x = v | (1u << bit);
+            const bool ok = listed ? (x <= x0 || count_list(x) >= kp) : count_all(x) >= kp;
+            if (ok) v = x;
+        }
+    }
+    const float eps = score_error_bound(s_aic, s_tq, cat_stats, s_red);
+    if (tid == 0) tau[b] = key_value(v) - 2.f * eps;
+}
+
+// out[0 .. K) = the capped top-K of the ascending lists a[0 .. K) and c[0 .. nc): their real entries merged into u
+// (merge path), then walked in order by warp 0, which drops an entry with cap earlier entries of its category
+// (item_cat[id]) and keeps the first K; KEY_NONE after them.  s_ccnt [G] is zero on entry and on exit.  u holds
+// K + nc keys, uc as many ints.  Ends with a barrier.
+__device__ void merge_topk_capped(const unsigned long long* a, int K, const unsigned long long* c, int nc,
+                                  unsigned long long* out, unsigned long long* u, int* uc,
+                                  const int32_t* __restrict__ item_cat, int cap, int* s_ccnt) {
+    const int tid = threadIdx.x, lane = tid & 31;
+    const int ra = rank_in(a, K, KEY_NONE), rc = rank_in(c, nc, KEY_NONE), m = ra + rc;
+    for (int i = tid; i < ra; i += 256) u[i + rank_in(c, rc, a[i])] = a[i];
+    for (int j = tid; j < rc; j += 256) u[j + rank_in(a, ra, c[j])] = c[j];
+    __syncthreads();
+    for (int i = tid; i < m; i += 256) uc[i] = item_cat[(uint32_t)u[i]];
+    __syncthreads();
+    if (tid < 32) {
+        int kept = 0;
+        for (int i0 = 0; i0 < m && kept < K; i0 += 32) {
+            const int i = i0 + lane;
+            const bool real = i < m;
+            const int g = real ? uc[i] : -1 - lane;
+            const uint32_t peers = __match_any_sync(0xffffffffu, g);
+            const uint32_t below = (1u << lane) - 1u;
+            const bool keep = real && s_ccnt[g < 0 ? 0 : g] + __popc(peers & below) < cap;
+            const uint32_t kb = __ballot_sync(0xffffffffu, keep);
+            const int pos = kept + __popc(kb & below);
+            if (keep && pos < K) out[pos] = u[i];
+            kept += __popc(kb);
+            __syncwarp();
+            if (real && lane == 31 - __clz(peers)) s_ccnt[g] += __popc(peers);
+            __syncwarp();
+        }
+        for (int i = min(kept, K) + lane; i < K; i += 32) out[i] = KEY_NONE;
+        for (int i = lane; i < m; i += 32) s_ccnt[uc[i]] = 0;
+    }
+    __syncthreads();
+}
+
+__global__ void __launch_bounds__(256, 2)
+recommend_category_scan_kernel(const float* chunkmax, const float* __restrict__ a_ic, const float* __restrict__ Tq,
+                               const float* __restrict__ item, const float* __restrict__ content,
+                               const int32_t* __restrict__ mwdhm, const int32_t* __restrict__ x_off,
+                               const int32_t* __restrict__ x_ids, const int32_t* __restrict__ clicks, int n_clicks,
+                               const int32_t* __restrict__ perm, const int32_t* __restrict__ item_cat,
+                               const int32_t* __restrict__ cat_chunk_off, int G, const int32_t* __restrict__ a_off,
+                               const int32_t* __restrict__ a_codes, int C, int K, int n_pad, int B, char* wspace,
+                               int32_t* __restrict__ out_ids, float* __restrict__ out_scores,
+                               int32_t* __restrict__ rescored, const float* __restrict__ cat_tau) {
+    PDL_ENTER();
+    __shared__ float s_aic[XW], s_tq[NB + 1];
+    __shared__ int s_x[RX];
+    __shared__ int s_q[256];
+    __shared__ unsigned long long s_top[2][RK];
+    __shared__ unsigned long long s_new[NCAND];
+    __shared__ unsigned long long s_u[RK + NCAND];
+    __shared__ int s_uc[RK + NCAND];
+    __shared__ uint32_t s_bits[RG / 32];
+    __shared__ int s_cst[RG], s_pre[RG + 1], s_ccnt[RG], s_w[3][8];
+    __shared__ float s_ctau[RG];
+    __shared__ int s_qn, s_cnt, s_last;
+    const int b = blockIdx.x, split = blockIdx.y, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    int32_t* ticket = reinterpret_cast<int32_t*>(wspace);
+    const float* tau = reinterpret_cast<const float*>(wspace) + TCAR_QROWS;
+    int32_t* part_cnt = reinterpret_cast<int32_t*>(wspace) + TCAR_QROWS + B;
+    unsigned long long* part = reinterpret_cast<unsigned long long*>(wspace + rec_keys_offset(B));
+    const int xo = x_off ? x_off[b] : 0;
+    const int nl = x_off ? x_off[b + 1] - xo : 0, nx = nl + n_clicks;
+    if (nl < 0 || nx > RX) return;                                   // block-uniform, and the same for every split
+    const bool capped = C < K;
+    int P = 1;
+    while (P < nx) P <<= 1;
+    for (int i = tid; i < P; i += 256)
+        s_x[i] = i < nl ? x_ids[xo + i] : i < nx ? clicks[(size_t)b * n_clicks + (i - nl)] - 1 : 0x7fffffff;
+    for (int c = tid; c < XW; c += 256) s_aic[c] = a_ic[(size_t)b * XW + c];
+    for (int c = tid; c < NB; c += 256) s_tq[c] = Tq[(size_t)b * NB + c];
+    for (int i = tid; i < RK; i += 256) s_top[0][i] = KEY_NONE;
+    for (int g = tid; g < G; g += 256) s_ccnt[g] = 0;
+    if (tid == 0) { s_qn = 0; s_cnt = 0; }
+    __syncthreads();
+    for (int k = 2; k <= P; k <<= 1) {
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int i = tid; i < P; i += 256) {
+                const int ixj = i ^ j;
+                if (ixj > i) {
+                    const int a = s_x[i], c = s_x[ixj];
+                    if (((i & k) == 0) ? a > c : a < c) { s_x[i] = c; s_x[ixj] = a; }
+                }
+            }
+            __syncthreads();
+        }
+    }
+    auto excluded = [&](int n) {
+        int lo = 0, hi = nx;
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (s_x[mid] < n) lo = mid + 1; else hi = mid;
+        }
+        return lo < nx && s_x[lo] == n;
+    };
+    const CatRanges r = category_ranges(cat_chunk_off, G, a_off, a_codes, b, 1, s_bits, s_cst, s_pre, s_w);
+    for (int a = tid; a < r.A; a += 256) s_ctau[a] = cat_tau[(size_t)b * RG + a];
+    __syncthreads();
+    const float* cm = chunkmax + (size_t)b * (n_pad / CH);
+    const float bound = tau[b];
+    const int per = (r.total + WSPLIT - 1) / WSPLIT;
+    const int i_lo = split * per, i_hi = min(i_lo + per, r.total);
+    int cur = 0, my_cnt = 0;
+    for (int i0 = i_lo; i0 < i_hi; i0 += 256) {
+        const int i = i0 + tid;
+        if (i < i_hi) {
+            const int a = allowed_index(s_pre, r.A, i);
+            const int chunk = s_cst[a] + i - s_pre[a];
+            if (cm[chunk] >= fmaxf(bound, s_ctau[a])) s_q[atomicAdd(&s_qn, 1)] = chunk;
+        }
+        __syncthreads();
+        const int qn = s_qn;
+        for (int q0 = 0; q0 < qn; q0 += NCH) {
+            const int ncand = min(qn - q0, NCH) * CH;
+            int P2 = 32;                                              // sort size: power of two >= ncand
+            while (P2 < ncand) P2 <<= 1;
+            if (tid < P2) s_new[tid] = KEY_NONE;
+            __syncthreads();
+            for (int ci = w; ci < ncand; ci += 32) {
+                // four candidates per warp and iteration, branch-free; a pad or an excluded id reads row 0 instead
+                int nn[4];
+                float sc[4];
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    const int cu = ci + 8 * u;
+                    const int n = cu < ncand ? perm[s_q[q0 + cu / CH] * CH + (cu % CH)] : -1;
+                    nn[u] = n >= 0 && !excluded(n) ? n : -1;
+                }
+#pragma unroll
+                for (int u = 0; u < 4; ++u)
+                    sc[u] = exact_score_e(s_aic, s_tq, item, content, mwdhm, nn[u] >= 0 ? nn[u] : 0, lane);
+                if (lane == 0) {
+#pragma unroll
+                    for (int u = 0; u < 4; ++u)
+                        if (nn[u] >= 0) { s_new[ci + 8 * u] = rerank_key(sc[u], nn[u]); ++my_cnt; }
+                }
+            }
+            for (int k = 2; k <= P2; k <<= 1) {
+                for (int j = k >> 1; j > 0; j >>= 1) {
+                    __syncthreads();
+                    const int ixj = tid ^ j;
+                    if (tid < P2 && ixj > tid) {
+                        const unsigned long long a = s_new[tid], c = s_new[ixj];
+                        if (((tid & k) == 0) ? a > c : a < c) { s_new[tid] = c; s_new[ixj] = a; }
+                    }
+                }
+            }
+            __syncthreads();
+            if (capped)
+                merge_topk_capped(s_top[cur], K, s_new, P2, s_top[cur ^ 1], s_u, s_uc, item_cat, C, s_ccnt);
+            else
+                merge_topk(s_top[cur], K, s_new, P2, s_top[cur ^ 1]);
+            cur ^= 1;
+        }
+        if (tid == 0) s_qn = 0;
+        __syncthreads();
+    }
+    if (lane == 0 && my_cnt) atomicAdd(&s_cnt, my_cnt);
+    unsigned long long* mine = part + ((size_t)split * B + b) * RK;
+    for (int i = tid; i < K; i += 256) mine[i] = s_top[cur][i];
+    __syncthreads();
+    if (tid == 0) part_cnt[(size_t)split * B + b] = s_cnt;
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) s_last = atomicAdd(&ticket[b], 1) == WSPLIT - 1;
+    __syncthreads();
+    if (!s_last) return;
+    __threadfence();
+    for (int s = 0; s < WSPLIT; ++s) {
+        if (s == split) continue;
+        const unsigned long long* other = part + ((size_t)s * B + b) * RK;
+        for (int i = tid; i < K; i += 256) s_new[i] = __ldcg(other + i);
+        __syncthreads();
+        if (capped)
+            merge_topk_capped(s_top[cur], K, s_new, K, s_top[cur ^ 1], s_u, s_uc, item_cat, C, s_ccnt);
+        else
+            merge_topk(s_top[cur], K, s_new, K, s_top[cur ^ 1]);
+        cur ^= 1;
+    }
+    for (int i = tid; i < K; i += 256) {
+        const unsigned long long key = s_top[cur][i];
+        out_ids[(size_t)b * K + i] = key == KEY_NONE ? -1 : (int)(uint32_t)key;
+        out_scores[(size_t)b * K + i] = key == KEY_NONE ? -INFINITY : key_value(~(uint32_t)(key >> 32));
+    }
+    if (tid == 0) {
+        if (rescored) {
+            int t = 0;
+            for (int s = 0; s < WSPLIT; ++s) t += __ldcg(part_cnt + (size_t)s * B + b);
+            rescored[b] = t;
+        }
+        ticket[b] = 0;
+    }
+}
+
 }  // namespace tcar
 
 using namespace tcar;
@@ -1628,6 +2051,40 @@ extern "C" int tcar_recommend_window(const float* chunkmax, const float* tilemax
     launch_pdl(recommend_scan_kernel<true>, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq, item,
                content, mwdhm, x_off, x_ids, clicks, n_clicks, K, N, n_pad, B, ws, ids, scores, rescored, item_time,
                win_lo, win_hi);
+    return (int)cudaGetLastError();
+}
+
+// tcar_recommend's workspace, then the per-category thresholds [B][TCAR_RECOMMEND_MAXG]
+static size_t rec_cat_tau_offset(int B) { return rec_keys_offset(B) + (size_t)WSPLIT * B * RK * 8; }
+
+extern "C" long long tcar_recommend_category_ws_bytes(int B) {
+    if (B < 0 || B > TCAR_QROWS) return TCAR_ERR_ARG;
+    return (long long)(rec_cat_tau_offset(B) + (size_t)B * RG * 4);
+}
+
+extern "C" int tcar_recommend_category(const float* chunkmax, const float* a_ic, const float* Tq, const float* item,
+                                       const float* content, const int32_t* mwdhm, const float* cat_stats,
+                                       const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B,
+                                       int n_pad, int K, const int32_t* perm, const int32_t* item_cat,
+                                       const int32_t* cat_chunk_off, int G, const int32_t* a_off,
+                                       const int32_t* a_codes, int C, void* workspace, int32_t* ids, float* scores,
+                                       int32_t* rescored, void* stream) {
+    if (B < 0 || B > TCAR_QROWS || n_pad < CH || n_pad % 128 || K < 1 || K > RK || G < 1 || G > RG || C < 1 ||
+        (clicks && (T < 1 || T > RX)) || !chunkmax || !a_ic || !Tq || !item || !content || !mwdhm || !cat_stats ||
+        (x_off && !x_ids) || (a_off && !a_codes) || !perm || !item_cat || !cat_chunk_off || !workspace || !ids ||
+        !scores)
+        return TCAR_ERR_ARG;
+    if (B == 0) return 0;
+    const int n_clicks = clicks ? T : 0;
+    char* ws = static_cast<char*>(workspace);
+    cudaError_t e = launch_pdl(recommend_category_select_kernel, dim3(B), dim3(256), 0, STREAM, chunkmax, a_ic, Tq,
+                               cat_stats, x_off, n_clicks, cat_chunk_off, G, a_off, a_codes, C, K, n_pad,
+                               reinterpret_cast<float*>(ws) + TCAR_QROWS,
+                               reinterpret_cast<float*>(ws + rec_cat_tau_offset(B)));
+    if (e != cudaSuccess) return (int)e;
+    launch_pdl(recommend_category_scan_kernel, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, a_ic, Tq, item, content,
+               mwdhm, x_off, x_ids, clicks, n_clicks, perm, item_cat, cat_chunk_off, G, a_off, a_codes, C, K, n_pad, B,
+               ws, ids, scores, rescored, reinterpret_cast<const float*>(ws + rec_cat_tau_offset(B)));
     return (int)cudaGetLastError();
 }
 

@@ -84,6 +84,14 @@ def max_age_hours(text):
     return h
 
 
+def max_per_category(text):
+    """--recommend_max_per_category: an integer >= 1."""
+    c = int(text)
+    if c < 1:
+        raise argparse.ArgumentTypeError("must be >= 1")
+    return c
+
+
 class _Parser(argparse.ArgumentParser):
     """Checks the flags that depend on one another right after parsing, before any data is loaded."""
 
@@ -91,6 +99,11 @@ class _Parser(argparse.ArgumentParser):
         ns = super().parse_args(args, namespace)
         if getattr(ns, "recommend_max_age_h", None) is not None and ns.recommend_k is None:
             self.error("--recommend_max_age_h requires --recommend_k")
+        if getattr(ns, "recommend_max_per_category", None) is not None:
+            if ns.recommend_k is None:
+                self.error("--recommend_max_per_category requires --recommend_k")
+            if ns.recommend_max_age_h is not None:
+                self.error("--recommend_max_per_category cannot be combined with --recommend_max_age_h")
         return ns
 
 
@@ -145,6 +158,9 @@ def build_parser():
     # not a reference flag: recommend only articles published at most H hours before the session's last input click
     # (the time-aware protocol: publish-time windows applied exactly on the device, Seq2SeqAttNN.recommend_split)
     parser.add_argument("--recommend_max_age_h", default=None, type=max_age_hours)
+    # not a reference flag: at most C articles of one category per recommended list (exact capped top-K on the device,
+    # Seq2SeqAttNN.recommend_split); also prints the lists' ILD and unexpectedness
+    parser.add_argument("--recommend_max_per_category", default=None, type=max_per_category)
     parser.add_argument("--inputdata", default="test", type=str)
     parser.add_argument("--threshold_acc", default=0.27, type=float)
     # additions

@@ -20,7 +20,8 @@ from . import parallel
 from .catalog_parallel import CatalogShardedTraining
 from .params import ParamStore, SMALL
 from .sampler import Sampler, pack_batch
-from .util import check_id_lists, check_item_times, check_windows
+from .util import (category_layout, check_id_lists, check_item_categories, check_item_times, check_windows,
+                   pad_sources)
 
 H, TH, XW, PW, NB, KEXT, QROWS, TOPK = nv.H, nv.TH, nv.XW, nv.PW, nv.NBINS, nv.KEXT, nv.QROWS, nv.TOPK
 
@@ -1382,7 +1383,39 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             self._item_time = torch.zeros(self.ps.n_pad, device=self.dev, dtype=torch.int32)
         self._item_time[:self.N].copy_(torch.from_numpy(t))
 
-    def recommend(self, bt, k=20, exclude_off=None, exclude_ids=None, exclude_clicked=False, window=None):
+    def set_item_categories(self, codes, n_categories=None):
+        """One category code per item for recommend(max_per_category=..., categories=...): N integers in [0, G),
+        G = n_categories (default max(codes) + 1) <= nv.RECOMMEND_MAXG.  Checked on the host (ValueError, nothing
+        uploaded).  Builds the catalog in category order (util.category_layout: N' <= N + 7 G positions) and iext_cat,
+        a second copy of the bf16 scoring operand whose row p is the ps.iext row of the item at position p, about
+        N' x 1280 bytes; recommend() rebuilds it whenever the item table has changed.  May be called again."""
+        codes, G = check_item_categories(codes, self.N, n_categories)
+        perm, off, n2 = category_layout(codes, G)
+        n_pad = (n2 + 255) // 256 * 256
+        dev = self.dev
+        if getattr(self, "_iext_cat", None) is None or self._iext_cat.shape[0] != n_pad:
+            old = getattr(self, "_cat_n_pad", None)
+            if old is not None and old != self.ps.n_pad:
+                self._score_ws.pop((old, False), None)       # the previous layout's score buffers
+            self._iext_cat = torch.zeros(n_pad, nv.KEXT, device=dev, dtype=torch.bfloat16)
+        else:
+            self._iext_cat[n2:].zero_()                      # rows >= N' are zero
+        self._cat_perm = torch.from_numpy(perm).to(dev)
+        self._cat_src = torch.from_numpy(pad_sources(perm)).to(dev)
+        self._cat_off = torch.from_numpy(off).to(dev)
+        self._item_cat = torch.from_numpy(codes).to(dev)
+        self._cat_G, self._cat_n, self._cat_n_pad = G, n2, n_pad
+        self._iext_cat_version = -1
+
+    def _ensure_iext_cat(self):
+        """Gather iext_cat from ps.iext again when the item table has changed since the last build (the rule of
+        _ensure_cat_stats): a plain row gather, off the per-batch path."""
+        if self._iext_cat_version != self.ps.version:
+            torch.index_select(self.ps.iext, 0, self._cat_src, out=self._iext_cat[:self._cat_n])
+            self._iext_cat_version = self.ps.version
+
+    def recommend(self, bt, k=20, exclude_off=None, exclude_ids=None, exclude_clicked=False, window=None,
+                  max_per_category=None, categories=None):
         """The exact top-k of the whole catalog for every session of bt (tcar_recommend), 1 <= k <= nv.RECOMMEND_MAXK,
         ordered by (score desc, id asc).  Scores are the exact fp32 scores of the full-catalog evaluation: with k <= 20
         and no exclusions the result is the prefix of eval_step's top-20, and an item scores bit for bit what eval_step
@@ -1402,7 +1435,13 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         session b to the items with lo[b] <= t[n] <= hi[b], t = the times of set_item_times (same clock unit).  The
         result is the exact top-k of the in-window, non-excluded items, with the same exact scores; a window with fewer
         than k of them pads with -1 / -inf.  The mask sits in the scoring GEMM's epilogue (tcar_score_fwd_window,
-        tcar_recommend_window), so the selection stays exact however few items a window holds."""
+        tcar_recommend_window), so the selection stays exact however few items a window holds.
+
+        Categories (after set_item_categories): max_per_category = C >= 1 leaves out an item that has C better items of
+        its category in the list (C >= k: no cap); categories = (off, codes) restricts session b to the categories
+        codes[off[b]:off[b + 1]] (CSR as the exclusion lists, codes in [0, G), duplicates allowed; an empty list gives
+        -1 / -inf throughout).  Exclusions compose with both; window does not (ValueError).  The result is the exact
+        capped, filtered top-k in the same format, by the scoring GEMM over iext_cat and tcar_recommend_category."""
         if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= nv.RECOMMEND_MAXK:
             raise ValueError(f"k must be an integer in [1, TCAR_RECOMMEND_MAXK = {nv.RECOMMEND_MAXK}], got {k!r}")
         if (exclude_off is None) != (exclude_ids is None):
@@ -1421,6 +1460,25 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             if getattr(self, "_item_time", None) is None:
                 raise ValueError("window needs item times: call set_item_times first")
             win = check_windows(window, B)
+        by_cat = max_per_category is not None or categories is not None
+        if by_cat:
+            if getattr(self, "_iext_cat", None) is None:
+                raise ValueError("max_per_category / categories need item categories: call set_item_categories first")
+            if window is not None:
+                raise ValueError("window cannot be combined with max_per_category / categories")
+            C = k
+            if max_per_category is not None:
+                if isinstance(max_per_category, (bool, np.bool_)) or not isinstance(max_per_category, (int, np.integer)) \
+                        or max_per_category < 1:
+                    raise ValueError(f"max_per_category must be an integer >= 1, got {max_per_category!r}")
+                C = int(min(max_per_category, k))
+            allowed = None
+            if categories is not None:
+                if not isinstance(categories, (tuple, list)) or len(categories) != 2:
+                    raise ValueError("categories must be a pair (off, codes) of integer arrays")
+                allowed, _ = check_id_lists(categories[0], categories[1], B, self._cat_G,
+                                            names=("categories off", "categories codes"),
+                                            nouns=("category", "categories"), limit=float("inf"), limit_name="")
         dev, p, ps = self.dev, nv.ptr, self.ps
         out_ids = torch.empty(B, k, device=dev, dtype=torch.int32)
         out_sc = torch.empty(B, k, device=dev)
@@ -1437,6 +1495,8 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         ws = self._score_buffers(ps.n_pad, False)
         if win is not None:
             return self._recommend_window(bt, k, host, exclude_clicked, win, out_ids, out_sc)
+        if by_cat:
+            return self._recommend_category(bt, k, host, exclude_clicked, C, allowed, out_ids, out_sc)
         # one unguarded eval-mode GEMM for the chunk / tile maxima; its softmax partial sums (which may overflow without
         # the guard) are not read
         nv.counted_call("tcar_score_fwd", 1, p(self.Q), p(ps.iext), p(self.c_ref), None, p(ws["part"]), p(ws["cmax"]),
@@ -1464,6 +1524,29 @@ class Seq2SeqAttNN(CatalogShardedTraining):
                         p(self._item_time), p(wv), p(wv[B:]))
         return out_ids, out_sc
 
+    def _recommend_category(self, bt, k, host, exclude_clicked, C, allowed, out_ids, out_sc):
+        """recommend() with item categories: the unchanged eval-mode GEMM over iext_cat (N' items in category order),
+        then tcar_recommend_category with the cap C (C = k: none) and the checked CSR allowed-code lists (None: all)."""
+        B, p, ps = bt.B, nv.ptr, self.ps
+        if getattr(self, "_rec_cat_ws", None) is None:
+            # tcar_recommend's layout (ticket counters first: zero once, every call leaves them at zero), then the
+            # per-category thresholds
+            self._rec_cat_ws = torch.zeros(int(nv.lib().tcar_recommend_category_ws_bytes(QROWS)), device=self.dev,
+                                           dtype=torch.uint8)
+        self._ensure_iext_cat()
+        ws = self._score_buffers(self._cat_n_pad, False)
+        nv.counted_call("tcar_score_fwd", 1, p(self.Q), p(self._iext_cat), p(self.c_ref), None, p(ws["part"]),
+                        p(ws["cmax"]), p(ws["tmax"]), B, self._cat_n, self._cat_n_pad, 1, self._cluster_for(B))
+        csr = self._stage_ints(host) if host is not None else None
+        acsr = self._stage_ints(allowed) if allowed is not None else None
+        nv.counted_call("tcar_recommend_category", 2, p(ws["cmax"]), p(self.a_ic), p(self.Tq), p(ps.item),
+                        p(ps.content), p(ps.mwdhm), p(self.cat_stats), p(csr),
+                        p(csr[B + 1:]) if csr is not None else None, p(bt.seq) if exclude_clicked else None, bt.T, B,
+                        self._cat_n_pad, k, p(self._cat_perm), p(self._item_cat), p(self._cat_off), self._cat_G,
+                        p(acsr), p(acsr[B + 1:]) if acsr is not None else None, C, p(self._rec_cat_ws), p(out_ids),
+                        p(out_sc), p(self.rec_rescored))
+        return out_ids, out_sc
+
     def recommend_split(self, sess, test_data, item_dict, args):
         """Recommend the top-K articles (args["recommend_k"], default 20) for every session of a split, optionally
         without the session's own clicks (args["recommend_exclude_clicked"]), in the batches test() uses.  Writes one
@@ -1477,13 +1560,27 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         [t_req - round(60 H) min, t_req], t_req = the click time of its last input click (util.session_windows): the
         time-aware protocol, which never recommends an article published after the request.  Article times are
         args["publish_time"] (one datetime per item, main.load_datas) in minutes since the epoch.  Then the result
-        also holds "label_outside": the sessions whose label was published outside their window (never a hit)."""
-        from .util import (count_outside, epoch_minutes, label_positions, recommend_line, session_windows, topk_metrics,
-                           topk_sums)
+        also holds "label_outside": the sessions whose label was published outside their window (never a hit).
+
+        args["recommend_max_per_category"] = C returns at most C articles of one category per list (exact: the capped
+        top-K, recommend(max_per_category=C)), with the categories of args["category_id"]; it cannot be combined with
+        recommend_max_age_h.  The articles without a category share one extra code here, unlike _categories(), which
+        gives each its own: every category is padded to whole 8-item chunks in the category-ordered catalog, and one
+        padded category per unknown article would blow up its size.  Then the result also holds "ild" and "unexp",
+        the reference's intra-list diversity and unexpectedness (getILD / getUnexp, padding dropped) averaged as test()
+        averages them: over the returned lists of at least two items."""
+        from .util import (count_outside, diversity_sums, epoch_minutes, label_positions, recommend_line,
+                           session_windows, topk_metrics, topk_sums)
         k = int(args.get("recommend_k") or 20)
         clicked = bool(args.get("recommend_exclude_clicked"))
         max_age = args.get("recommend_max_age_h")
         windowed = max_age is not None
+        cap = args.get("recommend_max_per_category")
+        capped = cap is not None
+        if capped:
+            if windowed:
+                raise ValueError("recommend_max_per_category cannot be combined with recommend_max_age_h")
+            self.set_item_categories(self._split_category_codes())
         if windowed:
             if not float(max_age) > 0:
                 raise ValueError(f"recommend_max_age_h must be > 0 hours, got {max_age!r}")
@@ -1492,9 +1589,10 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             item_time = epoch_minutes(args["publish_time"])
             self.set_item_times(item_time)
             max_age_min = int(round(60 * float(max_age)))
-        print("Recommending the top-{} articles{}{}...".format(
+        print("Recommending the top-{} articles{}{}{}...".format(
             k, " without the clicked ones" if clicked else "",
-            " published at most {} h before the request".format(max_age) if windowed else ""))
+            " published at most {} h before the request".format(max_age) if windowed else "",
+            ", at most {} per category".format(cap) if capped else ""))
         self.sync_item_table()
         session_dict_test = test_data[1]
         reverse = self.reverse_item if self.reverse_item is not None else \
@@ -1506,11 +1604,12 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         os.makedirs("saved", exist_ok=True)
         dist_on = parallel.is_distributed(self.world)
         path = "saved/recommend_{}{}.txt".format(args.get("foldnum", 0), "_rank{}".format(self.rank) if dist_on else "")
-        sums = np.zeros(5 if windowed else 4)
+        sums = np.zeros(5 if windowed else 7 if capped else 4)
 
         def launch(cur, nxt):
             bt, (kb, win) = cur
-            ids, sc = self.recommend(bt, k, exclude_clicked=clicked, window=win)
+            ids, sc = self.recommend(bt, k, exclude_clicked=clicked, window=win,
+                                     **({"max_per_category": int(cap)} if capped else {}))
             return kb, win, self.fetch_async(ids), self.fetch_async(sc)
 
         def consume(kb, win, ids_h, sc_h):
@@ -1519,6 +1618,9 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             sums[:4] += topk_sums(label_positions(ids, labels))
             if windowed:
                 sums[4] += count_outside(item_time[labels], *win)
+            if capped:
+                sums[4:] += diversity_sums(ids, [np.asarray(session_dict_test[key][:-1]) - 1 for key in kb],
+                                           self._categories())
             f.writelines(recommend_line(key, ids[b], sc[b], reverse) for b, key in enumerate(kb))
 
         with open(path, "w") as f:
@@ -1528,12 +1630,28 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         m = topk_metrics(total[:4])
         if windowed:
             m["label_outside"] = int(total[4])
+        if capped:
+            n = total[6]
+            m["ild"], m["unexp"] = (float(total[4] / n), float(total[5] / n)) if n > 0 else (float("nan"),) * 2
         self.last_recommend_metrics = m
         self.last_recommend_path = path
         print("Recommend: HR@{k}: {}, MRR@{k}: {}, nDCG@{k}: {} ({} sessions{}, written to {})".format(
             m["hr"], m["mrr"], m["ndcg"], m["sessions"],
             ", {} labels published outside their window".format(m["label_outside"]) if windowed else "", path, k=k))
+        if capped:
+            print("Recommend: ILD: {}, unexpectedness: {}".format(m["ild"], m["unexp"]))
         return m
+
+    def _split_category_codes(self):
+        """Category code of every item for recommend_split: args["category_id"] through reverse_item, codes in order
+        of first appearance; every item without a category gets one shared extra code (see recommend_split)."""
+        codes, index, none = np.empty(self.N, dtype=np.int64), {}, object()
+        getter = self.category_id.get if hasattr(self.category_id, "get") else None
+        for i in range(self.N):
+            art = self.reverse_item.get(i, none) if hasattr(self.reverse_item, "get") else self.reverse_item[i]
+            c = getter(art, none) if getter is not None else self.category_id[art]
+            codes[i] = index.setdefault(c, len(index))
+        return codes
 
     # ------------------------------------------------------------------------------------------- metrics
     def _categories(self):

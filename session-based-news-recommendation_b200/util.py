@@ -7,6 +7,8 @@ import time
 
 import numpy as np
 
+from ._native import CHUNK, RECOMMEND_MAXG
+
 
 def cau_metrics(preds, labels, cutoff=20):
     """util.py:8-18 on a materialised score matrix (used by tests / debugging; the hot path gets the rank from
@@ -172,6 +174,83 @@ def count_outside(times, lo, hi):
     """Number of sessions whose time (e.g. their label's publish time) lies outside their window [lo, hi]."""
     t = np.asarray(times, dtype=np.int64)
     return int(((t < np.asarray(lo)) | (t > np.asarray(hi))).sum())
+
+
+def check_item_categories(codes, N, G=None):
+    """Validate one category code per item before anything is uploaded: N integers in [0, G), G <= RECOMMEND_MAXG
+    (G defaults to max(codes) + 1).  Returns (the codes as an int32 host array, G); raises ValueError."""
+    c = np.asarray(codes).reshape(-1)
+    if c.size and c.dtype.kind not in "iu":
+        raise ValueError("item categories must be integers")
+    if c.shape[0] != N:
+        raise ValueError(f"item categories must hold N = {N} codes, got {c.shape[0]}")
+    if G is None:
+        G = max(int(c.max()) + 1, 1) if c.size else 1
+    if isinstance(G, (bool, np.bool_)) or not isinstance(G, (int, np.integer)) or not 1 <= G <= RECOMMEND_MAXG:
+        raise ValueError(f"the number of categories must be in [1, TCAR_RECOMMEND_MAXG = {RECOMMEND_MAXG}], got {G!r}")
+    if c.size and (c.min() < 0 or c.max() >= G):
+        n = int(np.argmax((c < 0) | (c >= G)))
+        raise ValueError(f"item {n}: category {int(c[n])} outside [0, {G})")
+    return c.astype(np.int32), int(G)
+
+
+def category_layout(codes, G):
+    """The catalog in category order for recommend(max_per_category / categories): codes = N ints in [0, G).
+    Items are sorted by (code, id) and every category is padded to a multiple of CHUNK positions by repeating its last
+    item, so that every chunk holds items of one category only and its maximum is the score of a real item.
+    Returns (perm int32 [N'], cat_chunk_off int32 [G + 1], N'): perm[p] = the original id at position p, -1 on a pad
+    (pad_sources gives the item a pad repeats); category g owns the chunks cat_chunk_off[g] .. cat_chunk_off[g + 1]
+    (empty for an empty category); N' = CHUNK * cat_chunk_off[G] <= N + 7 G."""
+    c = np.asarray(codes, dtype=np.int64).reshape(-1)
+    order = np.argsort(c, kind="stable")                       # by (code, id)
+    count = np.bincount(c, minlength=G)[:G]
+    off = np.zeros(G + 1, dtype=np.int64)
+    np.cumsum((count + CHUNK - 1) // CHUNK, out=off[1:])
+    first = np.zeros(G + 1, dtype=np.int64)                    # first sorted index of each category
+    np.cumsum(count, out=first[1:])
+    n2 = int(off[G]) * CHUNK
+    perm = np.full(n2, -1, dtype=np.int32)
+    cat = c[order]
+    perm[off[cat] * CHUNK + (np.arange(c.shape[0]) - first[cat])] = order
+    return perm, off.astype(np.int32), n2
+
+
+def pad_sources(perm):
+    """The id whose row every position of a category_layout holds: perm[p], or on a pad the item it repeats (the
+    last real position before it, which always lies in the same chunk and category).  int64 [N']."""
+    perm = np.asarray(perm)
+    last = np.where(perm >= 0, np.arange(perm.shape[0]), 0)
+    return perm[np.maximum.accumulate(last)].astype(np.int64) if perm.size else np.zeros(0, dtype=np.int64)
+
+
+def list_ild(cats):
+    """Intra-list diversity of one list's category codes (model_combine.py:174-182 of the reference): the share of
+    ordered pairs of distinct positions whose categories differ; 0 for a list of fewer than two items."""
+    c = np.asarray(cats).reshape(-1)
+    n = c.shape[0]
+    return float((c[:, None] != c[None, :]).sum()) / (n * (n - 1)) if n > 1 else 0.0
+
+
+def list_unexp(cats, clicked_cats):
+    """Unexpectedness of one list (model_combine.py:184-194 of the reference): the share of (recommended, clicked)
+    pairs whose categories differ; 0 for an empty list."""
+    c, ci = np.asarray(cats).reshape(-1), np.asarray(clicked_cats).reshape(-1)
+    if c.shape[0] == 0 or ci.shape[0] == 0:
+        return 0.0
+    return float((c[:, None] != ci[None, :]).sum()) / (c.shape[0] * ci.shape[0])
+
+
+def diversity_sums(ids, clicked, cat):
+    """Sums of list_ild and list_unexp over the returned lists ids [B, K] (the -1 padding dropped) of at least two
+    items, and their number (test() averages over those lists); clicked[b] = the 0-based ids of session b's clicks,
+    cat = the category code of every item.  float64 [3]; the sums add up across batches and ranks."""
+    cat = np.asarray(cat)
+    s = np.zeros(3)
+    for row, cl in zip(np.asarray(ids), clicked):
+        c = cat[row[row >= 0]]
+        if len(c) > 1:
+            s += (list_ild(c), list_unexp(c, cat[np.asarray(cl, dtype=np.int64)]), 1)
+    return s
 
 
 def _load(path):

@@ -4,6 +4,7 @@ with and without the session's own clicks excluded.
 
     python tools/recommend_probe.py [--shapes globo,mind]
     python tools/recommend_probe.py --window [--shapes globo,mind]
+    python tools/recommend_probe.py --category [--shapes globo,mind]
 
 recommend_split across ranks is checked by tools/split_check.py.
 
@@ -26,6 +27,18 @@ its own window of that many consecutive times) and K in {20, 100}, T = 1, no exc
                                              over 32 batches); ratio = window / none
   rescored_mean / rescored_max               items re-scored exactly per query with the window (rescored_nowin_mean:
                                              without)
+
+--category: at most C items per category and allowed categories (set_item_categories / recommend(max_per_category,
+categories) / tcar_recommend_category), item codes drawn uniformly from G categories: Globo (G = 461) and MIND
+(G = 17, 264) shapes, B = 512, T in {1, 20}, K in {20, 100}, C in {1, 2, K}, allowed = all / one category per session /
+10 % of the categories per session, no exclusions.  One JSON line per workload:
+  gemm_us_cold / gemm_cat_us_cold            the mode-1 scoring GEMM over ps.iext / over iext_cat alone
+                                             (torch.profiler, L2 overwritten before each call); gemm_ratio
+  select_us_cold / scan_us_cold (_warm)      recommend_category_select_kernel / _scan_kernel alone, as above
+  recommend_us / recommend_cat_us            Seq2SeqAttNN.recommend per batch without / with the categories (CUDA
+                                             events over 32 batches); ratio = with / without
+  rescored_mean / rescored_max               items re-scored exactly per query
+  rebuild_us                                 one rebuild of iext_cat from ps.iext (CUDA events, mean of 10)
 """
 import argparse
 import json
@@ -172,16 +185,119 @@ def window_workloads(model, mwdhm, shape, info, flush):
             print("recommend_probe_window " + json.dumps(res), flush=True)
 
 
+def profiled(calls, names, flush, reps=20):
+    """Mean device time per launch of the kernels whose names contain names[i], over reps rounds of calls."""
+    from torch.profiler import ProfilerActivity, profile
+    for c in calls:
+        nv.call(*c)
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            for c in calls:
+                if flush is not None:
+                    flush.zero_()
+                nv.call(*c)
+        torch.cuda.synchronize()
+    out = {}
+    for e in prof.key_averages():
+        for n in names:
+            if n in e.key:
+                out[n] = e.device_time_total / e.count
+    return [out[n] for n in names]
+
+
+def events_us(fn, n):
+    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    t0.record()
+    for i in range(n):
+        fn(i)
+    t1.record()
+    torch.cuda.synchronize()
+    return t0.elapsed_time(t1) / n * 1e3
+
+
+def category_workloads(model, mwdhm, shape, G, info, flush):
+    N, ps, p = model.N, model.ps, nv.ptr
+    rs = np.random.RandomState(G)
+    model.set_item_categories(rs.randint(0, G, N), G)
+    model._ensure_iext_cat()
+
+    def rebuild(i):
+        model._iext_cat_version = -1
+        model._ensure_iext_cat()
+    rebuild_us = events_us(rebuild, 10)
+    KB = 32
+    for T in (1, 20):
+        bts = []
+        for i in range(4):
+            packed = synth.make_index_batch(N, B, T, 0, mwdhm, seed=300 * T + i)
+            bts.append(model.to_device(torch.from_numpy(packed).pin_memory(), B, T, 0))
+        model.recommend(bts[0], 20, max_per_category=2)                # bts[0]'s session vectors stay in place
+        ws, wc = model._score_buffers(ps.n_pad, False), model._score_buffers(model._cat_n_pad, False)
+        g_plain = profiled([("tcar_score_fwd", p(model.Q), p(ps.iext), p(model.c_ref), None, p(ws["part"]),
+                             p(ws["cmax"]), p(ws["tmax"]), B, ps.N, ps.n_pad, 1, nv.CLUSTER_PAIR)],
+                           ["score_fwd_pair_kernel<1>"], flush)[0]
+        g_cat = profiled([("tcar_score_fwd", p(model.Q), p(model._iext_cat), p(model.c_ref), None, p(wc["part"]),
+                           p(wc["cmax"]), p(wc["tmax"]), B, model._cat_n, model._cat_n_pad, 1, nv.CLUSTER_PAIR)],
+                         ["score_fwd_pair_kernel<1>"], flush)[0]
+        allowed = {"all": None}
+        one = rs.randint(0, G, B).astype(np.int32)
+        allowed["one"] = (np.arange(B + 1, dtype=np.int32), one)
+        m = max(1, G // 10)
+        allowed["10%"] = (np.arange(B + 1, dtype=np.int32) * m,
+                          np.concatenate([rs.choice(G, m, replace=False) for _ in range(B)]).astype(np.int32))
+        for K in (20, 100):
+            plain = events_us(lambda i: model.recommend(bts[i % 4], K), KB)
+            for C in (1, 2, K):
+                for name, cats in allowed.items():
+                    kw = dict(max_per_category=C, categories=cats)
+                    resc = []
+                    for bt in bts:
+                        model.recommend(bt, K, **kw)
+                        resc.append(model.rec_rescored[:B].cpu().numpy())
+                    resc = np.concatenate(resc)
+                    model.recommend(bts[0], K, **kw)
+                    acsr = torch.from_numpy(np.concatenate(cats).astype(np.int32)).cuda() if cats else None
+                    ids = torch.empty(B, K, device=model.dev, dtype=torch.int32)
+                    sc = torch.empty(B, K, device=model.dev)
+                    call = [("tcar_recommend_category", p(wc["cmax"]), p(model.a_ic), p(model.Tq), p(ps.item),
+                             p(ps.content), p(ps.mwdhm), p(model.cat_stats), None, None, None, T, B,
+                             model._cat_n_pad, K, p(model._cat_perm), p(model._item_cat), p(model._cat_off), G,
+                             p(acsr), p(acsr[B + 1:]) if acsr is not None else None, C, p(model._rec_cat_ws), p(ids),
+                             p(sc), p(model.rec_rescored))]
+                    names = ["recommend_category_select_kernel", "recommend_category_scan_kernel"]
+                    sel_c, scan_c = profiled(call, names, flush)
+                    sel_w, scan_w = profiled(call, names, None)
+                    cat_us = events_us(lambda i: model.recommend(bts[i % 4], K, **kw), KB)
+                    res = dict(info, workload=f"{shape} N={N} G={G} B={B} T={T} K={K} C={C} allowed={name}", N=N,
+                               N_cat=model._cat_n, G=G, B=B, T=T, K=K, C=C, allowed=name,
+                               gemm_us_cold=round(g_plain, 2), gemm_cat_us_cold=round(g_cat, 2),
+                               gemm_ratio=round(g_cat / g_plain, 3), select_us_cold=round(sel_c, 2),
+                               scan_us_cold=round(scan_c, 2), select_us_warm=round(sel_w, 2),
+                               scan_us_warm=round(scan_w, 2), recommend_us=round(plain, 1),
+                               recommend_cat_us=round(cat_us, 1), ratio=round(cat_us / plain, 3),
+                               rescored_mean=round(float(resc.mean()), 1), rescored_max=int(resc.max()),
+                               rebuild_us=round(rebuild_us, 1))
+                    print("recommend_probe_category " + json.dumps(res), flush=True)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--shapes", default="globo,mind")
     ap.add_argument("--window", action="store_true", help="publish-time windows (see the module docstring)")
+    ap.add_argument("--category", action="store_true", help="caps and allowed categories (see the module docstring)")
     a = ap.parse_args()
     torch.cuda.set_device(0)
     info = gpu_info()
     flush = torch.empty(256 << 20, device="cuda", dtype=torch.uint8)
     for shape in a.shapes.split(","):
         model, mwdhm = make_model(SHAPES[shape])
+        if a.category:
+            for G in ((461,) if shape == "globo" else (17, 264)):
+                category_workloads(model, mwdhm, shape, G, info, flush)
+            del model
+            torch.cuda.empty_cache()
+            continue
         if a.window:
             window_workloads(model, mwdhm, shape, info, flush)
             del model

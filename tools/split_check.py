@@ -1,6 +1,7 @@
 """Run under torchrun: the split walkers of Seq2SeqAttNN -- test() (catalog-sharded eval_round, one round per `world`
 batches), test_impressions() and recommend_split() (batch i on rank i mod world; once more with 24 h publish-time
-windows) -- on one synthetic split at world N equal the same walkers at world 1.
+windows, once more with at most 2 articles per category) -- on one synthetic split at world N equal the same walkers at
+world 1.
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29513 \\
         tools/split_check.py
@@ -35,9 +36,16 @@ def publish_times(n):
     return [t0 + datetime.timedelta(minutes=int(m)) for m in rs.randint(0, 60 * 24 * 16, n)]
 
 
+def categories(item_dict):
+    """Article -> category over G = 461 codes, every 50th article without one."""
+    rs = np.random.RandomState(12)
+    return {art: int(rs.randint(0, 461)) for art, cnt in item_dict.items() if cnt % 50}
+
+
 def run_walkers(model, split, impressions, item_dict):
     """The walkers on the same batches (Sampler shuffles len_dict in place and draws from `random`); recommend_split
-    also with 24 h publish-time windows (written to recommend_1*.txt)."""
+    also with 24 h publish-time windows (written to recommend_1*.txt) and with at most 2 articles per category
+    (recommend_2*.txt)."""
     def fresh():
         random.seed(7)
         return (copy.deepcopy(split[0]), *split[1:])
@@ -48,6 +56,12 @@ def run_walkers(model, split, impressions, item_dict):
                                                      {"recommend_k": K, "recommend_exclude_clicked": True,
                                                       "recommend_max_age_h": 24.0, "publish_time": publish_times(N),
                                                       "foldnum": 1})}
+    model.reverse_item = {cnt - 1: art for art, cnt in item_dict.items()}
+    model.category_id = categories(item_dict)
+    out["recommend_capped"] = model.recommend_split(None, fresh(), item_dict,
+                                                    {"recommend_k": K, "recommend_exclude_clicked": True,
+                                                     "recommend_max_per_category": 2, "foldnum": 2})
+    model.reverse_item = model.category_id = model._cat_array = None
     model.test(None, fresh(), {})
     out["test"] = model.last_metrics
     return out
@@ -84,6 +98,7 @@ def main():
             return n, f.read().splitlines()
     lines_n, lines_1 = lines(0)
     win_n, win_1 = lines(1)
+    cap_n, cap_1 = lines(2)
     equal = {"test": close(a["test"], b["test"], exact=("coverage",), rel=("loss",)),
              "impressions": close(a["impressions"], b["impressions"], exact=("sessions", "skipped")),
              "recommend": close(a["recommend"], b["recommend"], exact=("sessions",)),
@@ -91,7 +106,10 @@ def main():
              "recommend_window": close(a["recommend_window"], b["recommend_window"],
                                        exact=("sessions", "label_outside")),
              "recommend_window_files": sorted(win_n) == sorted(win_1) and
-             len(win_1) == b["recommend_window"]["sessions"]}
+             len(win_1) == b["recommend_window"]["sessions"],
+             "recommend_capped": close(a["recommend_capped"], b["recommend_capped"], exact=("sessions",)),
+             "recommend_capped_files": sorted(cap_n) == sorted(cap_1) and
+             len(cap_1) == b["recommend_capped"]["sessions"]}
     ok = all(equal.values())
     print(f"rank {rank} split_check " + json.dumps(dict(gpu_info(), world=world, gpus=gpus, backend=dist.get_backend(),
                                                         sessions=SESSIONS, K=K, exclude_clicked=True, world_n=a,
