@@ -33,7 +33,7 @@ extern "C" {
 #define TCAR_TOPK 20      /* cutoff                          (model_combine.py:296,301)                */
 #define TCAR_CHUNK 8      /* items per eval chunk-max                                                   */
 #define TCAR_NCAND_CHUNKS 32 /* chunks re-scored per query (256 candidate items)                        */
-#define TCAR_MAX_EVAL_TILES 32768 /* 128-item tiles per catalog (shard) tcar_eval_topk_certified handles: 4.2 M items */
+#define TCAR_MAX_EVAL_TILES 32768 /* 128-item tiles per catalog (shard) the top-20 selection handles: 4.2 M items */
 /* One shard's evaluation results for <= 512 queries, as ONE contiguous block of 32-bit words (what a rank sends in the
  * single exchange of the catalog-sharded evaluation): planes at fixed offsets, each in the layout the kernels write. */
 #define TCAR_EVAL_OFF_SCORES 0                          /* float [512][20]  top-20 scores                           */
@@ -127,8 +127,8 @@ int tcar_impression_negatives(const int32_t* rows, const int32_t* impr_off, cons
  *                   E[b, n] at element ((n / 8) * 512 + b) * 8 + n % 8 (coalesced epilogue stores; the backward
  *                   kernels read it through a 3-D tensor map); rowsum_part [n_pad/128][512]
  *   mode 1 (eval) : chunkmax [512, n_pad/8] fp32 = max of S over 8 consecutive items, tilemax [512, n_pad/128]
- *                   fp32 = max over 128 consecutive items (first selection level of tcar_eval_topk), rowsum_part
- *                   as above
+ *                   fp32 = max over 128 consecutive items (first selection level of tcar_eval_topk_certified),
+ *                   rowsum_part as above
  *   cluster in {1,2,4}: CTAs per cluster sharing each item tile by TMA multicast (one 128x128 UMMA per CTA);
  *   cluster == TCAR_CLUSTER_PAIR: CTA pairs issuing 256x256 cta_group::2 UMMAs, each CTA streaming half of every
  *   item tile (the production configuration: twice the pipeline depth per byte of shared memory). */
@@ -393,8 +393,8 @@ int tcar_peer_fetch_rows(const int32_t* seq, const int32_t* label, const int32_t
  *            sums (fixed-order sum over n_tiles, as tcar_ce_finish) are stored in the zero pad column 639 of its dQ
  *            rows, so that one reduce-scatter delivers dQ and sum exp to the sessions' rank.
  *     bwd_i: one launch over all present groups (tcar_score_bwd_i_multi); sq_partial (nullable) = sums of squares of
- *            the complete dense gradient.  (TCAR_BWDI_LEGACY=1: the first present group overwrites g_item, later ones
- *            accumulate through tcar_score_bwd_i_acc.)
+ *            the complete dense gradient.  (More than TCAR_MAX_PEERS groups: the first present group overwrites
+ *            g_item, later ones accumulate through tcar_score_bwd_i_acc.)
  *     scatter: tcar_scatter_add_rows_range per group; ids = packed batches [7*B*T idx | 2*B ctx | B label | B*Nn neg],
  *            payload = [a_ic 512x500 | coef 512 | dXi B*T x 256] floats; slot_sq (nullable): [groups][hash_size]. */
 int tcar_score_fwd_groups(const void* q_bf16, long long q_stride, const float* c_ref, long long c_stride,
@@ -465,16 +465,13 @@ int tcar_ce_finish_groups(const float* rowsum_part, const float* rowmax_part, lo
  *     to the lower index), re-score their 256 items exactly in fp32, return top-20 ids/scores ordered by (score desc, id asc) and
  *     n_greater[b] = #candidates scoring strictly above the label (rank-1 whenever rank <= 20).
  *     chunkmax covers the N local items of this catalog shard; item/content/mwdhm are the GLOBAL fp32 tables,
- *     label holds global 0-based ids and item_offset is the global id of local item 0. */
-int tcar_eval_topk(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq, const float* item,
-                   const float* content, const int32_t* mwdhm, const int32_t* label, int32_t* top_ids,
-                   float* top_scores, int32_t* n_greater, int B, int N, int n_pad, int item_offset, void* stream);
-
-/* The same, CERTIFIED: cat_stats[2] (tcar_catalog_stats over the items this call scores, or any superset) bounds the
- * bf16-GEMM error of every chunk maximum; a query whose best un-re-scored chunk could still reach its 20th exact score
- * is flagged in uncertain[b] (1 / 0) with the bound tau[b], and tcar_eval_topk_widen completes it.  Together the two
- * calls return the exact top-20 (np.argsort(pred)[::-1][:20], model_combine.py:301, ties to the lower id) and the exact
- * rank whenever rank <= 20 -- not "with high probability". */
+ *     label holds global 0-based ids and item_offset is the global id of local item 0.
+ *     Certification: cat_stats[2] (tcar_catalog_stats over the items this call scores, or any superset) bounds the
+ *     bf16-GEMM error of every chunk maximum; a query whose best un-re-scored chunk could still reach its 20th exact
+ *     score is flagged in uncertain[b] (1 / 0) with the bound tau[b], and tcar_eval_topk_widen completes it.  Together
+ *     the two calls return the exact top-20 (np.argsort(pred)[::-1][:20], model_combine.py:301, ties to the lower id)
+ *     and the exact rank whenever rank <= 20 -- not "with high probability".  cat_stats = NULL skips the certification
+ *     (uncertain / tau unused). */
 int tcar_eval_topk_certified(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
                              const float* item, const float* content, const int32_t* mwdhm, const int32_t* label,
                              int32_t* top_ids, float* top_scores, int32_t* n_greater, int B, int N, int n_pad,
@@ -486,8 +483,9 @@ int tcar_eval_topk_certified(const float* chunkmax, const float* tilemax, const 
  *                      33rd entry (id -2) whose value bounds every chunk of the range that is NOT listed.  No re-scoring.
  *   tcar_eval_rescore  (query owner) `lists` such lists per query, list_stride words apart: the 32 best entries overall
  *                      are re-scored exactly from the fp32 tables (global ids, N_total items), top-20 / n_greater as in
- *                      tcar_eval_topk; the 33rd best value bounds everything else, queries it cannot certify are flagged
- *                      (uncertain, tau) for tcar_eval_topk_widen on every item range.  lists * 33 <= 512. */
+ *                      tcar_eval_topk_certified; the 33rd best value bounds everything else, queries it cannot
+ *                      certify are flagged (uncertain, tau) for tcar_eval_topk_widen on every item range.
+ *                      lists * 33 <= 512. */
 int tcar_eval_select(const float* chunkmax, const float* tilemax, float* sel_vals, int32_t* sel_ids, int B, int N,
                      int n_pad, int item_offset, void* stream);
 int tcar_eval_rescore(const float* sel_vals, const int32_t* sel_ids, int lists, long long list_stride, const float* a_ic,
@@ -541,9 +539,9 @@ int tcar_eval_merge_flagged(const void* blocks, long long block_words, const int
 /* (6b) candidate re-ranking: session b's list is cand_ids[cand_off[b] .. cand_off[b+1]) (0-based item ids, at most
  *      max_len <= TCAR_RERANK_MAXL entries; duplicates allowed).  a_ic / Tq are the session vectors of
  *      tcar_build_query; item / content / mwdhm the fp32 tables of the full-catalog evaluation.
- *        scores [nnz]   exact fp32 score of cand_ids[j], in input order: the arithmetic of tcar_eval_topk's re-scoring,
- *                       so a candidate scores bit for bit what the full-catalog top-20 reports for it
- *                       (model_combine.py:138);
+ *        scores [nnz]   exact fp32 score of cand_ids[j], in input order: the arithmetic of the top-20 re-scoring
+ *                       (tcar_eval_topk_certified), so a candidate scores bit for bit what the full-catalog top-20
+ *                       reports for it (model_combine.py:138);
  *        ranked [nnz]   each list's ids ordered by (score desc, id asc, input position asc);
  *      with label != NULL (label[b] = the positive, every other entry of the list is a negative):
  *        label_rank [B] 1 + #(negatives scoring strictly above the label): the label wins ties (util.py:14);
@@ -557,13 +555,14 @@ int tcar_rerank(const float* a_ic, const float* Tq, const float* item, const flo
 
 /* (6c) top-K recommendation: the exact top-K of the whole catalog per session, without the excluded ids.
  *      chunkmax / tilemax: the eval-mode scoring GEMM (tcar_score_fwd mode 1) over the N items for these B queries;
- *      a_ic / Tq / item / content / mwdhm as for tcar_eval_topk; cat_stats: tcar_catalog_stats over the N items.
+ *      a_ic / Tq / item / content / mwdhm as for tcar_eval_topk_certified; cat_stats: tcar_catalog_stats over the N
+ *      items.
  *      Exclusions of session b (0-based ids; duplicates and ids outside [0, N) allowed): x_ids[x_off[b] .. x_off[b+1])
  *      when x_off != NULL, and clicks[b*T .. b*T+T) - 1 when clicks != NULL (the 1-based click ids of the packed
  *      batch, T clicks per session); at most TCAR_RECOMMEND_MAXX entries in all, a session with more is not processed
  *      (outputs left as they are).
  *        ids [B][K]       item ids ordered by (exact score desc, id asc); -1 past the end of a small catalog
- *        scores [B][K]    their exact fp32 scores (the arithmetic of tcar_eval_topk's re-scoring, so bit for bit what
+ *        scores [B][K]    their exact fp32 scores (the arithmetic of the top-20 re-scoring, so bit for bit what
  *                         eval_step and tcar_rerank report for the same item); -inf past the end
  *        rescored [B]     (nullable) items re-scored exactly: the width of the band the error bound left open.
  *      1 <= K <= TCAR_RECOMMEND_MAXK.  workspace: tcar_recommend_ws_bytes(B) bytes (a buffer sized for B serves every

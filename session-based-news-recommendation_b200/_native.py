@@ -91,7 +91,6 @@ SIGNATURES = {
     "tcar_adam_item_rows": [_P] * 6 + [_F, _F, _P, _P, _I, _P, _I, _P, _I, _P],
     "tcar_adam_item_rows_groups": [_P] * 6 + [_F, _F, _P, _P, _LL, _P, _I, _I, _I, _P, _I, _I, _P],
     "tcar_refresh_iext_items": [_P, _P, _I, _P],
-    "tcar_eval_topk": [_P] * 11 + [_I] * 4 + [_P],
     "tcar_eval_topk_certified": [_P] * 11 + [_I] * 4 + [_P] * 3 + [_P],
     "tcar_eval_select": [_P] * 4 + [_I] * 4 + [_P],
     "tcar_eval_rescore": [_P, _P, _I, _LL] + [_P] * 9 + [_I, _I] + [_P] * 3 + [_P],

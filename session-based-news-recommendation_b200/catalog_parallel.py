@@ -77,8 +77,6 @@ class CatalogShardedTraining:
         # gathered one step early into the second buffer pair
         import os
         self.cat_lookahead = os.environ.get("TCAR_CATALOG_LOOKAHEAD", "0") == "1"
-        self._scatter_merged = os.environ.get("TCAR_SCATTER_LOOP", "0") != "1"
-        self._neg_side = os.environ.get("TCAR_CAT_NEG_SIDE", "0") == "1"     # opt-in: negative-feedback loss on the auxiliary stream
         self._ids_n = torch.zeros(1, device=dev, dtype=torch.int32)
         self._ids_all_n = torch.zeros(1, device=dev, dtype=torch.int32)
         self._cat_pre = None               # {"bt", "counts", "L"} of the batch whose ids / rows / forward are ahead
@@ -226,22 +224,9 @@ class CatalogShardedTraining:
         if B > 0 and not ahead:
             self._session_forward(bt)
         mark("session_fwd")
-        neg_done = None
-        if B > 0 and not self._neg_side:
+        if B > 0:
             nv.counted_call("tcar_neg_loss", 1, p(self.a_ic), p(ps.item), p(ps.content), p(bt.neg), None,
                             p(self.negloss), p(self.loss), p(self.coef), p(self.dA_neg), B, Nn)
-        elif B > 0:
-            # negative-feedback loss + its gradient wrt a_ic: needs a_ic and the (fetched) item rows only -- on the
-            # auxiliary stream beside the exchanges and the scoring GEMMs
-            main = torch.cuda.current_stream()
-            fork = torch.cuda.Event()
-            fork.record(main)
-            self._aux.wait_event(fork)
-            with torch.cuda.stream(self._aux):
-                nv.counted_call("tcar_neg_loss", 1, p(self.a_ic), p(ps.item), p(ps.content), p(bt.neg), None,
-                                p(self.negloss), p(self.loss), p(self.coef), p(self.dA_neg), B, Nn)
-                neg_done = torch.cuda.Event()
-                neg_done.record(self._aux)
         if on:
             self._gather(self._qc_all.view(-1), self._qc)
         mark("gather_q")
@@ -293,12 +278,9 @@ class CatalogShardedTraining:
         else:
             dq_raw = self._dq_all[0]
         if B > 0:
-            # CE = log(sum) (+ shift ln 2 for rows the guard shifted) from the strided sums column; the negative-feedback
-            # term was launched beside the scoring phases (neg_done)
+            # CE = log(sum) (+ shift ln 2 for rows the guard shifted) from the strided sums column
             nv.counted_call("tcar_ce_from_sums", 1, p(dq_raw[:, KEXT - 1:]), KEXT,
                             p(self._rowmax_all[me]) if guard else None, p(self.sumexp), p(self.ce), B)
-            if neg_done is not None:
-                torch.cuda.current_stream().wait_event(neg_done)
             nv.counted_call("tcar_loss_combine", 1, p(self.ce), p(self.negloss), p(self.loss), B)
             nv.counted_call("tcar_score_bwd_finish", 1, p(dq_raw), p(self.sumexp), p(self.dA_neg), p(self.a_ic),
                             p(ps.ct_tab), p(ps.item), p(ps.content), p(ps.mwdhm), p(bt.label), p(self.d_a_ic),
@@ -331,8 +313,8 @@ class CatalogShardedTraining:
         mark("score_bwd_i")
         # ---- the sparse rows (clicks, labels, negatives) of every rank's sessions that fall into the owned ranges
         # all source ranks against ONE hash table (tcar_scatter_add_rows_multi: three launches per step instead of
-        # three per source rank); TCAR_SCATTER_LOOP=1 keeps the per-rank passes (A/B switch)
-        merged = self._scatter_merged and ng > 1
+        # three per source rank)
+        merged = ng > 1
         ent = Bmax * T + Bmax + Bmax * Nn
         self._alloc_scatter(R * ent if merged else ent)
         nsq = self.hash_size if merged else R * self.hash_size

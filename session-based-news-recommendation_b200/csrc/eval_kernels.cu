@@ -613,13 +613,13 @@ eval_topk_kernel(const float* chunkmax, const float* tilemax, const float* __res
     }
 }
 
-// Second stage for the queries tcar_eval_topk could not certify: every chunk whose maximum reaches tau[b] = s20 - eps_b
-// is re-scored exactly (tiles below tau are skipped by their tile maximum), 32 chunks at a time, and merged into a
-// running top-20 by (score desc, id asc); n_greater is counted over the same exact scores.  The result is the exact
-// top-20 of the whole catalog (items below tau cannot reach the 20th score already found).  Cost grows with the number
-// of near-ties (in the limit a full exact scan), so a flagged query is spread over TCAR_WIDEN_SPLITS CTAs, each taking
-// a contiguous range of tiles and leaving a partial list in the workspace; the merge kernel behind it combines them.
-// A certified query costs nothing (its CTAs return at once).
+// Second stage for the queries tcar_eval_topk_certified could not certify: every chunk whose maximum reaches
+// tau[b] = s20 - eps_b is re-scored exactly (tiles below tau are skipped by their tile maximum), 32 chunks at a time,
+// and merged into a running top-20 by (score desc, id asc); n_greater is counted over the same exact scores.  The
+// result is the exact top-20 of the whole catalog (items below tau cannot reach the 20th score already found).  Cost
+// grows with the number of near-ties (in the limit a full exact scan), so a flagged query is spread over
+// TCAR_WIDEN_SPLITS CTAs, each taking a contiguous range of tiles and leaving a partial list in the workspace; the
+// merge kernel behind it combines them.  A certified query costs nothing (its CTAs return at once).
 constexpr int WQ_CAP = 4096;        // chunk queue: one sweep of 256 tiles x 16 chunks
 constexpr int WSPLIT = TCAR_WIDEN_SPLITS;
 // workspace per group: partial lists [S][512][20] ids | scores, counts [S][512], then one ticket per query (zero between
@@ -1795,15 +1795,6 @@ recommend_category_scan_kernel(const float* chunkmax, const float* __restrict__ 
 
 using namespace tcar;
 #define STREAM static_cast<cudaStream_t>(stream)
-
-extern "C" int tcar_eval_topk(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
-                              const float* item,
-                              const float* content, const int32_t* mwdhm, const int32_t* label, int32_t* top_ids,
-                              float* top_scores, int32_t* n_greater, int B, int N, int n_pad, int item_offset,
-                              void* stream) {
-    return tcar_eval_topk_certified(chunkmax, tilemax, a_ic, Tq, item, content, mwdhm, label, top_ids, top_scores,
-                                    n_greater, B, N, n_pad, item_offset, nullptr, nullptr, nullptr, stream);
-}
 
 extern "C" int tcar_eval_topk_certified(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
                                         const float* item, const float* content, const int32_t* mwdhm,

@@ -6,7 +6,6 @@
 #include <cuda_runtime.h>
 #include <cuda.h>
 #include <stdint.h>
-#include <stdlib.h>
 #include <string.h>
 #include "tcar_b200.h"
 #include "launch.cuh"
@@ -138,10 +137,8 @@ extern "C" int tcar_score_fwd_groups_guarded(const void* q_bf16, long long q_str
     if (!n_rows || groups < 1) return TCAR_ERR_ARG;
     int present = 0;
     for (int g = 0; g < groups; ++g) present += n_rows[g] > 0;
-    // several groups (or TCAR_FWD_MULTI=1): one launch over all of them; TCAR_FWD_MULTI=0 keeps the per-group launches
-    const char* env = getenv("TCAR_FWD_MULTI");
-    const bool multi = cluster == TCAR_CLUSTER_PAIR && groups <= TCAR_MAX_PEERS && (q_stride & 7) == 0 &&
-                       (env ? env[0] == '1' : present > 1);
+    // several groups: one launch over all of them
+    const bool multi = cluster == TCAR_CLUSTER_PAIR && groups <= TCAR_MAX_PEERS && (q_stride & 7) == 0 && present > 1;
     if (multi)
         return tcar_score_fwd_multi(q_bf16, q_stride, c_ref, c_stride, iext_bf16, e_out, e_stride, rowsum_part,
                                     part_stride, rowmax_part, rowmax, n_rows, groups, n_items, n_pad, stream);
@@ -166,10 +163,8 @@ extern "C" int tcar_score_bwd_q_groups(const void* e_bf16, long long e_stride, c
     int present = 0;
     for (int g = 0; g < groups; ++g) present += n_rows[g] > 0;
     // several groups: one launch over all of them (needs the groups' dQ blocks back to back and a part buffer of
-    // tcar_score_bwd_q_multi_part_elems floats); TCAR_BWDQ_LOOP=1 keeps the per-group launches (A/B switch)
-    const char* loop_env = getenv("TCAR_BWDQ_LOOP");
-    const bool multi = present > 1 && groups <= 16 && dq_stride == (long long)TCAR_QROWS * TCAR_KEXT &&
-                       !(loop_env && loop_env[0] == '1');
+    // tcar_score_bwd_q_multi_part_elems floats)
+    const bool multi = present > 1 && groups <= 16 && dq_stride == (long long)TCAR_QROWS * TCAR_KEXT;
     if (multi) {
         const int rc = tcar_score_bwd_q_multi(e_bf16, e_stride, iext_bf16, part, dq, n_rows, groups, n_pad, stream);
         if (rc) return rc;
@@ -197,10 +192,9 @@ extern "C" int tcar_score_bwd_i_groups(const void* e_bf16, long long e_stride, c
                                        float* g_item, float* sq_partial, const int* n_rows, int groups, int n_items,
                                        int n_pad, void* stream) {
     if (!n_rows || groups < 1) return TCAR_ERR_ARG;
-    // all groups concatenated along K in ONE launch, the gradient written once (score_bwd_i_tma_kernel<MULTI>);
-    // TCAR_BWDI_LEGACY=1 keeps one launch per group with read-modify-write accumulation (A/B switch)
-    const char* legacy = getenv("TCAR_BWDI_LEGACY");
-    if (groups <= TCAR_MAX_PEERS && !(legacy && legacy[0] == '1'))
+    // all groups concatenated along K in ONE launch, the gradient written once (score_bwd_i_tma_kernel<MULTI>); more
+    // groups than that kernel takes: one launch per group with read-modify-write accumulation
+    if (groups <= TCAR_MAX_PEERS)
         return tcar_score_bwd_i_multi(e_bf16, e_stride, qs_bf16, qs_stride, g_item, sq_partial, n_rows, groups, n_items,
                                       n_pad, stream);
     int done = 0, last = -1;

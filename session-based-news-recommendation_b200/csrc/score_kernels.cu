@@ -1443,17 +1443,11 @@ static int sm_count() {
     return n;
 }
 
-// L2 prefetch distance (stages) of the streamed GEMM operands; TCAR_TMA_PREFETCH_<FWD|BWDQ|BWDI>=n, else
-// TCAR_TMA_PREFETCH=n, overrides the default (0 = off); read per call so that one process can A/B it
-static int tma_prefetch_depth(int dflt, const char* which) {
-    const char* e = getenv(which);
-    if (!(e && e[0])) e = getenv("TCAR_TMA_PREFETCH");
-    if (e && e[0]) {
-        const int v = atoi(e);
-        return v < 0 ? 0 : (v > 64 ? 64 : v);
-    }
-    return dflt;
-}
+// L2 prefetch distance (stages) of the streamed GEMM operands (DESIGN §4.1): the forward gains equally at distances 4
+// to 12 and loses from 16 on; the dQ GEMM is bound by the L2 -> SM fill, where prefetches only add requests
+constexpr int PREFETCH_FWD = 12;
+constexpr int PREFETCH_BWD_Q = 0;
+constexpr int PREFETCH_BWD_I = 8;
 
 template <int CL>
 static int launch_fwd(const CUtensorMap& mq, const CUtensorMap& mi, const FwdParams& p, int n_clusters,
@@ -1544,7 +1538,7 @@ extern "C" int tcar_score_fwd_guarded(const void* q_bf16, const void* iext_bf16,
         const int mtiles = (n_rows + BM - 1) / BM;
         p.groups = (mtiles + 1) / 2;
         p.mode = mode;
-        p.prefetch = tma_prefetch_depth(12, "TCAR_TMA_PREFETCH_FWD");
+        p.prefetch = PREFETCH_FWD;
         int n_pairs = ((sm_count() / 2) / p.groups) * p.groups;
         if (n_pairs < p.groups) n_pairs = p.groups;
         if (n_pairs / p.groups > p.n_tiles) n_pairs = p.n_tiles * p.groups;
@@ -1606,7 +1600,7 @@ extern "C" int tcar_score_fwd_window(const void* q_bf16, const void* iext_bf16, 
     const int mtiles = (n_rows + BM - 1) / BM;
     p.groups = (mtiles + 1) / 2;
     p.mode = 2;
-    p.prefetch = tma_prefetch_depth(12, "TCAR_TMA_PREFETCH_FWD");
+    p.prefetch = PREFETCH_FWD;
     p.item_time = item_time;
     p.win_lo = win_lo;
     p.win_hi = win_hi;
@@ -1691,7 +1685,7 @@ static int score_fwd_multi_impl(const void* q_bf16, long long q_stride, const fl
     p.n_tiles = n_pad / P_BN;
     p.e_pitch = n_pad;
     p.n_rb = nrb;
-    p.prefetch = tma_prefetch_depth(12, "TCAR_TMA_PREFETCH_FWD");
+    p.prefetch = PREFETCH_FWD;
     int n_pairs = sm_count() / 2;
     if ((long long)n_pairs > (long long)nrb * p.n_tiles) n_pairs = nrb * p.n_tiles;
     const bool eval_mode = e_out == nullptr;
@@ -1740,7 +1734,7 @@ extern "C" int tcar_score_bwd_q(const void* e_bf16, const void* iext_bf16, float
     p.part = part;
     p.mtiles = (n_rows + BM - 1) / BM;
     p.splits = tcar_score_bwd_q_splits(n_rows, n_pad);
-    p.prefetch = tma_prefetch_depth(0, "TCAR_TMA_PREFETCH_BWDQ");
+    p.prefetch = PREFETCH_BWD_Q;
     p.kb_total = n_pad / BK;
     p.kb_per = (p.kb_total + p.splits - 1) / p.splits;
     p.rows_total = QROWS;
@@ -1792,7 +1786,7 @@ extern "C" int tcar_score_bwd_q_multi(const void* e_bf16, long long e_stride, co
     if (splits > p.kb_total) splits = p.kb_total;
     if (splits < 1) splits = 1;
     p.splits = splits;
-    p.prefetch = tma_prefetch_depth(0, "TCAR_TMA_PREFETCH_BWDQ");
+    p.prefetch = PREFETCH_BWD_Q;
     p.kb_per = (p.kb_total + splits - 1) / splits;
     p.rows_total = groups * QROWS;
     TCAR_SET_SMEM_ONCE(score_bwd_q_kernel<true>, Q_SMEM);
@@ -1833,13 +1827,6 @@ static int make_map_g(CUtensorMap* m, float* base, uint64_t rows) {
 
 static int bwd_i_grid(int n_pad) {
     int grid = (sm_count() / 2) * 2;
-    // TCAR_BWD_I_CTAS=n: leave SMs free for the session-side backward running beside this GEMM (train_step's
-    // bwd_overlap); read per call so that one process can A/B it
-    const char* e = getenv("TCAR_BWD_I_CTAS");
-    if (e && e[0]) {
-        const int v = atoi(e) & ~1;
-        if (v >= 2 && v < grid) grid = v;
-    }
     const int n_tiles = n_pad / BM;
     if (grid > 2 * n_tiles) grid = 2 * n_tiles;
     return grid;
@@ -1850,12 +1837,6 @@ extern "C" int tcar_score_bwd_i_ctas(int n_pad) { return bwd_i_grid(n_pad); }
 extern "C" int tcar_score_bwd_i(const void* e_bf16, const void* qs_bf16, float* g_item, float* sq_partial, int n_rows,
                                 int n_items, int n_pad, void* stream_) {
     return tcar_score_bwd_i_acc(e_bf16, qs_bf16, g_item, sq_partial, n_rows, n_items, n_pad, 0, stream_);
-}
-
-// TCAR_BWDI_LEGACY=1 keeps the first kernel (thread <-> row stores, one launch per group): the A/B switch
-static bool bwd_i_legacy() {
-    const char* e = getenv("TCAR_BWDI_LEGACY");
-    return e && e[0] == '1';
 }
 
 extern "C" int tcar_score_bwd_i_multi(const void* e_bf16, long long e_stride, const void* qs_bf16, long long qs_stride,
@@ -1869,7 +1850,7 @@ extern "C" int tcar_score_bwd_i_multi(const void* e_bf16, long long e_stride, co
     p.n_items = n_items;
     p.n_tiles = n_pad / BM;
     p.groups = groups;
-    p.prefetch = tma_prefetch_depth(8, "TCAR_TMA_PREFETCH_BWDI");
+    p.prefetch = PREFETCH_BWD_I;
     int present = 0, only = -1;
     for (int g = 0; g < TCAR_MAX_PEERS; ++g) {
         const int b = g < groups ? n_rows[g] : 0;
@@ -1910,7 +1891,7 @@ extern "C" int tcar_score_bwd_i_acc(const void* e_bf16, const void* qs_bf16, flo
                                     int n_rows, int n_items, int n_pad, int accumulate, void* stream_) {
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     if (n_rows < 1 || n_rows > QROWS || n_pad % 256 != 0) return TCAR_ERR_ARG;
-    if (!accumulate && !bwd_i_legacy())
+    if (!accumulate)
         return tcar_score_bwd_i_multi(e_bf16, 0, qs_bf16, 0, g_item, sq_partial, &n_rows, 1, n_items, n_pad, stream_);
     CUtensorMap me, mq;
     int rc = make_map_e(&me, e_bf16, n_pad, BK, BM / 8);

@@ -198,28 +198,22 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         # `_aux`: independent branches of the backward / update (query-path gradients, small-tensor Adam) that run
         # beside the main chain; joined by events, results do not depend on the interleaving (disjoint buffers)
         self._aux = torch.cuda.Stream(device=dev)
-        self.branch_streams = os.environ.get("TCAR_BRANCH_STREAMS", "1") != "0"
-        # session-side backward beside the dense item-gradient GEMM (see backward()); A/B: tools/step_ab.py
-        self.bwd_overlap = os.environ.get("TCAR_BWD_OVERLAP", "1") != "0"
         self._la_events = None
         self._update_done = None           # event recorded on `_side` after the pending item update
         self._ahead_done = None            # event recorded on `_ahead` after the prefetched session forward
         self._prefetched = None            # the Batch whose session forward has already been launched
-        self.adam_overlap_ctas = int(os.environ.get("TCAR_ADAM_OVERLAP_CTAS", "64"))
-        self.ahead_priority = os.environ.get("TCAR_AHEAD_PRIORITY", "1") != "0"
+        self.adam_overlap_ctas = 64
         # multi-GPU training layout: "dp" = data parallel + gradient all-reduce (north_star), "catalog" = the softmax
         # sharded over the item catalog (catalog_parallel.py; SURVEY 8e row 2)
         # overflow guard of the full-catalog softmax (TCAR_EXP_LIMIT2 in include/tcar_b200.h): TF subtracts the row
         # maximum (model_combine.py:145), the scoring kernel shifts by the label score; rows whose best candidate
         # outscores the label by more than 55 nats are re-run shifted by their maximum (two empty launches otherwise)
         self.softmax_guard = bool(args.get("softmax_guard", os.environ.get("TCAR_SOFTMAX_GUARD", "1") != "0"))
-        self.eval_certify = os.environ.get("TCAR_EVAL_CERTIFY", "1") != "0"
-        self.eval_two_stage = os.environ.get("TCAR_EVAL_TWO_STAGE", "1") != "0"
-        self.eval_group_launch = os.environ.get("TCAR_EVAL_GROUP_LAUNCH", "1") != "0"
+        self.eval_group_launch = True
         # single item range, <= 512 queries: the fused CTA-per-query kernel (121 us) beats warp-per-query selection +
         # re-scoring (63 + 72 us: 512 warps cannot fill the GPU); the sharded rounds select for world x 512 queries per
         # launch, where the warp kernel's time stays flat (tcar_eval_select_groups)
-        self.eval_warp_select = os.environ.get("TCAR_EVAL_WARP_SELECT", "0") != "0"
+        self.eval_warp_select = False
         self.train_parallel = "dp"
         self._item_table_synced = True
         mode = args.get("train_parallel") or "dp"
@@ -433,7 +427,7 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         else:
             self._session_forward(bt)
         ws = self._score_buffers(ps.n_pad, True)
-        if self.branch_streams and self.world == 1:
+        if self.world == 1:
             # the negative-feedback term needs a_ic and item rows only: beside the scoring GEMM on the auxiliary stream
             # (its CTAs use no shared memory to speak of, so they fit next to the GEMM's), off the critical path
             main = torch.cuda.current_stream()
@@ -494,10 +488,9 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         nv.counted_call("tcar_score_bwd_finish", 1, p(self.dq_raw), p(self.sumexp), p(self.dA_neg), p(self.a_ic),
                         p(ps.ct_tab), p(ps.item), p(ps.content), p(ps.mwdhm), p(bt.label), p(self.d_a_ic),
                         p(self.d_a_pt), p(self.dTq), p(self.Qs), B)
-        if self.bwd_overlap and self.world == 1:
+        if self.world == 1:
             # the dense item gradient GEMM (HBM-bound, persistent CTAs) on the side stream, the session-side backward
-            # (a chain of short latency-bound kernels that only needs d a_ic / d a_pt / dTq) beside it on this stream;
-            # TCAR_BWD_I_CTAS < 148 leaves whole SMs to the chain's GEMMs (the persistent CTAs own all shared memory)
+            # (a chain of short latency-bound kernels that only needs d a_ic / d a_pt / dTq) beside it on this stream
             main = torch.cuda.current_stream()
             fork = torch.cuda.Event()
             fork.record(main)
@@ -530,8 +523,7 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         nv.col_jobs([(dz_a, self.a_ic, dz_a, g["b_a"], B, XW, XW, 0), (dz_p, self.a_pt, dz_p, g["b_p"], B, PW, PW, 0)])
         # split the reduction dimension across CTAs only when one CTA would walk more than ~48 K blocks of 32: a split
         # costs a second (reduction) launch, which is worth it for long reductions only
-        old_policy = os.environ.get("TCAR_OLD_SPLITS") == "1"
-        ksp = (4 if B > 128 else 1) if old_policy else self._splits_for(B)
+        ksp = self._splits_for(B)
         nv.gemm_group([
             pr([(self.pooled, XW, 1, dz_a, None, XW, 1, B)], XW, XW, g["W_a"], XW, splits=ksp, part=self._part(XW, XW, ksp)),
             pr([(self.pooled_t, PW, 1, dz_p, None, PW, 1, B)], PW, PW, g["W_p"], PW, splits=ksp, part=self._part(PW, PW, ksp)),
@@ -543,7 +535,7 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         de = self.de.view(-1)                      # kernel layout: [3][B*T] with the ACTUAL B*T as stride
         dzq = self.dq
         main = torch.cuda.current_stream()
-        branch = self._aux if (self.branch_streams and self.world == 1) else main
+        branch = self._aux if self.world == 1 else main
         if branch is not main:
             ev = torch.cuda.Event()
             ev.record(main)
@@ -566,7 +558,7 @@ class Seq2SeqAttNN(CatalogShardedTraining):
                 ev_b.record(branch)
         # every gradient that consumes dU1 / dU2, one launch: four weight gradients (reduction over the B*T clicks
         # split across CTAs) and three data gradients
-        msp = max(1, min(16, M // 512)) if old_policy else self._splits_for(M)
+        msp = self._splits_for(M)
         self._part_off = 0
         nv.gemm_group([
             # rows 250..499 of X^T dU1 / X^T dU2 (the content half of X) are W_c's and W2's gradients: second
@@ -705,17 +697,14 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             done = torch.cuda.Event(enable_timing=timed)
             done.record(self._side)
         self._update_done = done
-        if self.ahead_priority:
-            self._ahead.wait_event(fork)
-            with torch.cuda.stream(self._ahead):
-                self._session_forward(next_bt, prefetch=True)
-                adone = torch.cuda.Event(enable_timing=timed)
-                adone.record(self._ahead)
-            self._ahead_done = adone
-            if timed:
-                self._la_events.append((fork, done, adone))
-        else:
+        self._ahead.wait_event(fork)
+        with torch.cuda.stream(self._ahead):
             self._session_forward(next_bt, prefetch=True)
+            adone = torch.cuda.Event(enable_timing=timed)
+            adone.record(self._ahead)
+        self._ahead_done = adone
+        if timed:
+            self._la_events.append((fork, done, adone))
         self._prefetched = next_bt
 
     def _update_small(self):
@@ -743,7 +732,7 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             loss = self.loss[:0]
         else:
             loss, _ = self.forward_train(bt)
-            if self.world == 1 and self.branch_streams:
+            if self.world == 1:
                 # the small-tensor update (norms, step counter, Adam, weight split) needs theta_g only: it runs on the
                 # auxiliary stream beside the scatter-add of the sparse item rows
                 self.backward(bt, scatter=False)
@@ -860,10 +849,6 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         ps, p = self.ps, nv.ptr
         bi = block.view(torch.int32)
         ids, sc, ngt = p(bi[nv.EVAL_OFF_IDS:]), p(block[nv.EVAL_OFF_SCORES:]), p(bi[nv.EVAL_OFF_NGT:])
-        if not self.eval_certify:            # A/B switch (TCAR_EVAL_CERTIFY=0): the uncertified 32-chunk selection
-            nv.counted_call("tcar_eval_topk", 1, p(ws["cmax"]), p(ws["tmax"]), p(a_ic), p(Tq), p(ps.item),
-                            p(ps.content), p(ps.mwdhm), p(label), ids, sc, ngt, B, n_loc, n_pad, lo)
-            return
         if self.eval_warp_select:
             # selection by one warp per query (tcar_eval_select), exact re-scoring + certification by one CTA per query
             sel = self._sel1
@@ -928,7 +913,7 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             self.Q, self.c_ref, self.a_ic, self.Tq = keep
         mine[4][:bt.B].copy_(bt.label)
 
-    # Two-stage round (default, `eval_two_stage`): an item range only SELECTS its 32 best chunks per query (bf16 chunk
+    # Two-stage round (the default): an item range only SELECTS its 32 best chunks per query (bf16 chunk
     # maxima, no re-scoring); the query's owner merges the ranges' lists and re-scores the 32 best chunks overall from
     # the replicated fp32 tables -- the exact re-scoring (256 candidate rows per query, the bandwidth-heavy part) is done
     # once per query instead of once per (query, item range).  Queries the owner cannot certify are widened by every
@@ -1098,7 +1083,7 @@ class Seq2SeqAttNN(CatalogShardedTraining):
                                 sumexp=blk[nv.EVAL_OFF_SUMEXP:], ce=self._ce_scratch, rowmax=blk[nv.EVAL_OFF_ROWMAX:])
             self._topk(ws, ag, Tg, lg, blk, Bg, n_loc, n_pad, lo)
 
-    def eval_round(self, bt, counts, shard=None, two_stage=None, next_bt=None):
+    def eval_round(self, bt, counts, shard=None, two_stage=True, next_bt=None):
         """Catalog-sharded evaluation that SCALES: every rank brings its OWN batch of <= 512 queries (bt; B may be 0 in
         the last round), so one round evaluates sum(counts) queries.  counts[g] = queries of rank g (the same list on
         every rank).  Per round (two-stage form, the default):
@@ -1122,7 +1107,6 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             self.sync_item_table()
         on = parallel.is_distributed(self.world)
         R, me = (self.world, self.rank) if on else (1, 0)
-        two_stage = self.eval_two_stage if two_stage is None else two_stage
         two_stage = two_stage and R * nv.EVAL_NSEL <= 512
         counts = [int(c) for c in counts]
         B = bt.B
@@ -1197,12 +1181,11 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         mark("merge")
         return out
 
-    def eval_round_virtual(self, bts, two_stage=None):
+    def eval_round_virtual(self, bts, two_stage=True):
         """Single-GPU emulation of eval_round over V = len(bts) ranks (tests): the same kernels with the same shard
         offsets and block layouts, the collectives replaced by copies.  Returns the per-rank results."""
         V = len(bts)
         counts = [b.B for b in bts]
-        two_stage = self.eval_two_stage if two_stage is None else two_stage
         two_stage = two_stage and V * nv.EVAL_NSEL <= 512
         self._alloc_eval_round(1)
         eq_all = torch.zeros(V, self.EQ_BYTES, device=self.dev, dtype=torch.uint8)

@@ -12,7 +12,7 @@ from ._native import CHUNK, RECOMMEND_MAXG
 
 def cau_metrics(preds, labels, cutoff=20):
     """util.py:8-18 on a materialised score matrix (used by tests / debugging; the hot path gets the rank from
-    tcar_eval_topk's n_greater instead)."""
+    tcar_eval_topk_certified's n_greater instead)."""
     preds = np.asarray(preds)
     recall, mrr, ndcg = [], [], []
     for row, lab in zip(preds, labels):

@@ -134,9 +134,10 @@ def test_score_bwd_i(native, B, N):
 
 
 @pytest.mark.parametrize("B,N", [(512, 5000), (77, 2333)])
-def test_score_bwd_i_tma_epilogue_equals_the_row_store_kernel(native, B, N, monkeypatch):
-    """The staged TMA-store epilogue (default) and the first kernel (thread <-> row stores, TCAR_BWDI_LEGACY=1) run the
-    same MMAs in the same order: gradient and per-CTA sums of squares bit-identical; rows beyond the table untouched."""
+def test_score_bwd_i_tma_epilogue_equals_the_row_store_kernel(native, B, N):
+    """The staged TMA-store epilogue (tcar_score_bwd_i) and the row-store kernel (thread <-> row stores; what
+    tcar_score_bwd_i_acc runs with accumulate = 1, here into a zero gradient, where 0 + x is exact) run the same MMAs
+    in the same order: gradient and per-CTA sums of squares bit-identical; rows beyond the table untouched."""
     g = torch.Generator(device="cuda").manual_seed(B + N)
     n_pad = (N + 255) // 256 * 256
     E = torch.zeros(QROWS, n_pad, device="cuda", dtype=torch.bfloat16)
@@ -144,26 +145,25 @@ def test_score_bwd_i_tma_epilogue_equals_the_row_store_kernel(native, B, N, monk
     Qs = torch.zeros(QROWS, 256, device="cuda", dtype=torch.bfloat16)
     Qs[:B, :250] = (torch.randn(B, 250, device="cuda", generator=g) * 0.2).bfloat16()
     Eb = e_to_blocked(E)
-    out = {}
-    for mode in ("1", "0"):
-        monkeypatch.setenv("TCAR_BWDI_LEGACY", mode)
-        gi = torch.full((N + 1 + 300, 256), 7.0, device="cuda")          # 300 guard rows behind the table
-        sqp = torch.zeros(native.lib().tcar_score_bwd_i_ctas(n_pad), device="cuda")
-        native.call("tcar_score_bwd_i", native.ptr(Eb), native.ptr(Qs), native.ptr(gi), native.ptr(sqp), B, N, n_pad)
-        torch.cuda.synchronize()
-        out[mode] = (gi, sqp)
-    monkeypatch.delenv("TCAR_BWDI_LEGACY")
-    assert torch.equal(out["0"][0][1: N + 1], out["1"][0][1: N + 1])
-    assert torch.equal(out["0"][1], out["1"][1])
-    assert (out["0"][0][0] == 7.0).all() and (out["0"][0][N + 1:] == 7.0).all()
+    ctas = native.lib().tcar_score_bwd_i_ctas(n_pad)
+    gi = torch.full((N + 1 + 300, 256), 7.0, device="cuda")              # 300 guard rows behind the table
+    sqp = torch.zeros(ctas, device="cuda")
+    native.call("tcar_score_bwd_i", native.ptr(Eb), native.ptr(Qs), native.ptr(gi), native.ptr(sqp), B, N, n_pad)
+    ref = torch.zeros(N + 1, 256, device="cuda")
+    ref_sqp = torch.zeros(ctas, device="cuda")
+    native.call("tcar_score_bwd_i_acc", native.ptr(Eb), native.ptr(Qs), native.ptr(ref), native.ptr(ref_sqp), B, N,
+                n_pad, 1)
+    torch.cuda.synchronize()
+    assert torch.equal(gi[1: N + 1], ref[1:])
+    assert torch.equal(sqp, ref_sqp)
+    assert (gi[0] == 7.0).all() and (gi[N + 1:] == 7.0).all()
 
 
 # ------------------------------------------------------------------------------------------- session groups (catalog-sharded step)
 @pytest.mark.parametrize("counts,N", [([512, 512], 5000), ([300, 0, 512, 77], 2333), ([512] * 8, 3000), ([1, 5], 300)])
-def test_score_groups_match_single_group_calls(native, counts, N, monkeypatch):
+def test_score_groups_match_single_group_calls(native, counts, N):
     """tcar_score_fwd_groups / _bwd_q_groups (one launch over all groups, tcar_score_bwd_q_multi) / _bwd_i_groups
     against the per-group entry points and a torch matmul over the same bf16 operands."""
-    import os
     R = len(counts)
     g = torch.Generator(device="cuda").manual_seed(N + R)
     n_pad = (N + 255) // 256 * 256
@@ -192,32 +192,31 @@ def test_score_groups_match_single_group_calls(native, counts, N, monkeypatch):
         native.call("tcar_score_fwd", p(Q[r]), p(I), p(c[r]), p(E1), p(p1), None, None, b, N, n_pad, 0, -2)
         torch.cuda.synchronize()
         assert torch.equal(E1.view(-1), E[r]) and torch.equal(p1.view(-1)[: tiles * QROWS], part[r])
-    # ---- dQ: single launch over all groups vs per-group launches vs fp64 matmul
+    # ---- dQ: tcar_score_bwd_q_groups (one launch over all groups when several are present) vs per-group
+    # tcar_score_bwd_q + tcar_rowsum_finish calls vs fp64 matmul
     qelems = max(int(lib.tcar_score_bwd_q_multi_part_elems(R)),
                  max(lib.tcar_score_bwd_q_splits(b, n_pad) for b in (1, 129, 257, 385)) * QROWS * KEXT)
     qpart = torch.zeros(qelems, device="cuda")
-    dq = {}
-    for mode in ("1", "0"):
-        monkeypatch.setenv("TCAR_BWDQ_LOOP", mode)
-        out = torch.zeros(R, QROWS, KEXT, device="cuda")
-        native.call("tcar_score_bwd_q_groups", p(E), QROWS * n_pad, p(I), p(qpart), p(out), QROWS * KEXT, p(part),
-                    tiles * QROWS, tiles, cnt, R, n_pad)
-        torch.cuda.synchronize()
-        dq[mode] = out
-    monkeypatch.delenv("TCAR_BWDQ_LOOP")
+    dq = torch.zeros(R, QROWS, KEXT, device="cuda")
+    native.call("tcar_score_bwd_q_groups", p(E), QROWS * n_pad, p(I), p(qpart), p(dq), QROWS * KEXT, p(part),
+                tiles * QROWS, tiles, cnt, R, n_pad)
+    torch.cuda.synchronize()
     for r, b in enumerate(counts):
         if b == 0:
             continue
+        dq1 = torch.zeros(QROWS, KEXT, device="cuda")
+        native.call("tcar_score_bwd_q", p(E[r]), p(I), p(qpart), p(dq1), b, n_pad)
+        native.call("tcar_rowsum_finish", p(part[r]), p(dq1[:, KEXT - 1:]), KEXT, tiles, b)
+        torch.cuda.synchronize()
         El = e_from_blocked(E[r], n_pad)[:b].double()
         ref = (El @ I.double()).float()
         ref[:, KEXT - 1] = El.float().sum(1)          # softmax partial sums ride in the pad column
         scale = ref[:, : KEXT - 1].abs().max().item()
-        for mode in ("1", "0"):
-            got = dq[mode][r, :b]
-            assert (got[:, : KEXT - 1] - ref[:, : KEXT - 1]).abs().max().item() / scale < 1e-4, (mode, r)
+        for name, got in (("groups", dq[r, :b]), ("single", dq1[:b])):
+            assert (got[:, : KEXT - 1] - ref[:, : KEXT - 1]).abs().max().item() / scale < 1e-4, (name, r)
             rs = got[:, KEXT - 1]
-            assert ((rs - ref[:, KEXT - 1]).abs() / ref[:, KEXT - 1]).max().item() < 2e-3, (mode, r)
-        assert torch.equal(dq["0"][r, :b, KEXT - 1], dq["1"][r, :b, KEXT - 1])
+            assert ((rs - ref[:, KEXT - 1]).abs() / ref[:, KEXT - 1]).max().item() < 2e-3, (name, r)
+        assert torch.equal(dq[r, :b, KEXT - 1], dq1[:b, KEXT - 1])
     # ---- dItems: first present group overwrites, later ones accumulate
     Qs = torch.zeros(R, QROWS, 256, device="cuda", dtype=torch.bfloat16)
     for r, b in enumerate(counts):
