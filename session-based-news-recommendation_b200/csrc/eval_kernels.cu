@@ -1206,6 +1206,161 @@ __device__ __forceinline__ void merge_topk(const unsigned long long* a, int K, c
 __host__ __device__ constexpr size_t rec_keys_offset(int B) {
     return ((size_t)(TCAR_QROWS + (1 + WSPLIT) * B) * 4 + 7) / 8 * 8;
 }
+// the threshold tau_b the select kernel left for query b
+__device__ __forceinline__ float rec_tau(const char* wspace, int b) {
+    return reinterpret_cast<const float*>(wspace)[TCAR_QROWS + b];
+}
+
+// Shared memory of both scan kernels, apart from their chunk queues.
+struct RecScanSmem {
+    unsigned long long top[2][RK];   // the running top-K, double-buffered (cur / cur ^ 1)
+    unsigned long long cand[NCAND];  // one batch of re-scored candidates; a partial list of another split at the end
+    int x[RX];                       // the exclusion list, sorted ascending
+    float aic[XW], tq[NB + 1];
+    int qn, cnt;                     // queued chunks, re-scored items
+};
+
+// Prologue of both scans for query blockIdx.x: the query row, an empty running list and the exclusion list (the CSR ids,
+// then the clicks - 1), padded with INT_MAX to a power of two and bitonic-sorted.  Returns its length nx, or -1 when the
+// list is malformed or longer than RX: block-uniform and the same for every split CTA, so the caller returns at once.
+// Ends with a barrier.
+__device__ __forceinline__ int rec_scan_prologue(RecScanSmem& s, const float* __restrict__ a_ic,
+                                                 const float* __restrict__ Tq, const int32_t* __restrict__ x_off,
+                                                 const int32_t* __restrict__ x_ids, const int32_t* __restrict__ clicks,
+                                                 int n_clicks) {
+    const int b = blockIdx.x, tid = threadIdx.x;
+    const int xo = x_off ? x_off[b] : 0;
+    const int nl = x_off ? x_off[b + 1] - xo : 0, nx = nl + n_clicks;
+    if (nl < 0 || nx > RX) return -1;
+    int P = 1;
+    while (P < nx) P <<= 1;
+    for (int i = tid; i < P; i += 256)
+        s.x[i] = i < nl ? x_ids[xo + i] : i < nx ? clicks[(size_t)b * n_clicks + (i - nl)] - 1 : 0x7fffffff;
+    for (int c = tid; c < XW; c += 256) s.aic[c] = a_ic[(size_t)b * XW + c];
+    for (int c = tid; c < NB; c += 256) s.tq[c] = Tq[(size_t)b * NB + c];
+    for (int i = tid; i < RK; i += 256) s.top[0][i] = KEY_NONE;
+    if (tid == 0) { s.qn = 0; s.cnt = 0; }
+    __syncthreads();
+    for (int k = 2; k <= P; k <<= 1) {
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int i = tid; i < P; i += 256) {
+                const int ixj = i ^ j;
+                if (ixj > i) {
+                    const int a = s.x[i], c = s.x[ixj];
+                    if (((i & k) == 0) ? a > c : a < c) { s.x[i] = c; s.x[ixj] = a; }
+                }
+            }
+            __syncthreads();
+        }
+    }
+    return nx;
+}
+
+// Re-scores the chunks a scan queued in s_q[0 .. s.qn) after the barrier this begins with, NCH chunks per batch:
+// item_at(p) is the item at catalog position p (chunk * CH + slot), or -1 to drop it; it and the excluded ids are
+// dropped before any row load.  Each batch is sorted and merged into s.top[cur] by merge(a, c, nc, out) (merge_topk or
+// merge_topk_capped with K bound), flipping cur; lane 0 of each warp counts its re-scored items in my_cnt.  Empties the
+// queue and ends with a barrier.
+template <class ItemAt, class Merge>
+__device__ __forceinline__ void rescore_queued(RecScanSmem& s, const int* s_q, int nx, ItemAt item_at, Merge merge,
+                                               const float* __restrict__ item, const float* __restrict__ content,
+                                               const int32_t* __restrict__ mwdhm, int& cur, int& my_cnt) {
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    auto excluded = [&](int n) {
+        int lo = 0, hi = nx;
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (s.x[mid] < n) lo = mid + 1; else hi = mid;
+        }
+        return lo < nx && s.x[lo] == n;
+    };
+    __syncthreads();
+    const int qn = s.qn;
+    for (int q0 = 0; q0 < qn; q0 += NCH) {
+        const int ncand = min(qn - q0, NCH) * CH;
+        int P2 = 32;                                                  // sort size: power of two >= ncand
+        while (P2 < ncand) P2 <<= 1;
+        if (tid < P2) s.cand[tid] = KEY_NONE;
+        __syncthreads();
+        for (int ci = w; ci < ncand; ci += 32) {
+            // four candidates per warp and iteration, branch-free, as in the widening pass; a dropped one reads row 0
+            int nn[4];
+            float sc[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const int cu = ci + 8 * u;
+                const int n = cu < ncand ? item_at(s_q[q0 + cu / CH] * CH + (cu % CH)) : -1;
+                nn[u] = n >= 0 && !excluded(n) ? n : -1;
+            }
+#pragma unroll
+            for (int u = 0; u < 4; ++u)
+                sc[u] = exact_score_e(s.aic, s.tq, item, content, mwdhm, nn[u] >= 0 ? nn[u] : 0, lane);
+            if (lane == 0) {
+#pragma unroll
+                for (int u = 0; u < 4; ++u)
+                    if (nn[u] >= 0) { s.cand[ci + 8 * u] = rerank_key(sc[u], nn[u]); ++my_cnt; }
+            }
+        }
+        for (int k = 2; k <= P2; k <<= 1) {
+            for (int j = k >> 1; j > 0; j >>= 1) {
+                __syncthreads();
+                const int ixj = tid ^ j;
+                if (tid < P2 && ixj > tid) {
+                    const unsigned long long a = s.cand[tid], c = s.cand[ixj];
+                    if (((tid & k) == 0) ? a > c : a < c) { s.cand[tid] = c; s.cand[ixj] = a; }
+                }
+            }
+        }
+        __syncthreads();
+        merge(s.top[cur], s.cand, P2, s.top[cur ^ 1]);
+        cur ^= 1;
+    }
+    if (tid == 0) s.qn = 0;
+    __syncthreads();
+}
+
+// The end of both scans: this split's partial list and count go to the workspace, then the ticket; the split CTA of the
+// query that finishes last merges the other lists (merge as in rescore_queued), writes ids / scores (-1 / -inf in empty
+// slots) and the total count, and resets the ticket to zero for the next call.
+template <class Merge>
+__device__ __forceinline__ void finish_splits(RecScanSmem& s, int cur, int my_cnt, Merge merge, int K, int B,
+                                              char* wspace, int32_t* __restrict__ out_ids,
+                                              float* __restrict__ out_scores, int32_t* __restrict__ rescored) {
+    const int b = blockIdx.x, split = blockIdx.y, tid = threadIdx.x, lane = tid & 31;
+    int32_t* ticket = reinterpret_cast<int32_t*>(wspace);
+    int32_t* part_cnt = reinterpret_cast<int32_t*>(wspace) + TCAR_QROWS + B;
+    unsigned long long* part = reinterpret_cast<unsigned long long*>(wspace + rec_keys_offset(B));
+    if (lane == 0 && my_cnt) atomicAdd(&s.cnt, my_cnt);
+    unsigned long long* mine = part + ((size_t)split * B + b) * RK;
+    for (int i = tid; i < K; i += 256) mine[i] = s.top[cur][i];
+    __syncthreads();
+    if (tid == 0) part_cnt[(size_t)split * B + b] = s.cnt;
+    __threadfence();
+    __syncthreads();
+    if (!__syncthreads_or(tid == 0 && atomicAdd(&ticket[b], 1) == WSPLIT - 1)) return;
+    __threadfence();
+    for (int sp = 0; sp < WSPLIT; ++sp) {
+        if (sp == split) continue;
+        const unsigned long long* other = part + ((size_t)sp * B + b) * RK;
+        for (int i = tid; i < K; i += 256) s.cand[i] = __ldcg(other + i);
+        __syncthreads();
+        merge(s.top[cur], s.cand, K, s.top[cur ^ 1]);
+        cur ^= 1;
+    }
+    for (int r = tid; r < K; r += 256) {
+        const unsigned long long key = s.top[cur][r];
+        out_ids[(size_t)b * K + r] = key == KEY_NONE ? -1 : (int)(uint32_t)key;
+        out_scores[(size_t)b * K + r] = key == KEY_NONE ? -INFINITY : key_value(~(uint32_t)(key >> 32));
+    }
+    if (tid == 0) {
+        if (rescored) {
+            int t = 0;
+            for (int sp = 0; sp < WSPLIT; ++sp) t += __ldcg(part_cnt + (size_t)sp * B + b);
+            rescored[b] = t;
+        }
+        ticket[b] = 0;
+    }
+}
 
 template <bool WINDOW>
 __global__ void __launch_bounds__(256, 2)
@@ -1217,57 +1372,30 @@ recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* 
                       int32_t* __restrict__ rescored, const int32_t* __restrict__ item_time,
                       const int32_t* __restrict__ win_lo, const int32_t* __restrict__ win_hi) {
     PDL_ENTER();
-    __shared__ float s_aic[XW], s_tq[NB + 1];
-    __shared__ int s_x[RX];
+    __shared__ RecScanSmem s;
     __shared__ int s_q[WQ_CAP];
-    __shared__ unsigned long long s_top[2][RK];
-    __shared__ unsigned long long s_new[NCAND];
-    __shared__ int s_qn, s_cnt, s_last;
-    const int b = blockIdx.x, split = blockIdx.y, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
-    int32_t* ticket = reinterpret_cast<int32_t*>(wspace);
-    const float* tau = reinterpret_cast<const float*>(wspace) + TCAR_QROWS;
-    int32_t* part_cnt = reinterpret_cast<int32_t*>(wspace) + TCAR_QROWS + B;
-    unsigned long long* part = reinterpret_cast<unsigned long long*>(wspace + rec_keys_offset(B));
-    const int xo = x_off ? x_off[b] : 0;
-    const int nl = x_off ? x_off[b + 1] - xo : 0, nx = nl + n_clicks;
-    if (nl < 0 || nx > RX) return;                                   // block-uniform, and the same for every split
-    // the exclusion list, sorted ascending (padded with INT_MAX to a power of two)
-    int P = 1;
-    while (P < nx) P <<= 1;
-    for (int i = tid; i < P; i += 256)
-        s_x[i] = i < nl ? x_ids[xo + i] : i < nx ? clicks[(size_t)b * n_clicks + (i - nl)] - 1 : 0x7fffffff;
-    for (int c = tid; c < XW; c += 256) s_aic[c] = a_ic[(size_t)b * XW + c];
-    for (int c = tid; c < NB; c += 256) s_tq[c] = Tq[(size_t)b * NB + c];
-    for (int i = tid; i < RK; i += 256) s_top[0][i] = KEY_NONE;
-    if (tid == 0) { s_qn = 0; s_cnt = 0; }
-    __syncthreads();
-    for (int k = 2; k <= P; k <<= 1) {
-        for (int j = k >> 1; j > 0; j >>= 1) {
-            for (int i = tid; i < P; i += 256) {
-                const int ixj = i ^ j;
-                if (ixj > i) {
-                    const int a = s_x[i], c = s_x[ixj];
-                    if (((i & k) == 0) ? a > c : a < c) { s_x[i] = c; s_x[ixj] = a; }
-                }
-            }
-            __syncthreads();
-        }
-    }
-    auto excluded = [&](int n) {
-        int lo = 0, hi = nx;
-        while (lo < hi) {
-            const int mid = (lo + hi) >> 1;
-            if (s_x[mid] < n) lo = mid + 1; else hi = mid;
-        }
-        return lo < nx && s_x[lo] == n;
-    };
+    const int b = blockIdx.x, split = blockIdx.y, tid = threadIdx.x;
+    const int nx = rec_scan_prologue(s, a_ic, Tq, x_off, x_ids, clicks, n_clicks);
+    if (nx < 0) return;
     const int32_t w_lo = WINDOW ? win_lo[b] : 0, w_hi = WINDOW ? win_hi[b] : 0;
     const int nchunks = (N + CH - 1) / CH, ntiles = (N + 127) / 128;
     const float* cm = chunkmax + (size_t)b * (n_pad / CH);
     const float* tm = tilemax + (size_t)b * (n_pad / 128);
-    const float bound = tau[b];
+    const float bound = rec_tau(wspace, b);
     const int per = (ntiles + WSPLIT - 1) / WSPLIT;
     const int t_lo = split * per, t_hi = min(t_lo + per, ntiles);
+    // ids >= N and (WINDOW) ids outside the session's window are dropped
+    auto item_at = [&](int n) {
+        if (n >= N) return -1;
+        if (WINDOW) {
+            const int32_t t = item_time[n];
+            if (t < w_lo || t > w_hi) return -1;
+        }
+        return n;
+    };
+    auto merge = [&](const unsigned long long* a, const unsigned long long* c, int nc, unsigned long long* out) {
+        merge_topk(a, K, c, nc, out);
+    };
     int cur = 0, my_cnt = 0;
     for (int t0 = t_lo; t0 < t_hi; t0 += 256) {
         const int tile = t0 + tid;
@@ -1280,92 +1408,12 @@ recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* 
             for (int c = 0; c < TILE_CH; ++c) {
                 const int chunk = tile * TILE_CH + c;
                 const float cv = c % 4 == 0 ? v[c / 4].x : c % 4 == 1 ? v[c / 4].y : c % 4 == 2 ? v[c / 4].z : v[c / 4].w;
-                if (chunk < nchunks && cv >= bound && (!WINDOW || cv > -INFINITY)) s_q[atomicAdd(&s_qn, 1)] = chunk;
+                if (chunk < nchunks && cv >= bound && (!WINDOW || cv > -INFINITY)) s_q[atomicAdd(&s.qn, 1)] = chunk;
             }
         }
-        __syncthreads();
-        const int qn = s_qn;
-        for (int q0 = 0; q0 < qn; q0 += NCH) {
-            const int ncand = min(qn - q0, NCH) * CH;
-            int P2 = 32;                                              // sort size: power of two >= ncand
-            while (P2 < ncand) P2 <<= 1;
-            if (tid < P2) s_new[tid] = KEY_NONE;
-            __syncthreads();
-            for (int ci = w; ci < ncand; ci += 32) {
-                // four candidates per warp and iteration, branch-free, as in the widening pass; an excluded id, one
-                // >= N or (WINDOW) one outside the session's window reads row 0 instead of its own
-                int nn[4];
-                float sc[4];
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    const int cu = ci + 8 * u;
-                    const int n = cu < ncand ? s_q[q0 + cu / CH] * CH + (cu % CH) : N;
-                    bool ok = n < N;
-                    if (WINDOW && ok) {
-                        const int32_t t = item_time[n];
-                        ok = w_lo <= t && t <= w_hi;
-                    }
-                    nn[u] = ok && !excluded(n) ? n : -1;
-                }
-#pragma unroll
-                for (int u = 0; u < 4; ++u)
-                    sc[u] = exact_score_e(s_aic, s_tq, item, content, mwdhm, nn[u] >= 0 ? nn[u] : 0, lane);
-                if (lane == 0) {
-#pragma unroll
-                    for (int u = 0; u < 4; ++u)
-                        if (nn[u] >= 0) { s_new[ci + 8 * u] = rerank_key(sc[u], nn[u]); ++my_cnt; }
-                }
-            }
-            for (int k = 2; k <= P2; k <<= 1) {
-                for (int j = k >> 1; j > 0; j >>= 1) {
-                    __syncthreads();
-                    const int ixj = tid ^ j;
-                    if (tid < P2 && ixj > tid) {
-                        const unsigned long long a = s_new[tid], c = s_new[ixj];
-                        if (((tid & k) == 0) ? a > c : a < c) { s_new[tid] = c; s_new[ixj] = a; }
-                    }
-                }
-            }
-            __syncthreads();
-            merge_topk(s_top[cur], K, s_new, P2, s_top[cur ^ 1]);
-            cur ^= 1;
-        }
-        if (tid == 0) s_qn = 0;
-        __syncthreads();
+        rescore_queued(s, s_q, nx, item_at, merge, item, content, mwdhm, cur, my_cnt);
     }
-    // partial list and count of this split, then the ticket: the last split CTA of the query merges all of them
-    if (lane == 0 && my_cnt) atomicAdd(&s_cnt, my_cnt);
-    unsigned long long* mine = part + ((size_t)split * B + b) * RK;
-    for (int i = tid; i < K; i += 256) mine[i] = s_top[cur][i];
-    __syncthreads();
-    if (tid == 0) part_cnt[(size_t)split * B + b] = s_cnt;
-    __threadfence();
-    __syncthreads();
-    if (tid == 0) s_last = atomicAdd(&ticket[b], 1) == WSPLIT - 1;
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    for (int s = 0; s < WSPLIT; ++s) {
-        if (s == split) continue;
-        const unsigned long long* other = part + ((size_t)s * B + b) * RK;
-        for (int i = tid; i < K; i += 256) s_new[i] = __ldcg(other + i);
-        __syncthreads();
-        merge_topk(s_top[cur], K, s_new, K, s_top[cur ^ 1]);
-        cur ^= 1;
-    }
-    for (int r = tid; r < K; r += 256) {
-        const unsigned long long key = s_top[cur][r];
-        out_ids[(size_t)b * K + r] = key == KEY_NONE ? -1 : (int)(uint32_t)key;
-        out_scores[(size_t)b * K + r] = key == KEY_NONE ? -INFINITY : key_value(~(uint32_t)(key >> 32));
-    }
-    if (tid == 0) {
-        if (rescored) {
-            int t = 0;
-            for (int s = 0; s < WSPLIT; ++s) t += __ldcg(part_cnt + (size_t)s * B + b);
-            rescored[b] = t;
-        }
-        ticket[b] = 0;
-    }
+    finish_splits(s, cur, my_cnt, merge, K, B, wspace, out_ids, out_scores, rescored);
 }
 
 // ------------------------------------------------------------------------- top-K recommendation by category (§4.9)
@@ -1642,153 +1690,43 @@ recommend_category_scan_kernel(const float* chunkmax, const float* __restrict__ 
                                int32_t* __restrict__ out_ids, float* __restrict__ out_scores,
                                int32_t* __restrict__ rescored, const float* __restrict__ cat_tau) {
     PDL_ENTER();
-    __shared__ float s_aic[XW], s_tq[NB + 1];
-    __shared__ int s_x[RX];
+    __shared__ RecScanSmem s;
     __shared__ int s_q[256];
-    __shared__ unsigned long long s_top[2][RK];
-    __shared__ unsigned long long s_new[NCAND];
     __shared__ unsigned long long s_u[RK + NCAND];
     __shared__ int s_uc[RK + NCAND];
     __shared__ uint32_t s_bits[RG / 32];
     __shared__ int s_cst[RG], s_pre[RG + 1], s_ccnt[RG], s_w[3][8];
     __shared__ float s_ctau[RG];
-    __shared__ int s_qn, s_cnt, s_last;
-    const int b = blockIdx.x, split = blockIdx.y, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
-    int32_t* ticket = reinterpret_cast<int32_t*>(wspace);
-    const float* tau = reinterpret_cast<const float*>(wspace) + TCAR_QROWS;
-    int32_t* part_cnt = reinterpret_cast<int32_t*>(wspace) + TCAR_QROWS + B;
-    unsigned long long* part = reinterpret_cast<unsigned long long*>(wspace + rec_keys_offset(B));
-    const int xo = x_off ? x_off[b] : 0;
-    const int nl = x_off ? x_off[b + 1] - xo : 0, nx = nl + n_clicks;
-    if (nl < 0 || nx > RX) return;                                   // block-uniform, and the same for every split
-    const bool capped = C < K;
-    int P = 1;
-    while (P < nx) P <<= 1;
-    for (int i = tid; i < P; i += 256)
-        s_x[i] = i < nl ? x_ids[xo + i] : i < nx ? clicks[(size_t)b * n_clicks + (i - nl)] - 1 : 0x7fffffff;
-    for (int c = tid; c < XW; c += 256) s_aic[c] = a_ic[(size_t)b * XW + c];
-    for (int c = tid; c < NB; c += 256) s_tq[c] = Tq[(size_t)b * NB + c];
-    for (int i = tid; i < RK; i += 256) s_top[0][i] = KEY_NONE;
+    const int b = blockIdx.x, split = blockIdx.y, tid = threadIdx.x;
+    const int nx = rec_scan_prologue(s, a_ic, Tq, x_off, x_ids, clicks, n_clicks);
+    if (nx < 0) return;
     for (int g = tid; g < G; g += 256) s_ccnt[g] = 0;
-    if (tid == 0) { s_qn = 0; s_cnt = 0; }
-    __syncthreads();
-    for (int k = 2; k <= P; k <<= 1) {
-        for (int j = k >> 1; j > 0; j >>= 1) {
-            for (int i = tid; i < P; i += 256) {
-                const int ixj = i ^ j;
-                if (ixj > i) {
-                    const int a = s_x[i], c = s_x[ixj];
-                    if (((i & k) == 0) ? a > c : a < c) { s_x[i] = c; s_x[ixj] = a; }
-                }
-            }
-            __syncthreads();
-        }
-    }
-    auto excluded = [&](int n) {
-        int lo = 0, hi = nx;
-        while (lo < hi) {
-            const int mid = (lo + hi) >> 1;
-            if (s_x[mid] < n) lo = mid + 1; else hi = mid;
-        }
-        return lo < nx && s_x[lo] == n;
-    };
     const CatRanges r = category_ranges(cat_chunk_off, G, a_off, a_codes, b, 1, s_bits, s_cst, s_pre, s_w);
     for (int a = tid; a < r.A; a += 256) s_ctau[a] = cat_tau[(size_t)b * RG + a];
-    __syncthreads();
     const float* cm = chunkmax + (size_t)b * (n_pad / CH);
-    const float bound = tau[b];
+    const float bound = rec_tau(wspace, b);
     const int per = (r.total + WSPLIT - 1) / WSPLIT;
     const int i_lo = split * per, i_hi = min(i_lo + per, r.total);
+    auto item_at = [&](int p) { return perm[p]; };                   // -1 on a pad
+    const bool capped = C < K;
+    auto merge = [&](const unsigned long long* a, const unsigned long long* c, int nc, unsigned long long* out) {
+        if (capped)
+            merge_topk_capped(a, K, c, nc, out, s_u, s_uc, item_cat, C, s_ccnt);
+        else
+            merge_topk(a, K, c, nc, out);
+    };
     int cur = 0, my_cnt = 0;
+    __syncthreads();
     for (int i0 = i_lo; i0 < i_hi; i0 += 256) {
         const int i = i0 + tid;
         if (i < i_hi) {
             const int a = allowed_index(s_pre, r.A, i);
             const int chunk = s_cst[a] + i - s_pre[a];
-            if (cm[chunk] >= fmaxf(bound, s_ctau[a])) s_q[atomicAdd(&s_qn, 1)] = chunk;
+            if (cm[chunk] >= fmaxf(bound, s_ctau[a])) s_q[atomicAdd(&s.qn, 1)] = chunk;
         }
-        __syncthreads();
-        const int qn = s_qn;
-        for (int q0 = 0; q0 < qn; q0 += NCH) {
-            const int ncand = min(qn - q0, NCH) * CH;
-            int P2 = 32;                                              // sort size: power of two >= ncand
-            while (P2 < ncand) P2 <<= 1;
-            if (tid < P2) s_new[tid] = KEY_NONE;
-            __syncthreads();
-            for (int ci = w; ci < ncand; ci += 32) {
-                // four candidates per warp and iteration, branch-free; a pad or an excluded id reads row 0 instead
-                int nn[4];
-                float sc[4];
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    const int cu = ci + 8 * u;
-                    const int n = cu < ncand ? perm[s_q[q0 + cu / CH] * CH + (cu % CH)] : -1;
-                    nn[u] = n >= 0 && !excluded(n) ? n : -1;
-                }
-#pragma unroll
-                for (int u = 0; u < 4; ++u)
-                    sc[u] = exact_score_e(s_aic, s_tq, item, content, mwdhm, nn[u] >= 0 ? nn[u] : 0, lane);
-                if (lane == 0) {
-#pragma unroll
-                    for (int u = 0; u < 4; ++u)
-                        if (nn[u] >= 0) { s_new[ci + 8 * u] = rerank_key(sc[u], nn[u]); ++my_cnt; }
-                }
-            }
-            for (int k = 2; k <= P2; k <<= 1) {
-                for (int j = k >> 1; j > 0; j >>= 1) {
-                    __syncthreads();
-                    const int ixj = tid ^ j;
-                    if (tid < P2 && ixj > tid) {
-                        const unsigned long long a = s_new[tid], c = s_new[ixj];
-                        if (((tid & k) == 0) ? a > c : a < c) { s_new[tid] = c; s_new[ixj] = a; }
-                    }
-                }
-            }
-            __syncthreads();
-            if (capped)
-                merge_topk_capped(s_top[cur], K, s_new, P2, s_top[cur ^ 1], s_u, s_uc, item_cat, C, s_ccnt);
-            else
-                merge_topk(s_top[cur], K, s_new, P2, s_top[cur ^ 1]);
-            cur ^= 1;
-        }
-        if (tid == 0) s_qn = 0;
-        __syncthreads();
+        rescore_queued(s, s_q, nx, item_at, merge, item, content, mwdhm, cur, my_cnt);
     }
-    if (lane == 0 && my_cnt) atomicAdd(&s_cnt, my_cnt);
-    unsigned long long* mine = part + ((size_t)split * B + b) * RK;
-    for (int i = tid; i < K; i += 256) mine[i] = s_top[cur][i];
-    __syncthreads();
-    if (tid == 0) part_cnt[(size_t)split * B + b] = s_cnt;
-    __threadfence();
-    __syncthreads();
-    if (tid == 0) s_last = atomicAdd(&ticket[b], 1) == WSPLIT - 1;
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    for (int s = 0; s < WSPLIT; ++s) {
-        if (s == split) continue;
-        const unsigned long long* other = part + ((size_t)s * B + b) * RK;
-        for (int i = tid; i < K; i += 256) s_new[i] = __ldcg(other + i);
-        __syncthreads();
-        if (capped)
-            merge_topk_capped(s_top[cur], K, s_new, K, s_top[cur ^ 1], s_u, s_uc, item_cat, C, s_ccnt);
-        else
-            merge_topk(s_top[cur], K, s_new, K, s_top[cur ^ 1]);
-        cur ^= 1;
-    }
-    for (int i = tid; i < K; i += 256) {
-        const unsigned long long key = s_top[cur][i];
-        out_ids[(size_t)b * K + i] = key == KEY_NONE ? -1 : (int)(uint32_t)key;
-        out_scores[(size_t)b * K + i] = key == KEY_NONE ? -INFINITY : key_value(~(uint32_t)(key >> 32));
-    }
-    if (tid == 0) {
-        if (rescored) {
-            int t = 0;
-            for (int s = 0; s < WSPLIT; ++s) t += __ldcg(part_cnt + (size_t)s * B + b);
-            rescored[b] = t;
-        }
-        ticket[b] = 0;
-    }
+    finish_splits(s, cur, my_cnt, merge, K, B, wspace, out_ids, out_scores, rescored);
 }
 
 }  // namespace tcar
@@ -2001,14 +1939,26 @@ extern "C" long long tcar_recommend_ws_bytes(int B) {
     return (long long)(rec_keys_offset(B) + (size_t)WSPLIT * B * RK * 8);
 }
 
-extern "C" int tcar_recommend(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
-                              const float* item, const float* content, const int32_t* mwdhm, const float* cat_stats,
-                              const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B, int N,
-                              int n_pad, int K, void* workspace, int32_t* ids, float* scores, int32_t* rescored,
-                              void* stream) {
-    if (B < 0 || B > TCAR_QROWS || N < 1 || n_pad < N || n_pad % 128 || K < 1 || K > RK ||
-        (clicks && (T < 1 || T > RX)) || !chunkmax || !tilemax || !a_ic || !Tq || !item || !content || !mwdhm ||
-        !cat_stats || (x_off && !x_ids) || !workspace || !ids || !scores)
+// the argument checks the three recommend entry points share
+static bool rec_args_ok(const float* chunkmax, const float* a_ic, const float* Tq, const float* item,
+                        const float* content, const int32_t* mwdhm, const float* cat_stats, const int32_t* x_off,
+                        const int32_t* x_ids, const int32_t* clicks, int T, int B, int n_pad, int K,
+                        const void* workspace, const int32_t* ids, const float* scores) {
+    return B >= 0 && B <= TCAR_QROWS && n_pad % 128 == 0 && K >= 1 && K <= RK && !(clicks && (T < 1 || T > RX)) &&
+           chunkmax && a_ic && Tq && item && content && mwdhm && cat_stats && !(x_off && !x_ids) && workspace && ids &&
+           scores;
+}
+
+// tcar_recommend and tcar_recommend_window: the selection, then the scan
+template <bool WINDOW>
+static int launch_recommend(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
+                            const float* item, const float* content, const int32_t* mwdhm, const float* cat_stats,
+                            const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B, int N,
+                            int n_pad, int K, void* workspace, int32_t* ids, float* scores, int32_t* rescored,
+                            const int32_t* item_time, const int32_t* win_lo, const int32_t* win_hi, void* stream) {
+    if (!rec_args_ok(chunkmax, a_ic, Tq, item, content, mwdhm, cat_stats, x_off, x_ids, clicks, T, B, n_pad, K,
+                     workspace, ids, scores) ||
+        N < 1 || n_pad < N || !tilemax)
         return TCAR_ERR_ARG;
     if (B == 0) return 0;
     const int n_clicks = clicks ? T : 0;
@@ -2016,11 +1966,20 @@ extern "C" int tcar_recommend(const float* chunkmax, const float* tilemax, const
     cudaError_t e = launch_pdl(recommend_select_kernel, dim3(B), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq,
                                cat_stats, x_off, n_clicks, K, N, n_pad, reinterpret_cast<float*>(ws) + TCAR_QROWS);
     if (e != cudaSuccess) return (int)e;
-    launch_pdl(recommend_scan_kernel<false>, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq, item,
-               content, mwdhm, x_off, x_ids, clicks, n_clicks, K, N, n_pad, B, ws, ids, scores, rescored,
-               static_cast<const int32_t*>(nullptr), static_cast<const int32_t*>(nullptr),
-               static_cast<const int32_t*>(nullptr));
+    launch_pdl(recommend_scan_kernel<WINDOW>, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq, item,
+               content, mwdhm, x_off, x_ids, clicks, n_clicks, K, N, n_pad, B, ws, ids, scores, rescored, item_time,
+               win_lo, win_hi);
     return (int)cudaGetLastError();
+}
+
+extern "C" int tcar_recommend(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
+                              const float* item, const float* content, const int32_t* mwdhm, const float* cat_stats,
+                              const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B, int N,
+                              int n_pad, int K, void* workspace, int32_t* ids, float* scores, int32_t* rescored,
+                              void* stream) {
+    return launch_recommend<false>(chunkmax, tilemax, a_ic, Tq, item, content, mwdhm, cat_stats, x_off, x_ids, clicks,
+                                   T, B, N, n_pad, K, workspace, ids, scores, rescored, nullptr, nullptr, nullptr,
+                                   stream);
 }
 
 extern "C" int tcar_recommend_window(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
@@ -2029,20 +1988,10 @@ extern "C" int tcar_recommend_window(const float* chunkmax, const float* tilemax
                                      const int32_t* clicks, int T, int B, int N, int n_pad, int K, void* workspace,
                                      int32_t* ids, float* scores, int32_t* rescored, const int32_t* item_time,
                                      const int32_t* win_lo, const int32_t* win_hi, void* stream) {
-    if (B < 0 || B > TCAR_QROWS || N < 1 || n_pad < N || n_pad % 128 || K < 1 || K > RK ||
-        (clicks && (T < 1 || T > RX)) || !chunkmax || !tilemax || !a_ic || !Tq || !item || !content || !mwdhm ||
-        !cat_stats || (x_off && !x_ids) || !workspace || !ids || !scores || !item_time || !win_lo || !win_hi)
-        return TCAR_ERR_ARG;
-    if (B == 0) return 0;
-    const int n_clicks = clicks ? T : 0;
-    char* ws = static_cast<char*>(workspace);
-    cudaError_t e = launch_pdl(recommend_select_kernel, dim3(B), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq,
-                               cat_stats, x_off, n_clicks, K, N, n_pad, reinterpret_cast<float*>(ws) + TCAR_QROWS);
-    if (e != cudaSuccess) return (int)e;
-    launch_pdl(recommend_scan_kernel<true>, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq, item,
-               content, mwdhm, x_off, x_ids, clicks, n_clicks, K, N, n_pad, B, ws, ids, scores, rescored, item_time,
-               win_lo, win_hi);
-    return (int)cudaGetLastError();
+    if (!item_time || !win_lo || !win_hi) return TCAR_ERR_ARG;
+    return launch_recommend<true>(chunkmax, tilemax, a_ic, Tq, item, content, mwdhm, cat_stats, x_off, x_ids, clicks,
+                                  T, B, N, n_pad, K, workspace, ids, scores, rescored, item_time, win_lo, win_hi,
+                                  stream);
 }
 
 // tcar_recommend's workspace, then the per-category thresholds [B][TCAR_RECOMMEND_MAXG]
@@ -2060,10 +2009,9 @@ extern "C" int tcar_recommend_category(const float* chunkmax, const float* a_ic,
                                        const int32_t* cat_chunk_off, int G, const int32_t* a_off,
                                        const int32_t* a_codes, int C, void* workspace, int32_t* ids, float* scores,
                                        int32_t* rescored, void* stream) {
-    if (B < 0 || B > TCAR_QROWS || n_pad < CH || n_pad % 128 || K < 1 || K > RK || G < 1 || G > RG || C < 1 ||
-        (clicks && (T < 1 || T > RX)) || !chunkmax || !a_ic || !Tq || !item || !content || !mwdhm || !cat_stats ||
-        (x_off && !x_ids) || (a_off && !a_codes) || !perm || !item_cat || !cat_chunk_off || !workspace || !ids ||
-        !scores)
+    if (!rec_args_ok(chunkmax, a_ic, Tq, item, content, mwdhm, cat_stats, x_off, x_ids, clicks, T, B, n_pad, K,
+                     workspace, ids, scores) ||
+        n_pad < CH || G < 1 || G > RG || C < 1 || (a_off && !a_codes) || !perm || !item_cat || !cat_chunk_off)
         return TCAR_ERR_ARG;
     if (B == 0) return 0;
     const int n_clicks = clicks ? T : 0;

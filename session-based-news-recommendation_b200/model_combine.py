@@ -1468,66 +1468,45 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         if B == 0:
             return out_ids, out_sc
         if getattr(self, "_rec_ws", None) is None:
-            # ticket counters first: zero once, every call leaves them at zero
-            self._rec_ws = torch.zeros(int(nv.lib().tcar_recommend_ws_bytes(QROWS)), device=dev, dtype=torch.uint8)
+            # one workspace for the three selections, sized for the category one (tcar_recommend's layout plus the
+            # per-category thresholds: QROWS x TCAR_RECOMMEND_MAXG x 4 B = 2 MiB more); its ticket counters come first:
+            # zero once, every call leaves them at zero
+            self._rec_ws = torch.zeros(int(nv.lib().tcar_recommend_category_ws_bytes(QROWS)), device=dev,
+                                       dtype=torch.uint8)
             self.rec_rescored = torch.zeros(QROWS, device=dev, dtype=torch.int32)
         if not self._item_table_synced:
             self.sync_item_table()         # after catalog-sharded training every rank holds only its own rows
         self._session_forward(bt)
         self._ensure_cat_stats()
-        ws = self._score_buffers(ps.n_pad, False)
+        # the chunk / tile maxima of one unguarded eval-mode GEMM (its softmax partial sums, which may overflow without
+        # the guard, are not read): over ps.iext, with the windows applied in the epilogue, or over iext_cat (N' items
+        # in category order); the windows go up through the pinned ring like the exclusion lists
         if win is not None:
-            return self._recommend_window(bt, k, host, exclude_clicked, win, out_ids, out_sc)
+            ws = self._score_buffers(ps.n_pad, False)
+            wv = self._stage_ints(win)
+            nv.counted_call("tcar_score_fwd_window", 1, p(self.Q), p(ps.iext), p(self.c_ref), p(ws["part"]),
+                            p(ws["cmax"]), p(ws["tmax"]), p(self._item_time), p(wv), p(wv[B:]), B, N, ps.n_pad)
+        else:
+            if by_cat:
+                self._ensure_iext_cat()
+            iext, n, n_pad = (self._iext_cat, self._cat_n, self._cat_n_pad) if by_cat else (ps.iext, N, ps.n_pad)
+            ws = self._score_buffers(n_pad, False)
+            nv.counted_call("tcar_score_fwd", 1, p(self.Q), p(iext), p(self.c_ref), None, p(ws["part"]), p(ws["cmax"]),
+                            p(ws["tmax"]), B, n, n_pad, 1, self._cluster_for(B))
+        csr = self._stage_ints(host) if host is not None else None
+        query = (p(self.a_ic), p(self.Tq), p(ps.item), p(ps.content), p(ps.mwdhm), p(self.cat_stats), p(csr),
+                 p(csr[B + 1:]) if csr is not None else None, p(bt.seq) if exclude_clicked else None, bt.T, B)
+        out = (p(self._rec_ws), p(out_ids), p(out_sc), p(self.rec_rescored))
         if by_cat:
-            return self._recommend_category(bt, k, host, exclude_clicked, C, allowed, out_ids, out_sc)
-        # one unguarded eval-mode GEMM for the chunk / tile maxima; its softmax partial sums (which may overflow without
-        # the guard) are not read
-        nv.counted_call("tcar_score_fwd", 1, p(self.Q), p(ps.iext), p(self.c_ref), None, p(ws["part"]), p(ws["cmax"]),
-                        p(ws["tmax"]), B, N, ps.n_pad, 1, self._cluster_for(B))
-        csr = self._stage_ints(host) if host is not None else None
-        nv.counted_call("tcar_recommend", 2, p(ws["cmax"]), p(ws["tmax"]), p(self.a_ic), p(self.Tq), p(ps.item),
-                        p(ps.content), p(ps.mwdhm), p(self.cat_stats), p(csr),
-                        p(csr[B + 1:]) if csr is not None else None, p(bt.seq) if exclude_clicked else None, bt.T, B,
-                        N, ps.n_pad, k, p(self._rec_ws), p(out_ids), p(out_sc), p(self.rec_rescored))
-        return out_ids, out_sc
-
-    def _recommend_window(self, bt, k, host, exclude_clicked, win, out_ids, out_sc):
-        """recommend() with checked windows win = int32 [lo | hi]: the windowed GEMM (masked chunk / tile maxima), then
-        the windowed selection and scan.  The windows go up through the pinned ring like the exclusion lists."""
-        B, N, p, ps = bt.B, self.N, nv.ptr, self.ps
-        ws = self._score_buffers(ps.n_pad, False)
-        wv = self._stage_ints(win)
-        nv.counted_call("tcar_score_fwd_window", 1, p(self.Q), p(ps.iext), p(self.c_ref), p(ws["part"]), p(ws["cmax"]),
-                        p(ws["tmax"]), p(self._item_time), p(wv), p(wv[B:]), B, N, ps.n_pad)
-        csr = self._stage_ints(host) if host is not None else None
-        nv.counted_call("tcar_recommend_window", 2, p(ws["cmax"]), p(ws["tmax"]), p(self.a_ic), p(self.Tq),
-                        p(ps.item), p(ps.content), p(ps.mwdhm), p(self.cat_stats), p(csr),
-                        p(csr[B + 1:]) if csr is not None else None, p(bt.seq) if exclude_clicked else None, bt.T, B,
-                        N, ps.n_pad, k, p(self._rec_ws), p(out_ids), p(out_sc), p(self.rec_rescored),
-                        p(self._item_time), p(wv), p(wv[B:]))
-        return out_ids, out_sc
-
-    def _recommend_category(self, bt, k, host, exclude_clicked, C, allowed, out_ids, out_sc):
-        """recommend() with item categories: the unchanged eval-mode GEMM over iext_cat (N' items in category order),
-        then tcar_recommend_category with the cap C (C = k: none) and the checked CSR allowed-code lists (None: all)."""
-        B, p, ps = bt.B, nv.ptr, self.ps
-        if getattr(self, "_rec_cat_ws", None) is None:
-            # tcar_recommend's layout (ticket counters first: zero once, every call leaves them at zero), then the
-            # per-category thresholds
-            self._rec_cat_ws = torch.zeros(int(nv.lib().tcar_recommend_category_ws_bytes(QROWS)), device=self.dev,
-                                           dtype=torch.uint8)
-        self._ensure_iext_cat()
-        ws = self._score_buffers(self._cat_n_pad, False)
-        nv.counted_call("tcar_score_fwd", 1, p(self.Q), p(self._iext_cat), p(self.c_ref), None, p(ws["part"]),
-                        p(ws["cmax"]), p(ws["tmax"]), B, self._cat_n, self._cat_n_pad, 1, self._cluster_for(B))
-        csr = self._stage_ints(host) if host is not None else None
-        acsr = self._stage_ints(allowed) if allowed is not None else None
-        nv.counted_call("tcar_recommend_category", 2, p(ws["cmax"]), p(self.a_ic), p(self.Tq), p(ps.item),
-                        p(ps.content), p(ps.mwdhm), p(self.cat_stats), p(csr),
-                        p(csr[B + 1:]) if csr is not None else None, p(bt.seq) if exclude_clicked else None, bt.T, B,
-                        self._cat_n_pad, k, p(self._cat_perm), p(self._item_cat), p(self._cat_off), self._cat_G,
-                        p(acsr), p(acsr[B + 1:]) if acsr is not None else None, C, p(self._rec_cat_ws), p(out_ids),
-                        p(out_sc), p(self.rec_rescored))
+            acsr = self._stage_ints(allowed) if allowed is not None else None
+            nv.counted_call("tcar_recommend_category", 2, p(ws["cmax"]), *query, self._cat_n_pad, k,
+                            p(self._cat_perm), p(self._item_cat), p(self._cat_off), self._cat_G, p(acsr),
+                            p(acsr[B + 1:]) if acsr is not None else None, C, *out)
+        elif win is not None:
+            nv.counted_call("tcar_recommend_window", 2, p(ws["cmax"]), p(ws["tmax"]), *query, N, ps.n_pad, k, *out,
+                            p(self._item_time), p(wv), p(wv[B:]))
+        else:
+            nv.counted_call("tcar_recommend", 2, p(ws["cmax"]), p(ws["tmax"]), *query, N, ps.n_pad, k, *out)
         return out_ids, out_sc
 
     def recommend_split(self, sess, test_data, item_dict, args):

@@ -3,7 +3,7 @@ the oracle's forward(), against the full-catalog evaluation it must agree with b
 without exclusions.
 
 Reference: the oracle's softmax_input (model_combine.py:138) with the excluded ids set to -inf, ordered by (score desc,
-id asc) and cut to K."""
+id asc) and cut to K (recommend_ref.topk_ref)."""
 import pickle
 
 import numpy as np
@@ -12,84 +12,8 @@ import torch
 
 pytestmark = pytest.mark.gpu
 
-from oracle import tcar_oracle as O  # noqa: E402
-from test_gpu_parity import batch_for, build, oracle_inputs  # noqa: E402
-
-GLOBO_N = 364047
-
-
-def oracle_scores(model, content, mwdhm, batch):
-    params, c64, m64 = oracle_inputs(model, content, mwdhm)
-    with torch.no_grad():
-        return O.forward(params, c64, m64, batch)["softmax_input"].numpy()
-
-
-def recommend_ref(S, K, excluded):
-    """fp64 reference: per row the K best eligible items by (score desc, id asc), padded with -1 / -inf, and whether
-    the first K + 1 eligible scores are separated by more than 2e-5 |score| (the margin_ok rule)."""
-    B, N = S.shape
-    ids = np.full((B, K), -1, np.int64)
-    sc = np.full((B, K), -np.inf)
-    margin = np.zeros(B, bool)
-    for b in range(B):
-        s = S[b].copy()
-        ex = np.array(sorted(excluded[b]), np.int64)
-        s[ex] = -np.inf
-        order = np.lexsort((np.arange(N), -s))
-        order = order[np.isfinite(s[order])]
-        n = min(K, len(order))
-        ids[b, :n], sc[b, :n] = order[:n], s[order[:n]]
-        head = s[order[:K + 1]]
-        margin[b] = len(head) < 2 or bool((np.abs(np.diff(head)) > 2e-5 * np.abs(head).max()).all())
-    return ids, sc, margin
-
-
-def own_order_ok(ids, sc):
-    """Every row is ordered exactly by (score desc, id asc) of its own fp32 scores, padding last."""
-    for i_row, s_row in zip(ids, sc):
-        n = int((i_row >= 0).sum())
-        assert (i_row[n:] == -1).all() and np.isneginf(s_row[n:]).all()
-        i, s = i_row[:n].astype(np.int64), s_row[:n].astype(np.float64)
-        assert (np.lexsort((i, -s)) == np.arange(n)).all()
-        assert len(set(i.tolist())) == n
-
-
-def make_lists(rs, N, lens, dup=False):
-    off = np.zeros(len(lens) + 1, dtype=np.int32)
-    off[1:] = np.cumsum(lens)
-    ids = rs.randint(0, N, int(off[-1])).astype(np.int32)
-    if dup:
-        for b, L in enumerate(lens):
-            if L > 2:
-                ids[off[b] + L - 1] = ids[off[b]]
-                ids[off[b] + 1] = ids[off[b]]
-    return off, ids
-
-
-def excluded_sets(B, off, ids, seq=None):
-    ex = [set() for _ in range(B)]
-    if off is not None:
-        for b in range(B):
-            ex[b].update(ids[off[b]:off[b + 1]].tolist())
-    if seq is not None:
-        for b in range(B):
-            ex[b].update((seq[b] - 1).tolist())
-    return ex
-
-
-def check_against_reference(ids, sc, S, K, excluded):
-    r_ids, r_sc, margin = recommend_ref(S, K, excluded)
-    own_order_ok(ids, sc)
-    valid = r_ids >= 0
-    assert ((ids >= 0) == valid).all(), "padding where the reference has no eligible item"
-    np.testing.assert_allclose(sc[valid], r_sc[valid], rtol=1e-4, atol=1e-5)
-    assert (ids[margin] == r_ids[margin]).all(), "ids exact on margin-checked rows"
-    # every row: the returned items are eligible and are as good as the reference's, position by position
-    for b in range(len(ids)):
-        got = ids[b][ids[b] >= 0]
-        assert not (set(got.tolist()) & excluded[b])
-        np.testing.assert_allclose(S[b, got], r_sc[b, :len(got)], rtol=1e-4, atol=1e-5)
-    return margin
+from recommend_ref import GLOBO_N, check_topk, excluded_sets, make_lists, oracle_scores  # noqa: E402
+from test_gpu_parity import batch_for, build  # noqa: E402
 
 
 @pytest.mark.parametrize("B,N,K,T,kind", [(1, 300, 1, 1, "plain"), (7, 2000, 100, 3, "dup"),
@@ -115,7 +39,7 @@ def test_recommend_matches_fp64_reference(B, N, K, T, kind):
     assert torch.equal(ids, ids2) and torch.equal(sc, sc2), "a second run must be bit-identical"
     S = oracle_scores(model, content, mwdhm, batch)
     ex = excluded_sets(B, off, lst, batch["seq"].numpy() if clicked else None)
-    margin = check_against_reference(ids.cpu().numpy(), sc.cpu().numpy(), S, K, ex)
+    margin = check_topk(ids.cpu().numpy(), sc.cpu().numpy(), S, K, ex)
     if K <= 100:
         assert margin.mean() > 0.5, "fixture must be mostly margin-checked"
     if kind == "small":
@@ -203,7 +127,7 @@ def test_wide_bands_near_tie_clusters():
     n_band = model.rec_rescored[:B].cpu().numpy()
     assert n_band.max() >= 1000, "fixture should open a band of hundreds of chunks"
     S = oracle_scores(model, cont, mw, batch)
-    check_against_reference(ids.cpu().numpy(), sc.cpu().numpy(), S, K,
+    check_topk(ids.cpu().numpy(), sc.cpu().numpy(), S, K,
                             excluded_sets(B, None, None, batch["seq"].numpy()))
     model.cat_stats.fill_(1e4)                  # eps_b ~ 1e4 ||q||: the band is the whole catalog
     ids2, sc2 = model.recommend(bt, K, exclude_clicked=True)

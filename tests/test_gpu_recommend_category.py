@@ -11,67 +11,8 @@ import torch
 
 pytestmark = pytest.mark.gpu
 
-from test_gpu_parity import batch_for, build, oracle_inputs  # noqa: E402
-from test_gpu_recommend import excluded_sets, make_lists, own_order_ok  # noqa: E402
-from oracle import tcar_oracle as O  # noqa: E402
-
-GLOBO_N = 364047
-
-
-def oracle_scores(model, content, mwdhm, batch):
-    params, c64, m64 = oracle_inputs(model, content, mwdhm)
-    with torch.no_grad():
-        return O.forward(params, c64, m64, batch)["softmax_input"].numpy()
-
-
-def capped_ref(S, K, C, cat, allowed, excluded):
-    """fp64 greedy reference: per row walk the eligible items (allowed category, not excluded) by (score desc, id asc),
-    drop an item that has C items of its category before it, stop at K kept.  Returns ids / scores padded with -1 / -inf
-    and whether the scores that decide the walk (the first C + 1 of each category up to one item past its end) are
-    separated by more than 2e-5 |score| (the ids are then exact)."""
-    B, N = S.shape
-    ids = np.full((B, K), -1, np.int64)
-    sc = np.full((B, K), -np.inf)
-    margin = np.zeros(B, bool)
-    for b in range(B):
-        s = S[b].copy()
-        if allowed[b] is not None:
-            s[~np.isin(cat, np.asarray(sorted(allowed[b]), np.int64))] = -np.inf
-        s[np.array(sorted(excluded[b]), np.int64)] = -np.inf
-        order = np.lexsort((np.arange(N), -s))
-        order = order[np.isfinite(s[order])]
-        used, n, decide = {}, 0, []
-        for j in order:
-            g = int(cat[j])
-            seen = used.get(g, 0)
-            used[g] = seen + 1
-            if seen <= C:
-                decide.append(s[j])
-            if n == K:
-                break
-            if seen < C:
-                ids[b, n], sc[b, n] = j, s[j]
-                n += 1
-        head = np.array(decide)
-        margin[b] = len(head) < 2 or bool((np.abs(np.diff(head)) > 2e-5 * np.abs(head).max()).all())
-    return ids, sc, margin
-
-
-def check_capped(ids, sc, S, K, C, cat, allowed, excluded):
-    r_ids, r_sc, margin = capped_ref(S, K, C, cat, allowed, excluded)
-    own_order_ok(ids, sc)
-    assert ((ids >= 0) == (r_ids >= 0)).all(), "padding where the reference has no eligible item"
-    valid = r_ids >= 0
-    np.testing.assert_allclose(sc[valid], r_sc[valid], rtol=1e-4, atol=1e-5)
-    assert (ids[margin] == r_ids[margin]).all(), "ids exact on margin-checked rows"
-    for b in range(len(ids)):
-        got = ids[b][ids[b] >= 0]
-        assert not (set(got.tolist()) & excluded[b])
-        if allowed[b] is not None:
-            assert set(cat[got].tolist()) <= allowed[b]
-        assert np.bincount(cat[got]).max(initial=0) <= C, "at most C per category"
-        np.testing.assert_allclose(S[b, got], r_sc[b, :len(got)], rtol=1e-4, atol=1e-5)
-    return margin
+from recommend_ref import GLOBO_N, check_topk, excluded_sets, make_lists, oracle_scores, own_order_ok  # noqa: E402
+from test_gpu_parity import batch_for, build  # noqa: E402
 
 
 def make_codes(rs, N, G, K):
@@ -131,7 +72,7 @@ def test_category_matches_fp64_reference(B, N, G, K, C, kind):
         torch.cuda.synchronize()
         assert torch.equal(ids, ids2) and torch.equal(sc, sc2), "a second run must be bit-identical"
         ids_h, sc_h = ids.cpu().numpy(), sc.cpu().numpy()
-        margin = check_capped(ids_h, sc_h, S, K, C, cat, sets_, ex)
+        margin = check_topk(ids_h, sc_h, S, K, ex, C, cat, sets_)
         if K <= 100:
             assert margin.mean() > 0.5, "fixture must be mostly margin-checked"
         if allowed is not None:
@@ -332,7 +273,7 @@ def test_few_categories_small_cap_scan_each_category_to_its_own_bound():
     for C in (1, 2):
         ids, sc = [x.clone() for x in model.recommend(bt, K, exclude_clicked=True, max_per_category=C)]
         torch.cuda.synchronize()
-        margin = check_capped(ids.cpu().numpy(), sc.cpu().numpy(), S, K, C, cat, [None] * B, ex)
+        margin = check_topk(ids.cpu().numpy(), sc.cpu().numpy(), S, K, ex, C, cat)
         assert margin.mean() > 0.5
         assert (ids.cpu().numpy()[:, G * C:] == -1).all() and (ids.cpu().numpy()[:, :G * C] >= 0).all()
         assert model.rec_rescored[:B].float().mean().item() < N / 10, "each category to its own bound, not all of it"
@@ -358,7 +299,7 @@ def test_capped_select_counts_every_chunk_when_the_list_is_not_enough(N):
     ids, sc = model.recommend(bt, K, max_per_category=C)
     torch.cuda.synchronize()
     S = oracle_scores(model, content, mwdhm, batch)
-    check_capped(ids.cpu().numpy(), sc.cpu().numpy(), S, K, C, cat, [None] * B, [set() for _ in range(B)])
+    check_topk(ids.cpu().numpy(), sc.cpu().numpy(), S, K, [set() for _ in range(B)], C, cat)
 
 
 def test_capped_select_with_more_tied_chunks_than_its_list():
@@ -397,4 +338,4 @@ def test_capped_select_with_more_tied_chunks_than_its_list():
                 break
     assert ids[0].tolist() == want and (sc[0] == sc[0, 0]).all()
     S = oracle_scores(model, cont, mw, batch)
-    check_capped(ids, sc, S, K, C, cat, [None] * B, [set() for _ in range(B)])
+    check_topk(ids, sc, S, K, [set() for _ in range(B)], C, cat)

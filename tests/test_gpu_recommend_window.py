@@ -11,18 +11,10 @@ import torch
 
 pytestmark = pytest.mark.gpu
 
-from test_gpu_parity import batch_for, build, oracle_inputs  # noqa: E402
-from test_gpu_recommend import check_against_reference, own_order_ok  # noqa: E402
-from oracle import tcar_oracle as O  # noqa: E402
+from recommend_ref import GLOBO_N, check_topk, excluded_sets, make_lists, oracle_scores, own_order_ok  # noqa: E402
+from test_gpu_parity import batch_for, build  # noqa: E402
 
-GLOBO_N = 364047
 I32_MIN, I32_MAX = -2 ** 31, 2 ** 31 - 1
-
-
-def oracle_scores(model, content, mwdhm, batch):
-    params, c64, m64 = oracle_inputs(model, content, mwdhm)
-    with torch.no_grad():
-        return O.forward(params, c64, m64, batch)["softmax_input"].numpy()
 
 
 # ------------------------------------------------------------------------------------------------ the windowed GEMM
@@ -138,7 +130,6 @@ def in_window(times, lo, hi):
                                           (10, GLOBO_N, 256, 3, "clicked")])
 def test_window_matches_fp64_reference(B, N, K, T, kind):
     from tcar_b200 import _native as nv
-    from test_gpu_recommend import excluded_sets, make_lists
     model, content, mwdhm, _ = build(N, emb_scale=20.0)
     bt, batch = batch_for(model, N, B, T, 0, mwdhm, seed=B + K + 1)
     rs = np.random.RandomState(K + 5)
@@ -161,7 +152,7 @@ def test_window_matches_fp64_reference(B, N, K, T, kind):
     S = np.where(in_window(times, lo, hi), oracle_scores(model, content, mwdhm, batch), -np.inf)  # out of window
     ex = excluded_sets(B, off, lst, batch["seq"].numpy() if clicked else None)
     ids_h, sc_h = ids.cpu().numpy(), sc.cpu().numpy()
-    check_against_reference(ids_h, sc_h, S, K, ex)
+    check_topk(ids_h, sc_h, S, K, ex)
     got_t = np.where(ids_h >= 0, times[np.maximum(ids_h, 0)], lo[:, None])
     assert ((got_t >= lo[:, None]) & (got_t <= hi[:, None])).all(), "every returned item is in its window"
     if B >= 5:

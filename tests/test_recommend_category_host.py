@@ -6,6 +6,8 @@ import types
 import numpy as np
 import pytest
 
+from recommend_ref import topk_ref
+
 
 def check_layout(codes, G):
     from tcar_b200.util import category_layout, pad_sources
@@ -63,7 +65,8 @@ def capped_topk(S, K, C, cat, allowed=None, excluded=()):
 
 def test_capped_reference_properties():
     """Capping is decomposable: the capped top-K of A u B is the capped top-K of the two capped lists' union (what the
-    per-CTA lists and their final merge rely on), and C >= K is no cap."""
+    per-CTA lists and their final merge rely on), and C >= K is no cap.  recommend_ref.topk_ref agrees with this
+    brute force."""
     rs = np.random.RandomState(1)
     N, G = 400, 9
     cat = rs.randint(0, G, N)
@@ -82,6 +85,17 @@ def test_capped_reference_properties():
         assert capped_topk(union, K, C, cat, allowed, ex) == [j for j in want], trial
         assert capped_topk(S, K, K, cat) == capped_topk(S, K, 10 ** 9, cat)
         assert all(np.bincount(cat[want], minlength=G).max(initial=0) <= C for _ in [0])
+        # the fp64 reference of the GPU tests: row by row the brute force above, and without a cap or categories the
+        # same ids, scores and margins as with C = K and one category
+        rows = np.stack([S, np.round(rs.randn(N), 1), np.round(rs.randn(N), 3)])
+        r_ex = [ex, set(), set(rs.choice(N, 10).tolist())]
+        r_allowed = [allowed, None, set(rs.choice(G, 3, replace=False).tolist())]
+        r_ids = topk_ref(rows, K, r_ex, C, cat, r_allowed)[0]
+        for row, r_row in zip(range(3), r_ids):
+            assert r_row[r_row >= 0].tolist() == capped_topk(rows[row], K, C, cat, r_allowed[row], r_ex[row]), trial
+        plain = topk_ref(rows, K, r_ex)
+        one_cat = topk_ref(rows, K, r_ex, K, np.zeros(N, np.int64), [None] * 3)
+        assert all(np.array_equal(x, y) for x, y in zip(plain, one_cat)), trial
 
 
 def test_item_category_checks():

@@ -263,7 +263,7 @@ def category_workloads(model, mwdhm, shape, G, info, flush):
                     call = [("tcar_recommend_category", p(wc["cmax"]), p(model.a_ic), p(model.Tq), p(ps.item),
                              p(ps.content), p(ps.mwdhm), p(model.cat_stats), None, None, None, T, B,
                              model._cat_n_pad, K, p(model._cat_perm), p(model._item_cat), p(model._cat_off), G,
-                             p(acsr), p(acsr[B + 1:]) if acsr is not None else None, C, p(model._rec_cat_ws), p(ids),
+                             p(acsr), p(acsr[B + 1:]) if acsr is not None else None, C, p(model._rec_ws), p(ids),
                              p(sc), p(model.rec_rescored))]
                     names = ["recommend_category_select_kernel", "recommend_category_scan_kernel"]
                     sel_c, scan_c = profiled(call, names, flush)
