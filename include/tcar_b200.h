@@ -156,6 +156,20 @@ int tcar_score_fwd_tiles(int n_pad);
 int tcar_score_fwd_window(const void* q_bf16, const void* iext_bf16, const float* c_ref, float* rowsum_part,
                           float* chunkmax, float* tilemax, const int32_t* item_time, const int32_t* win_lo,
                           const int32_t* win_hi, int n_rows, int n_items, int n_pad, void* stream);
+/* Eval mode with a freshness decay per session row (DESIGN §4.10): chunkmax / tilemax as mode 1, but of the decayed
+ * score r = s - p instead of s, with
+ *   age = min(max(t_ref[b] - item_time[n], 0), TCAR_DECAY_MAX_AGE)   (exact, then exact in fp32)
+ *   p   = rate[b] * age                                              (one fp32 multiply)
+ *   r   = s - p                                                      (one fp32 subtract)
+ * (item_time / t_ref int32 in one clock unit, rate[b] >= 0 and finite in score units per clock unit; items published
+ * after t_ref[b] get age 0).  Items >= n_items, and with win_lo / win_hi (both given, or both NULL for no window)
+ * items outside [win_lo[b], win_hi[b]], count as -inf as in tcar_score_fwd_window.  No softmax partial sums: only the
+ * maxima are written.  item_time holds n_pad entries.  Always the CTA-pair kernel (score_fwd_pair_kernel<3>); tilemax
+ * is nullable.  The inputs of tcar_recommend_decay. */
+#define TCAR_DECAY_MAX_AGE 8388607   /* 2^23 - 1: ages saturate here (about 16 years in minutes) */
+int tcar_score_fwd_decay(const void* q_bf16, const void* iext_bf16, float* chunkmax, float* tilemax,
+                         const int32_t* item_time, const int32_t* t_ref, const float* rate, const int32_t* win_lo,
+                         const int32_t* win_hi, int n_rows, int n_items, int n_pad, void* stream);
 
 /* (4a) softmax cross-entropy from the partial sums (model_combine.py:145): sumexp[b] = sum_tiles part,
  *      ce[b] = log(sumexp[b]) (because c_ref is the label score). Fixed summation order. */
@@ -585,6 +599,17 @@ int tcar_recommend_window(const float* chunkmax, const float* tilemax, const flo
                           const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B, int N,
                           int n_pad, int K, void* workspace, int32_t* ids, float* scores, int32_t* rescored,
                           const int32_t* item_time, const int32_t* win_lo, const int32_t* win_hi, void* stream);
+/* The same ranked by the decayed score r = s - rate[b] * age of tcar_score_fwd_decay: the exact top-K, by (r desc,
+ * id asc), of the non-excluded items (and with win_lo / win_hi, both given or both NULL, of the in-window ones);
+ * scores holds r, from the exact fp32 score s of tcar_recommend and the same p as the GEMM epilogue.  chunkmax /
+ * tilemax must come from tcar_score_fwd_decay with the same item_time / t_ref / rate / window.  Padding and rescored
+ * as tcar_recommend_window.  Same workspace, limits and launches as tcar_recommend. */
+int tcar_recommend_decay(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
+                         const float* item, const float* content, const int32_t* mwdhm, const float* cat_stats,
+                         const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B, int N,
+                         int n_pad, int K, void* workspace, int32_t* ids, float* scores, int32_t* rescored,
+                         const int32_t* item_time, const int32_t* t_ref, const float* rate, const int32_t* win_lo,
+                         const int32_t* win_hi, void* stream);
 /* The same with at most C items of one category and a per-session set of allowed categories: the exact top-K, by
  * (score desc, id asc), of the non-excluded items of the allowed categories, in which an item that has C better items
  * of its category in the list is left out (C >= K: no cap).  G <= TCAR_RECOMMEND_MAXG categories, item_cat [N] the

@@ -25,6 +25,7 @@ RERANK_MAXL = 2048     # TCAR_RERANK_MAXL: longest candidate list of tcar_rerank
 RECOMMEND_MAXK = 256   # TCAR_RECOMMEND_MAXK: largest K of tcar_recommend
 RECOMMEND_MAXX = 1024  # TCAR_RECOMMEND_MAXX: exclusion entries per session of tcar_recommend, clicks included
 RECOMMEND_MAXG = 1024  # TCAR_RECOMMEND_MAXG: most categories of tcar_recommend_category
+DECAY_MAX_AGE = 2 ** 23 - 1  # TCAR_DECAY_MAX_AGE: ages of the freshness decay saturate here (clock units)
 
 _P, _I, _F, _LL = C.c_void_p, C.c_int, C.c_float, C.c_longlong
 
@@ -42,6 +43,7 @@ SIGNATURES = {
     "tcar_score_fwd_guarded": [_P] * 9 + [_I] * 5 + [_P],
     "tcar_score_fwd_tiles": [_I],
     "tcar_score_fwd_window": [_P] * 9 + [_I] * 3 + [_P],
+    "tcar_score_fwd_decay": [_P] * 9 + [_I] * 3 + [_P],
     "tcar_ce_finish": [_P] * 3 + [_I, _I, _P],
     "tcar_ce_finish_guarded": [_P] * 5 + [_I, _I, _I, _P],
     "tcar_neg_loss": [_P] * 9 + [_I, _I, _P],
@@ -108,6 +110,7 @@ SIGNATURES = {
     "tcar_recommend_ws_bytes": [_I],
     "tcar_recommend": [_P] * 11 + [_I] * 5 + [_P] * 4 + [_P],
     "tcar_recommend_window": [_P] * 11 + [_I] * 5 + [_P] * 7 + [_P],
+    "tcar_recommend_decay": [_P] * 11 + [_I] * 5 + [_P] * 9 + [_P],
     "tcar_recommend_category_ws_bytes": [_I],
     "tcar_recommend_category": [_P] * 10 + [_I] * 4 + [_P] * 3 + [_I] + [_P] * 2 + [_I] + [_P] * 4 + [_P],
 }

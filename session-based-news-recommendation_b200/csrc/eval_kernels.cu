@@ -19,6 +19,7 @@
 #include <stdint.h>
 #include "tcar_b200.h"
 #include "launch.cuh"
+#include "decay.cuh"
 
 namespace tcar {
 
@@ -1129,12 +1130,13 @@ __device__ __forceinline__ uint32_t block_kth_key(int n, int k, Get get, int* s_
     return prefix;
 }
 
-__global__ void __launch_bounds__(256)
-recommend_select_kernel(const float* chunkmax, const float* tilemax, const float* __restrict__ a_ic,
-                        const float* __restrict__ Tq, const float* __restrict__ cat_stats,
-                        const int32_t* __restrict__ x_off, int n_clicks, int K, int N, int n_pad,
-                        float* __restrict__ tau) {
-    PDL_ENTER();
+// The select kernels' body: tau[b] = margin(the K'-th largest chunk maximum, eps_b).
+template <class Margin>
+__device__ __forceinline__ void recommend_select(const float* chunkmax, const float* tilemax,
+                                                 const float* __restrict__ a_ic, const float* __restrict__ Tq,
+                                                 const float* __restrict__ cat_stats,
+                                                 const int32_t* __restrict__ x_off, int n_clicks, int K, int N,
+                                                 int n_pad, float* __restrict__ tau, Margin margin) {
     __shared__ float s_aic[XW], s_tq[NB + 1];
     __shared__ float s_red[32];
     __shared__ int s_hist[256], s_misc[2];
@@ -1170,7 +1172,44 @@ recommend_select_kernel(const float* chunkmax, const float* tilemax, const float
         return c < nchunks ? cm[c] : -INFINITY;
     }, s_hist, s_misc);
     const float eps = score_error_bound(s_aic, s_tq, cat_stats, s_red);
-    if (tid == 0) tau[b] = key_value(kk) - 2.f * eps;
+    if (tid == 0) tau[b] = margin(key_value(kk), eps);
+}
+
+__global__ void __launch_bounds__(256)
+recommend_select_kernel(const float* chunkmax, const float* tilemax, const float* __restrict__ a_ic,
+                        const float* __restrict__ Tq, const float* __restrict__ cat_stats,
+                        const int32_t* __restrict__ x_off, int n_clicks, int K, int N, int n_pad,
+                        float* __restrict__ tau) {
+    PDL_ENTER();
+    recommend_select(chunkmax, tilemax, a_ic, Tq, cat_stats, x_off, n_clicks, K, N, n_pad, tau,
+                     [](float v, float eps) { return v - 2.f * eps; });
+}
+
+// With a freshness decay (§4.10) the maxima and the re-scored values are decayed scores r = fl(s - p), p = the same
+// fp32 penalty on both sides, s_gemm the GEMM's fp32 accumulator and s the exact fp32 score:
+//   r_gemm = fl(x), x = s_gemm - p;  r = fl(y), y = s - p;  |x - y| = |s_gemm - s| <= eps_b (score_error_bound)
+//   |fl(z) - z| <= u |z|, u = 2^-24  ->  |r_gemm - r| <= eps_b (1 + u) + c |r_gemm|  and  <= eps_b (1 + u) + c |r|,
+//   c = 2u / (1 - u)  (from |x| <= |r_gemm| / (1 - u) and |y| <= |x| + eps_b, and symmetrically).
+// g(v) = v - eps_b (1 + u) - c |v| is non-decreasing (c < 1).  The K' chunks with the largest maxima hold K' distinct
+// eligible items with r_gemm >= v, so r >= g(r_gemm) >= g(v) for each: the exact K-th best eligible r_K >= g(v).  A
+// member of the exact top-K has r >= r_K >= g(v), so its r_gemm >= g(r) >= g(g(v)) and its chunk is re-scored when
+// tau_b <= g(g(v)).  decay_margin applies g twice with 2^-21 = 8u for c: eps (score_error_bound's value, already
+// 1.0001 eps_b) covers eps_b (1 + u), and the slack of 8u over c covers the fp32 rounding of the two subtractions and
+// additions here.  The multiplies by 2^-21 are exact.  v = -inf gives -inf (never NaN), as without a decay; a v whose
+// margin overflows gives -inf too, a full scan.  With rate = 0 the relative term does not vanish: it widens the band
+// by 2^-20 |v| (a few fp32 ulps of v), which the exact re-scoring absorbs.
+__device__ __forceinline__ float decay_margin(float v, float eps) {
+    const float l = v - (eps + 0x1p-21f * fabsf(v));
+    return l - (eps + 0x1p-21f * fabsf(l));
+}
+
+__global__ void __launch_bounds__(256)
+recommend_decay_select_kernel(const float* chunkmax, const float* tilemax, const float* __restrict__ a_ic,
+                              const float* __restrict__ Tq, const float* __restrict__ cat_stats,
+                              const int32_t* __restrict__ x_off, int n_clicks, int K, int N, int n_pad,
+                              float* __restrict__ tau) {
+    PDL_ENTER();
+    recommend_select(chunkmax, tilemax, a_ic, Tq, cat_stats, x_off, n_clicks, K, N, n_pad, tau, decay_margin);
 }
 
 // number of entries of a sorted list below x
@@ -1258,12 +1297,14 @@ __device__ __forceinline__ int rec_scan_prologue(RecScanSmem& s, const float* __
 
 // Re-scores the chunks a scan queued in s_q[0 .. s.qn) after the barrier this begins with, NCH chunks per batch:
 // item_at(p) is the item at catalog position p (chunk * CH + slot), or -1 to drop it; it and the excluded ids are
-// dropped before any row load.  Each batch is sorted and merged into s.top[cur] by merge(a, c, nc, out) (merge_topk or
+// dropped before any row load.  xform(s, n) is the value item n is ranked by, from its exact score s: s itself, or
+// (§4.10) the decayed score.  Each batch is sorted and merged into s.top[cur] by merge(a, c, nc, out) (merge_topk or
 // merge_topk_capped with K bound), flipping cur; lane 0 of each warp counts its re-scored items in my_cnt.  Empties the
 // queue and ends with a barrier.
-template <class ItemAt, class Merge>
-__device__ __forceinline__ void rescore_queued(RecScanSmem& s, const int* s_q, int nx, ItemAt item_at, Merge merge,
-                                               const float* __restrict__ item, const float* __restrict__ content,
+template <class ItemAt, class Xform, class Merge>
+__device__ __forceinline__ void rescore_queued(RecScanSmem& s, const int* s_q, int nx, ItemAt item_at, Xform xform,
+                                               Merge merge, const float* __restrict__ item,
+                                               const float* __restrict__ content,
                                                const int32_t* __restrict__ mwdhm, int& cur, int& my_cnt) {
     const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
     auto excluded = [&](int n) {
@@ -1294,7 +1335,8 @@ __device__ __forceinline__ void rescore_queued(RecScanSmem& s, const int* s_q, i
             }
 #pragma unroll
             for (int u = 0; u < 4; ++u)
-                sc[u] = exact_score_e(s.aic, s.tq, item, content, mwdhm, nn[u] >= 0 ? nn[u] : 0, lane);
+                sc[u] = xform(exact_score_e(s.aic, s.tq, item, content, mwdhm, nn[u] >= 0 ? nn[u] : 0, lane),
+                              nn[u] >= 0 ? nn[u] : 0);
             if (lane == 0) {
 #pragma unroll
                 for (int u = 0; u < 4; ++u)
@@ -1362,7 +1404,9 @@ __device__ __forceinline__ void finish_splits(RecScanSmem& s, int cur, int my_cn
     }
 }
 
-template <bool WINDOW>
+// DECAY (§4.10): items are ranked by their decayed score (decay.cuh), with the session's t_ref[b] / rate[b]; the
+// chunk and tile maxima are those of tcar_score_fwd_decay, where -inf again means "no eligible item".
+template <bool WINDOW, bool DECAY>
 __global__ void __launch_bounds__(256, 2)
 recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* __restrict__ a_ic,
                       const float* __restrict__ Tq, const float* __restrict__ item, const float* __restrict__ content,
@@ -1370,14 +1414,17 @@ recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* 
                       const int32_t* __restrict__ x_ids, const int32_t* __restrict__ clicks, int n_clicks, int K, int N,
                       int n_pad, int B, char* wspace, int32_t* __restrict__ out_ids, float* __restrict__ out_scores,
                       int32_t* __restrict__ rescored, const int32_t* __restrict__ item_time,
-                      const int32_t* __restrict__ win_lo, const int32_t* __restrict__ win_hi) {
+                      const int32_t* __restrict__ win_lo, const int32_t* __restrict__ win_hi,
+                      const int32_t* __restrict__ t_ref, const float* __restrict__ rate) {
     PDL_ENTER();
+    constexpr bool MASKED = WINDOW || DECAY;
     __shared__ RecScanSmem s;
     __shared__ int s_q[WQ_CAP];
     const int b = blockIdx.x, split = blockIdx.y, tid = threadIdx.x;
     const int nx = rec_scan_prologue(s, a_ic, Tq, x_off, x_ids, clicks, n_clicks);
     if (nx < 0) return;
     const int32_t w_lo = WINDOW ? win_lo[b] : 0, w_hi = WINDOW ? win_hi[b] : 0;
+    const DecayRow drow = decay_row(DECAY ? t_ref[b] : 0, DECAY ? rate[b] : 0.f);
     const int nchunks = (N + CH - 1) / CH, ntiles = (N + 127) / 128;
     const float* cm = chunkmax + (size_t)b * (n_pad / CH);
     const float* tm = tilemax + (size_t)b * (n_pad / 128);
@@ -1393,14 +1440,15 @@ recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* 
         }
         return n;
     };
+    auto xform = [&](float sc, int n) { return DECAY ? decayed(sc, drow, item_time[n]) : sc; };
     auto merge = [&](const unsigned long long* a, const unsigned long long* c, int nc, unsigned long long* out) {
         merge_topk(a, K, c, nc, out);
     };
     int cur = 0, my_cnt = 0;
     for (int t0 = t_lo; t0 < t_hi; t0 += 256) {
         const int tile = t0 + tid;
-        // WINDOW: a chunk (tile) whose masked maximum is -inf holds no in-window item -- skipped even when bound = -inf
-        if (tile < t_hi && tm[tile] >= bound && (!WINDOW || tm[tile] > -INFINITY)) {
+        // MASKED: a chunk (tile) whose masked maximum is -inf holds no eligible item -- skipped even when bound = -inf
+        if (tile < t_hi && tm[tile] >= bound && (!MASKED || tm[tile] > -INFINITY)) {
             float4 v[TILE_CH / 4];
 #pragma unroll
             for (int c = 0; c < TILE_CH / 4; ++c) v[c] = reinterpret_cast<const float4*>(cm + (size_t)tile * TILE_CH)[c];
@@ -1408,10 +1456,10 @@ recommend_scan_kernel(const float* chunkmax, const float* tilemax, const float* 
             for (int c = 0; c < TILE_CH; ++c) {
                 const int chunk = tile * TILE_CH + c;
                 const float cv = c % 4 == 0 ? v[c / 4].x : c % 4 == 1 ? v[c / 4].y : c % 4 == 2 ? v[c / 4].z : v[c / 4].w;
-                if (chunk < nchunks && cv >= bound && (!WINDOW || cv > -INFINITY)) s_q[atomicAdd(&s.qn, 1)] = chunk;
+                if (chunk < nchunks && cv >= bound && (!MASKED || cv > -INFINITY)) s_q[atomicAdd(&s.qn, 1)] = chunk;
             }
         }
-        rescore_queued(s, s_q, nx, item_at, merge, item, content, mwdhm, cur, my_cnt);
+        rescore_queued(s, s_q, nx, item_at, xform, merge, item, content, mwdhm, cur, my_cnt);
     }
     finish_splits(s, cur, my_cnt, merge, K, B, wspace, out_ids, out_scores, rescored);
 }
@@ -1724,7 +1772,8 @@ recommend_category_scan_kernel(const float* chunkmax, const float* __restrict__ 
             const int chunk = s_cst[a] + i - s_pre[a];
             if (cm[chunk] >= fmaxf(bound, s_ctau[a])) s_q[atomicAdd(&s.qn, 1)] = chunk;
         }
-        rescore_queued(s, s_q, nx, item_at, merge, item, content, mwdhm, cur, my_cnt);
+        rescore_queued(s, s_q, nx, item_at, [](float sc, int) { return sc; }, merge, item, content, mwdhm, cur,
+                       my_cnt);
     }
     finish_splits(s, cur, my_cnt, merge, K, B, wspace, out_ids, out_scores, rescored);
 }
@@ -1949,13 +1998,14 @@ static bool rec_args_ok(const float* chunkmax, const float* a_ic, const float* T
            scores;
 }
 
-// tcar_recommend and tcar_recommend_window: the selection, then the scan
-template <bool WINDOW>
+// tcar_recommend, tcar_recommend_window and tcar_recommend_decay: the selection, then the scan
+template <bool WINDOW, bool DECAY>
 static int launch_recommend(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
                             const float* item, const float* content, const int32_t* mwdhm, const float* cat_stats,
                             const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B, int N,
                             int n_pad, int K, void* workspace, int32_t* ids, float* scores, int32_t* rescored,
-                            const int32_t* item_time, const int32_t* win_lo, const int32_t* win_hi, void* stream) {
+                            const int32_t* item_time, const int32_t* win_lo, const int32_t* win_hi,
+                            const int32_t* t_ref, const float* rate, void* stream) {
     if (!rec_args_ok(chunkmax, a_ic, Tq, item, content, mwdhm, cat_stats, x_off, x_ids, clicks, T, B, n_pad, K,
                      workspace, ids, scores) ||
         N < 1 || n_pad < N || !tilemax)
@@ -1963,12 +2013,13 @@ static int launch_recommend(const float* chunkmax, const float* tilemax, const f
     if (B == 0) return 0;
     const int n_clicks = clicks ? T : 0;
     char* ws = static_cast<char*>(workspace);
-    cudaError_t e = launch_pdl(recommend_select_kernel, dim3(B), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq,
-                               cat_stats, x_off, n_clicks, K, N, n_pad, reinterpret_cast<float*>(ws) + TCAR_QROWS);
+    cudaError_t e = launch_pdl(DECAY ? recommend_decay_select_kernel : recommend_select_kernel, dim3(B), dim3(256), 0,
+                               STREAM, chunkmax, tilemax, a_ic, Tq, cat_stats, x_off, n_clicks, K, N, n_pad,
+                               reinterpret_cast<float*>(ws) + TCAR_QROWS);
     if (e != cudaSuccess) return (int)e;
-    launch_pdl(recommend_scan_kernel<WINDOW>, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq, item,
-               content, mwdhm, x_off, x_ids, clicks, n_clicks, K, N, n_pad, B, ws, ids, scores, rescored, item_time,
-               win_lo, win_hi);
+    launch_pdl(recommend_scan_kernel<WINDOW, DECAY>, dim3(B, WSPLIT), dim3(256), 0, STREAM, chunkmax, tilemax, a_ic, Tq,
+               item, content, mwdhm, x_off, x_ids, clicks, n_clicks, K, N, n_pad, B, ws, ids, scores, rescored,
+               item_time, win_lo, win_hi, t_ref, rate);
     return (int)cudaGetLastError();
 }
 
@@ -1977,9 +2028,9 @@ extern "C" int tcar_recommend(const float* chunkmax, const float* tilemax, const
                               const int32_t* x_off, const int32_t* x_ids, const int32_t* clicks, int T, int B, int N,
                               int n_pad, int K, void* workspace, int32_t* ids, float* scores, int32_t* rescored,
                               void* stream) {
-    return launch_recommend<false>(chunkmax, tilemax, a_ic, Tq, item, content, mwdhm, cat_stats, x_off, x_ids, clicks,
-                                   T, B, N, n_pad, K, workspace, ids, scores, rescored, nullptr, nullptr, nullptr,
-                                   stream);
+    return launch_recommend<false, false>(chunkmax, tilemax, a_ic, Tq, item, content, mwdhm, cat_stats, x_off, x_ids,
+                                          clicks, T, B, N, n_pad, K, workspace, ids, scores, rescored, nullptr, nullptr,
+                                          nullptr, nullptr, nullptr, stream);
 }
 
 extern "C" int tcar_recommend_window(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
@@ -1989,9 +2040,22 @@ extern "C" int tcar_recommend_window(const float* chunkmax, const float* tilemax
                                      int32_t* ids, float* scores, int32_t* rescored, const int32_t* item_time,
                                      const int32_t* win_lo, const int32_t* win_hi, void* stream) {
     if (!item_time || !win_lo || !win_hi) return TCAR_ERR_ARG;
-    return launch_recommend<true>(chunkmax, tilemax, a_ic, Tq, item, content, mwdhm, cat_stats, x_off, x_ids, clicks,
-                                  T, B, N, n_pad, K, workspace, ids, scores, rescored, item_time, win_lo, win_hi,
-                                  stream);
+    return launch_recommend<true, false>(chunkmax, tilemax, a_ic, Tq, item, content, mwdhm, cat_stats, x_off, x_ids,
+                                         clicks, T, B, N, n_pad, K, workspace, ids, scores, rescored, item_time, win_lo,
+                                         win_hi, nullptr, nullptr, stream);
+}
+
+extern "C" int tcar_recommend_decay(const float* chunkmax, const float* tilemax, const float* a_ic, const float* Tq,
+                                    const float* item, const float* content, const int32_t* mwdhm,
+                                    const float* cat_stats, const int32_t* x_off, const int32_t* x_ids,
+                                    const int32_t* clicks, int T, int B, int N, int n_pad, int K, void* workspace,
+                                    int32_t* ids, float* scores, int32_t* rescored, const int32_t* item_time,
+                                    const int32_t* t_ref, const float* rate, const int32_t* win_lo,
+                                    const int32_t* win_hi, void* stream) {
+    if (!item_time || !t_ref || !rate || !win_lo != !win_hi) return TCAR_ERR_ARG;
+    auto run = win_lo ? launch_recommend<true, true> : launch_recommend<false, true>;
+    return run(chunkmax, tilemax, a_ic, Tq, item, content, mwdhm, cat_stats, x_off, x_ids, clicks, T, B, N, n_pad, K,
+               workspace, ids, scores, rescored, item_time, win_lo, win_hi, t_ref, rate, stream);
 }
 
 // tcar_recommend's workspace, then the per-category thresholds [B][TCAR_RECOMMEND_MAXG]

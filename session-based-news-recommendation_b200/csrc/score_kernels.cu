@@ -23,6 +23,7 @@
 #include "sm100_ptx.cuh"
 #include "tcar_b200.h"
 #include "launch.cuh"
+#include "decay.cuh"
 
 namespace tcar {
 
@@ -58,11 +59,15 @@ struct FwdParams {
     int n_rows;             // valid sessions B
     int e_pitch;            // Npad
     int groups;             // number of session groups (ceil(ceil(B/128)/CL))
-    int mode;               // 0 = train, 1 = eval, 2 = eval with a publish-time window per row (pair kernel only)
+    int mode;               // 0 = train, 1 = eval, 2 = eval with a publish-time window per row, 3 = eval with a
+                            // freshness decay per row (2 and 3: pair kernel only)
     int prefetch;           // pair kernel: L2 prefetch distance of the streamed item operand in stages (0 = off)
     const int32_t* item_time;   // MODE 2: [e_pitch] time of every item
     const int32_t* win_lo;      // MODE 2: [512] window of every row: item n is in row b's window when
     const int32_t* win_hi;      //         win_lo[b] <= item_time[n] <= win_hi[b]; the others count as -inf
+                                // MODE 3: item_time as MODE 2, win_lo / win_hi both null (no window) or as MODE 2
+    const int32_t* t_ref;       // MODE 3: [512] request time of every row
+    const float* rate;          // MODE 3: [512] decay rate of every row (decay.cuh)
 };
 
 // exponent shift of one session row in log2 units: the label score, plus -- in pass 2 of the overflow guard -- the
@@ -371,6 +376,46 @@ __device__ __forceinline__ void fwd_epilogue_chunk(const uint32_t (&v)[32], cons
         fwd_epilogue_chunk_t<MODE, false>(v, p, cshift, row_ok, store_ok, row, nb, psum, tmax, amax, wlo, wspan, wempty);
 }
 
+// MODE 3 (eval with a freshness decay, DESIGN §4.10): the chunk maxima (and the running tile maximum) of the decayed
+// scores r = decayed(s, d, t) of one row's 32 items nb .. nb+31; items >= N and items outside the row's window (wlo /
+// wspan / wempty as MODE 2; wspan = ~0 without a window) count as -inf.  No exp and no partial sums.  t = the 32 item
+// times, loaded by the caller before the tcgen05.wait::ld of these scores (load_times).
+__device__ __forceinline__ void load_times(const FwdParams& p, int nb, int4 (&t)[8]) {
+    const int4* tp = reinterpret_cast<const int4*>(p.item_time + nb);
+#pragma unroll
+    for (int g = 0; g < 8; ++g) t[g] = __ldg(tp + g);
+}
+
+template <bool TAIL>
+__device__ __forceinline__ void fwd_decay_chunk_t(const uint32_t (&v)[32], const int4 (&t)[8], const FwdParams& p,
+                                                  const DecayRow& d, uint32_t wlo, uint32_t wspan, bool wempty,
+                                                  bool row_ok, uint32_t row, int nb, float& tmax) {
+    float4 m;
+    float* mm = reinterpret_cast<float*>(&m);
+#pragma unroll
+    for (int g = 0; g < 4; ++g) {
+        float mx = -INFINITY;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const int k = g * 8 + j;
+            const int4 tq = t[k / 4];
+            const int32_t tv = k % 4 == 0 ? tq.x : k % 4 == 1 ? tq.y : k % 4 == 2 ? tq.z : tq.w;
+            const bool ok = !wempty && (uint32_t)tv - wlo <= wspan && !(TAIL && nb + k >= p.n_items);
+            mx = ok ? fmaxf(mx, decayed(__uint_as_float(v[k]), d, tv)) : mx;
+        }
+        mm[g] = mx;
+        tmax = fmaxf(tmax, mx);
+    }
+    if (row_ok) *reinterpret_cast<float4*>(p.chunkmax + (size_t)row * (p.e_pitch / 8) + nb / 8) = m;
+}
+
+__device__ __forceinline__ void fwd_decay_chunk(const uint32_t (&v)[32], const int4 (&t)[8], const FwdParams& p,
+                                                const DecayRow& d, uint32_t wlo, uint32_t wspan, bool wempty,
+                                                bool row_ok, bool tail, uint32_t row, int nb, float& tmax) {
+    if (tail) fwd_decay_chunk_t<true>(v, t, p, d, wlo, wspan, wempty, row_ok, row, nb, tmax);
+    else fwd_decay_chunk_t<false>(v, t, p, d, wlo, wspan, wempty, row_ok, row, nb, tmax);
+}
+
 template <int MODE>
 __global__ void __launch_bounds__(P_THREADS, 1)
 score_fwd_pair_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_i,
@@ -481,6 +526,60 @@ score_fwd_pair_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_co
                     if (++stage == P_STAGES) { stage = 0; phase ^= 1; }
                 }
             }
+        }
+    } else if (MODE == 3 && warp >= 4) {
+        // ================= epilogue of the decayed maxima: the TMEM walk of the epilogue below =================
+        const uint32_t e = warp - 4;
+        const uint32_t q = e & 3, h = e >> 2;
+        const uint32_t row = mtile * BM + q * 32 + lane;
+        const bool row_ok = row < (uint32_t)p.n_rows;
+        DecayRow d = decay_row(0, 0.f);
+        uint32_t wlo = 0, wspan = ~0u;
+        bool wempty = false;
+        if (row_ok) {                               // the row's decay and window, loaded once
+            d = decay_row(p.t_ref[row], p.rate[row]);
+            if (p.win_lo) {
+                const int32_t lo = p.win_lo[row], hi = p.win_hi[row];
+                wlo = (uint32_t)lo;
+                wspan = (uint32_t)hi - (uint32_t)lo;
+                wempty = lo > hi;
+            }
+        }
+        const uint32_t acc_empty_l = mapa_u32(acc_empty, 0);
+        for (uint32_t it = 0; it < my_tiles; ++it) {
+            const uint32_t acc = it % P_NACC;
+            const uint32_t acc_phase = (it / P_NACC) & 1;
+            const uint32_t tile = tile0 + it * tile_step;
+            const int n0 = tile * P_BN + h * 128;
+            mbar_wait(&acc_full[acc], acc_phase);
+            tc_fence_after();
+            const uint32_t taddr = tmem_base + ((q * 32) << 16) + acc * P_BN + h * 128;
+            const bool tail = n0 + 128 > p.n_items;
+            float tmax = -INFINITY;
+            uint32_t va[32], vb[32];
+            int4 ta[8], tb[8];
+            // each chunk's item times are requested before the wait for its scores
+            tmem_ld32(taddr, va);
+            load_times(p, n0, ta);
+            tmem_ld_wait();
+            tmem_ld32(taddr + 32, vb);
+            load_times(p, n0 + 32, tb);
+            fwd_decay_chunk(va, ta, p, d, wlo, wspan, wempty, row_ok, tail, row, n0, tmax);
+            tmem_ld_wait();
+            tmem_ld32(taddr + 64, va);
+            load_times(p, n0 + 64, ta);
+            fwd_decay_chunk(vb, tb, p, d, wlo, wspan, wempty, row_ok, tail, row, n0 + 32, tmax);
+            tmem_ld_wait();
+            tmem_ld32(taddr + 96, vb);
+            load_times(p, n0 + 96, tb);
+            fwd_decay_chunk(va, ta, p, d, wlo, wspan, wempty, row_ok, tail, row, n0 + 64, tmax);
+            tmem_ld_wait();
+            // every TMEM read of this accumulator half is in registers -> hand it back to the MMA warp
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive_cluster(acc_empty_l + acc * 8);
+            fwd_decay_chunk(vb, tb, p, d, wlo, wspan, wempty, row_ok, tail, row, n0 + 96, tmax);
+            if (row_ok && p.tilemax) p.tilemax[(size_t)row * (p.e_pitch / 128) + tile * 2 + h] = tmax;
         }
     } else if (warp >= 4) {
         // ================= epilogue: thread <-> session row, warp <-> (TMEM lane quarter, column half) =================
@@ -1608,6 +1707,43 @@ extern "C" int tcar_score_fwd_window(const void* q_bf16, const void* iext_bf16, 
     if (n_pairs < p.groups) n_pairs = p.groups;
     if (n_pairs / p.groups > p.n_tiles) n_pairs = p.n_tiles * p.groups;
     return launch_fwd_pair<2>(mq, mi, p, n_pairs, stream);
+}
+
+// Eval mode with a freshness decay per row (and an optional window): score_fwd_pair_kernel<3>, the same grid as
+// tcar_score_fwd_window
+extern "C" int tcar_score_fwd_decay(const void* q_bf16, const void* iext_bf16, float* chunkmax, float* tilemax,
+                                    const int32_t* item_time, const int32_t* t_ref, const float* rate,
+                                    const int32_t* win_lo, const int32_t* win_hi, int n_rows, int n_items, int n_pad,
+                                    void* stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    if (n_rows < 1 || n_rows > QROWS || n_items < 1 || n_pad % 256 != 0 || n_items > n_pad || !q_bf16 || !iext_bf16 ||
+        !chunkmax || !item_time || !t_ref || !rate || !win_lo != !win_hi)
+        return TCAR_ERR_ARG;
+    CUtensorMap mq, mi;
+    int rc = make_map_bf16(&mq, q_bf16, QROWS, KEXT, KEXT, BK, BM);
+    if (rc) return rc;
+    rc = make_map_bf16(&mi, iext_bf16, n_pad, KEXT, KEXT, BK, P_HALF);
+    if (rc) return rc;
+    FwdParams p = {};
+    p.chunkmax = chunkmax;
+    p.tilemax = tilemax;
+    p.n_items = n_items;
+    p.n_tiles = n_pad / P_BN;
+    p.n_rows = n_rows;
+    p.e_pitch = n_pad;
+    const int mtiles = (n_rows + BM - 1) / BM;
+    p.groups = (mtiles + 1) / 2;
+    p.mode = 3;
+    p.prefetch = PREFETCH_FWD;
+    p.item_time = item_time;
+    p.win_lo = win_lo;
+    p.win_hi = win_hi;
+    p.t_ref = t_ref;
+    p.rate = rate;
+    int n_pairs = ((sm_count() / 2) / p.groups) * p.groups;
+    if (n_pairs < p.groups) n_pairs = p.groups;
+    if (n_pairs / p.groups > p.n_tiles) n_pairs = p.n_tiles * p.groups;
+    return launch_fwd_pair<3>(mq, mi, p, n_pairs, stream);
 }
 
 extern "C" int tcar_score_fwd_tiles(int n_pad) { return n_pad / F_BN; }

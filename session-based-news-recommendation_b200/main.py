@@ -84,6 +84,14 @@ def max_age_hours(text):
     return h
 
 
+def half_life_hours(text):
+    """--recommend_half_life_h: a finite float number of hours > 0."""
+    h = float(text)
+    if not 0 < h < float("inf"):
+        raise argparse.ArgumentTypeError("must be a finite number of hours > 0")
+    return h
+
+
 def max_per_category(text):
     """--recommend_max_per_category: an integer >= 1."""
     c = int(text)
@@ -104,6 +112,11 @@ class _Parser(argparse.ArgumentParser):
                 self.error("--recommend_max_per_category requires --recommend_k")
             if ns.recommend_max_age_h is not None:
                 self.error("--recommend_max_per_category cannot be combined with --recommend_max_age_h")
+        if getattr(ns, "recommend_half_life_h", None) is not None:
+            if ns.recommend_k is None:
+                self.error("--recommend_half_life_h requires --recommend_k")
+            if ns.recommend_max_per_category is not None:
+                self.error("--recommend_half_life_h cannot be combined with --recommend_max_per_category")
         return ns
 
 
@@ -161,6 +174,10 @@ def build_parser():
     # not a reference flag: at most C articles of one category per recommended list (exact capped top-K on the device,
     # Seq2SeqAttNN.recommend_split); also prints the lists' ILD and unexpectedness
     parser.add_argument("--recommend_max_per_category", default=None, type=max_per_category)
+    # not a reference flag: rank by the score minus a freshness penalty that halves an article's recommendation
+    # probability every H hours of age at the session's last input click (exact on the device, recommend(decay=...));
+    # also prints the mean age of the returned articles
+    parser.add_argument("--recommend_half_life_h", default=None, type=half_life_hours)
     parser.add_argument("--inputdata", default="test", type=str)
     parser.add_argument("--threshold_acc", default=0.27, type=float)
     # additions

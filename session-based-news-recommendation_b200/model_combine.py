@@ -20,8 +20,8 @@ from . import parallel
 from .catalog_parallel import CatalogShardedTraining
 from .params import ParamStore, SMALL
 from .sampler import Sampler, pack_batch
-from .util import (category_layout, check_id_lists, check_item_categories, check_item_times, check_windows,
-                   pad_sources)
+from .util import (category_layout, check_decay, check_id_lists, check_item_categories, check_item_times,
+                   check_windows, pad_sources)
 
 H, TH, XW, PW, NB, KEXT, QROWS, TOPK = nv.H, nv.TH, nv.XW, nv.PW, nv.NBINS, nv.KEXT, nv.QROWS, nv.TOPK
 
@@ -1357,7 +1357,7 @@ class Seq2SeqAttNN(CatalogShardedTraining):
 
     # ------------------------------------------------------------------------------------------- top-K recommendation
     def set_item_times(self, times):
-        """One time per item for recommend(window=...): N integers of any integer type, each within int32, in whatever
+        """One time per item for recommend(window=..., decay=...): N integers of any integer type, each within int32, in whatever
         clock unit the windows use (recommend_split: minutes since the epoch).  Checked on the host (ValueError, nothing
         uploaded), then copied once to an int32 [n_pad] device buffer; may be called again at any time, e.g. to
         withdraw an article by giving it a time no window reaches."""
@@ -1365,6 +1365,7 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         if getattr(self, "_item_time", None) is None:
             self._item_time = torch.zeros(self.ps.n_pad, device=self.dev, dtype=torch.int32)
         self._item_time[:self.N].copy_(torch.from_numpy(t))
+        self._item_time_min = int(t.min()) if self.N else 0     # the oldest item: check_decay's largest penalty
 
     def set_item_categories(self, codes, n_categories=None):
         """One category code per item for recommend(max_per_category=..., categories=...): N integers in [0, G),
@@ -1398,7 +1399,7 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             self._iext_cat_version = self.ps.version
 
     def recommend(self, bt, k=20, exclude_off=None, exclude_ids=None, exclude_clicked=False, window=None,
-                  max_per_category=None, categories=None):
+                  max_per_category=None, categories=None, decay=None):
         """The exact top-k of the whole catalog for every session of bt (tcar_recommend), 1 <= k <= nv.RECOMMEND_MAXK,
         ordered by (score desc, id asc).  Scores are the exact fp32 scores of the full-catalog evaluation: with k <= 20
         and no exclusions the result is the prefix of eval_step's top-20, and an item scores bit for bit what eval_step
@@ -1420,10 +1421,19 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         than k of them pads with -1 / -inf.  The mask sits in the scoring GEMM's epilogue (tcar_score_fwd_window,
         tcar_recommend_window), so the selection stays exact however few items a window holds.
 
+        Freshness decay: decay = (t_ref, rate), t_ref a host array of B integers within int32 (the request times, in
+        the clock unit of set_item_times) and rate one number or B numbers, finite and >= 0 (score units per clock
+        unit), ranks session b by r = s - p, p = rate[b] * age, age = min(max(t_ref[b] - t[n], 0), DECAY_MAX_AGE)
+        (util.decay_penalty: age exact in float32, one float32 multiply and one float32 subtract; items published
+        after t_ref get age 0).  The result is the exact top-k by (r desc, id asc) and scores holds r.  A rate whose
+        penalty for the oldest item is not finite in float32 is refused.  The penalty sits in the scoring GEMM's
+        epilogue (tcar_score_fwd_decay, tcar_recommend_decay), so an article just outside the undecayed top-k is still
+        found.  Composes with the exclusions and window.
+
         Categories (after set_item_categories): max_per_category = C >= 1 leaves out an item that has C better items of
         its category in the list (C >= k: no cap); categories = (off, codes) restricts session b to the categories
         codes[off[b]:off[b + 1]] (CSR as the exclusion lists, codes in [0, G), duplicates allowed; an empty list gives
-        -1 / -inf throughout).  Exclusions compose with both; window does not (ValueError).  The result is the exact
+        -1 / -inf throughout).  Exclusions compose with both; window and decay do not (ValueError).  The result is the exact
         capped, filtered top-k in the same format, by the scoring GEMM over iext_cat and tcar_recommend_category."""
         if isinstance(k, (bool, np.bool_)) or not isinstance(k, (int, np.integer)) or not 1 <= k <= nv.RECOMMEND_MAXK:
             raise ValueError(f"k must be an integer in [1, TCAR_RECOMMEND_MAXK = {nv.RECOMMEND_MAXK}], got {k!r}")
@@ -1443,12 +1453,19 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             if getattr(self, "_item_time", None) is None:
                 raise ValueError("window needs item times: call set_item_times first")
             win = check_windows(window, B)
+        dec = None
+        if decay is not None:
+            if getattr(self, "_item_time", None) is None:
+                raise ValueError("decay needs item times: call set_item_times first")
+            dec = check_decay(decay, B, [self._item_time_min])
         by_cat = max_per_category is not None or categories is not None
         if by_cat:
             if getattr(self, "_iext_cat", None) is None:
                 raise ValueError("max_per_category / categories need item categories: call set_item_categories first")
             if window is not None:
                 raise ValueError("window cannot be combined with max_per_category / categories")
+            if decay is not None:
+                raise ValueError("decay cannot be combined with max_per_category / categories")
             C = k
             if max_per_category is not None:
                 if isinstance(max_per_category, (bool, np.bool_)) or not isinstance(max_per_category, (int, np.integer)) \
@@ -1480,8 +1497,16 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         self._ensure_cat_stats()
         # the chunk / tile maxima of one unguarded eval-mode GEMM (its softmax partial sums, which may overflow without
         # the guard, are not read): over ps.iext, with the windows applied in the epilogue, or over iext_cat (N' items
-        # in category order); the windows go up through the pinned ring like the exclusion lists
-        if win is not None:
+        # in category order); the windows and the decay go up through the pinned ring like the exclusion lists.  With a
+        # decay the GEMM writes the maxima of the decayed scores, with its window if there is one.
+        if dec is not None:
+            ws = self._score_buffers(ps.n_pad, False)
+            wv = self._stage_ints(win) if win is not None else None
+            dv = self._stage_ints(dec)
+            wargs = (p(wv), p(wv[B:])) if wv is not None else (None, None)
+            nv.counted_call("tcar_score_fwd_decay", 1, p(self.Q), p(ps.iext), p(ws["cmax"]), p(ws["tmax"]),
+                            p(self._item_time), p(dv), p(dv[B:]), *wargs, B, N, ps.n_pad)
+        elif win is not None:
             ws = self._score_buffers(ps.n_pad, False)
             wv = self._stage_ints(win)
             nv.counted_call("tcar_score_fwd_window", 1, p(self.Q), p(ps.iext), p(self.c_ref), p(ws["part"]),
@@ -1502,6 +1527,9 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             nv.counted_call("tcar_recommend_category", 2, p(ws["cmax"]), *query, self._cat_n_pad, k,
                             p(self._cat_perm), p(self._item_cat), p(self._cat_off), self._cat_G, p(acsr),
                             p(acsr[B + 1:]) if acsr is not None else None, C, *out)
+        elif dec is not None:
+            nv.counted_call("tcar_recommend_decay", 2, p(ws["cmax"]), p(ws["tmax"]), *query, N, ps.n_pad, k, *out,
+                            p(self._item_time), p(dv), p(dv[B:]), *wargs)
         elif win is not None:
             nv.counted_call("tcar_recommend_window", 2, p(ws["cmax"]), p(ws["tmax"]), *query, N, ps.n_pad, k, *out,
                             p(self._item_time), p(wv), p(wv[B:]))
@@ -1530,31 +1558,48 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         gives each its own: every category is padded to whole 8-item chunks in the category-ordered catalog, and one
         padded category per unknown article would blow up its size.  Then the result also holds "ild" and "unexp",
         the reference's intra-list diversity and unexpectedness (getILD / getUnexp, padding dropped) averaged as test()
-        averages them: over the returned lists of at least two items."""
+        averages them: over the returned lists of at least two items.
+
+        args["recommend_half_life_h"] = H > 0 (hours) ranks every session by the decayed score of recommend(decay=...)
+        with t_ref = t_req (util.session_request_times) and rate = ln 2 / (60 H) per minute, so that an article's
+        recommendation probability halves every H hours of age; it composes with recommend_max_age_h and cannot be
+        combined with recommend_max_per_category.  Then the result also holds "mean_age_h": the mean age
+        max(t_req - publish time, 0) of the returned articles in hours (padding dropped)."""
         from .util import (count_outside, diversity_sums, epoch_minutes, label_positions, recommend_line,
-                           session_windows, topk_metrics, topk_sums)
+                           session_request_times, session_windows, topk_metrics, topk_sums)
         k = int(args.get("recommend_k") or 20)
         clicked = bool(args.get("recommend_exclude_clicked"))
         max_age = args.get("recommend_max_age_h")
         windowed = max_age is not None
+        half_life = args.get("recommend_half_life_h")
+        decayed = half_life is not None
         cap = args.get("recommend_max_per_category")
         capped = cap is not None
         if capped:
             if windowed:
                 raise ValueError("recommend_max_per_category cannot be combined with recommend_max_age_h")
+            if decayed:
+                raise ValueError("recommend_max_per_category cannot be combined with recommend_half_life_h")
             self.set_item_categories(self._split_category_codes())
-        if windowed:
-            if not float(max_age) > 0:
-                raise ValueError(f"recommend_max_age_h must be > 0 hours, got {max_age!r}")
+        if windowed and not float(max_age) > 0:
+            raise ValueError(f"recommend_max_age_h must be > 0 hours, got {max_age!r}")
+        if decayed and not (0 < float(half_life) < float("inf")):
+            raise ValueError(f"recommend_half_life_h must be a finite number of hours > 0, got {half_life!r}")
+        if windowed or decayed:
             if args.get("publish_time") is None:
-                raise ValueError("recommend_max_age_h needs every article's publish time in args['publish_time']")
+                raise ValueError("{} needs every article's publish time in args['publish_time']".format(
+                    "recommend_max_age_h" if windowed else "recommend_half_life_h"))
             item_time = epoch_minutes(args["publish_time"])
             self.set_item_times(item_time)
+        if windowed:
             max_age_min = int(round(60 * float(max_age)))
-        print("Recommending the top-{} articles{}{}{}...".format(
+        if decayed:
+            rate = float(np.log(2.0) / (60.0 * float(half_life)))
+        print("Recommending the top-{} articles{}{}{}{}...".format(
             k, " without the clicked ones" if clicked else "",
             " published at most {} h before the request".format(max_age) if windowed else "",
-            ", at most {} per category".format(cap) if capped else ""))
+            ", at most {} per category".format(cap) if capped else "",
+            ", ranked with a freshness half-life of {} h".format(half_life) if decayed else ""))
         self.sync_item_table()
         session_dict_test = test_data[1]
         reverse = self.reverse_item if self.reverse_item is not None else \
@@ -1563,31 +1608,39 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         keys = list(sampler.session_id_batches)
         # this rank's windows up front, so that the producer thread does no dictionary work per batch
         wins = [session_windows(kb, test_data[2], max_age_min) for kb in keys] if windowed else [None] * len(keys)
+        t_reqs = [session_request_times(kb, test_data[2]) for kb in keys] if decayed else [None] * len(keys)
         os.makedirs("saved", exist_ok=True)
         dist_on = parallel.is_distributed(self.world)
         path = "saved/recommend_{}{}.txt".format(args.get("foldnum", 0), "_rank{}".format(self.rank) if dist_on else "")
-        sums = np.zeros(5 if windowed else 7 if capped else 4)
+        # HR / MRR / nDCG / sessions, then label_outside (window), ILD / unexpectedness / lists (cap), and the summed
+        # age in minutes / number of returned articles (decay)
+        sums = np.zeros((5 if windowed else 7 if capped else 4) + (2 if decayed else 0))
 
         def launch(cur, nxt):
-            bt, (kb, win) = cur
+            bt, (kb, win, t_req) = cur
             ids, sc = self.recommend(bt, k, exclude_clicked=clicked, window=win,
-                                     **({"max_per_category": int(cap)} if capped else {}))
-            return kb, win, self.fetch_async(ids), self.fetch_async(sc)
+                                     **({"max_per_category": int(cap)} if capped else {}),
+                                     **({"decay": (t_req, rate)} if decayed else {}))
+            return kb, win, t_req, self.fetch_async(ids), self.fetch_async(sc)
 
-        def consume(kb, win, ids_h, sc_h):
+        def consume(kb, win, t_req, ids_h, sc_h):
             ids, sc = ids_h.get().numpy(), sc_h.get().numpy()
             labels = [session_dict_test[key][-1] - 1 for key in kb]
             sums[:4] += topk_sums(label_positions(ids, labels))
             if windowed:
                 sums[4] += count_outside(item_time[labels], *win)
             if capped:
-                sums[4:] += diversity_sums(ids, [np.asarray(session_dict_test[key][:-1]) - 1 for key in kb],
-                                           self._categories())
+                sums[4:7] += diversity_sums(ids, [np.asarray(session_dict_test[key][:-1]) - 1 for key in kb],
+                                            self._categories())
+            if decayed:
+                got = ids >= 0
+                age = np.maximum(t_req[:, None] - item_time[np.maximum(ids, 0)], 0)
+                sums[-2:] += (age[got].sum(), got.sum())
             f.writelines(recommend_line(key, ids[b], sc[b], reverse) for b, key in enumerate(kb))
 
         with open(path, "w") as f:
             pipelined(zip((self.stage_to_device(packed, B, T, Nn) for packed, B, T, Nn in prefetch_packed(sampler)),
-                          zip(keys, wins)), launch, consume)
+                          zip(keys, wins, t_reqs)), launch, consume)
         total = self._sum_over_ranks(sums)
         m = topk_metrics(total[:4])
         if windowed:
@@ -1595,6 +1648,8 @@ class Seq2SeqAttNN(CatalogShardedTraining):
         if capped:
             n = total[6]
             m["ild"], m["unexp"] = (float(total[4] / n), float(total[5] / n)) if n > 0 else (float("nan"),) * 2
+        if decayed:
+            m["mean_age_h"] = float(total[-2] / total[-1] / 60) if total[-1] > 0 else float("nan")
         self.last_recommend_metrics = m
         self.last_recommend_path = path
         print("Recommend: HR@{k}: {}, MRR@{k}: {}, nDCG@{k}: {} ({} sessions{}, written to {})".format(
@@ -1602,6 +1657,9 @@ class Seq2SeqAttNN(CatalogShardedTraining):
             ", {} labels published outside their window".format(m["label_outside"]) if windowed else "", path, k=k))
         if capped:
             print("Recommend: ILD: {}, unexpectedness: {}".format(m["ild"], m["unexp"]))
+        if decayed:
+            print("Recommend: mean age of the returned articles: {} h (half-life {} h)".format(m["mean_age_h"],
+                                                                                              half_life))
         return m
 
     def _split_category_codes(self):

@@ -7,7 +7,7 @@ import time
 
 import numpy as np
 
-from ._native import CHUNK, RECOMMEND_MAXG
+from ._native import CHUNK, DECAY_MAX_AGE, RECOMMEND_MAXG
 
 
 def cau_metrics(preds, labels, cutoff=20):
@@ -162,11 +162,63 @@ def check_windows(window, B):
     return out
 
 
+def decay_penalty(t_ref, rate, times):
+    """The penalty p = rate * age of the freshness decay (DESIGN §4.10, csrc/decay.cuh) in float32, for session
+    request times t_ref [B], rates [B] and item times [N] -> [B, N]: age = min(max(t_ref - t, 0), DECAY_MAX_AGE),
+    exact in float32, then one float32 multiply.  The decayed score is s - p, one float32 subtract."""
+    age = np.clip(np.asarray(t_ref, np.int64).reshape(-1, 1) - np.asarray(times, np.int64).reshape(1, -1), 0,
+                  DECAY_MAX_AGE).astype(np.float32)
+    return np.asarray(rate, np.float32).reshape(-1, 1) * age
+
+
+def check_decay(decay, B, times):
+    """Validate the freshness decay (t_ref, rate) of B sessions before anything is launched: t_ref holds B integers
+    within int32 (the clock unit of the item times), rate is one number or B numbers, each finite and >= 0 (score
+    units per clock unit), and every session's largest penalty over the catalog (item times `times`, int32 [N]) is
+    finite in float32.  Returns the int32 host array [t_ref | the rates' float32 bits] the kernels read; raises
+    ValueError naming the first bad session."""
+    if not isinstance(decay, (tuple, list)) or len(decay) != 2:
+        raise ValueError("decay must be a pair (t_ref, rate)")
+    t_ref = np.asarray(decay[0]).reshape(-1)
+    if t_ref.size and t_ref.dtype.kind not in "iu":
+        raise ValueError("decay t_ref must hold integers")
+    if t_ref.shape[0] != B:
+        raise ValueError(f"decay t_ref must hold B = {B} values, got {t_ref.shape[0]}")
+    if B and (t_ref.min() < INT32_MIN or t_ref.max() > INT32_MAX):
+        b = int(np.argmax((t_ref < INT32_MIN) | (t_ref > INT32_MAX)))
+        raise ValueError(f"session {b}: decay t_ref {int(t_ref[b])} outside int32")
+    rate = np.asarray(decay[1])
+    if rate.dtype.kind not in "iuf" or rate.ndim > 1 or (rate.ndim == 1 and rate.shape[0] != B):
+        raise ValueError(f"decay rate must be one number or B = {B} numbers")
+    rate = np.broadcast_to(rate.astype(np.float64), (B,))
+    if B and not (np.isfinite(rate) & (rate >= 0)).all():
+        b = int(np.argmax(~(np.isfinite(rate) & (rate >= 0))))
+        raise ValueError(f"session {b}: decay rate {float(rate[b])} is not finite and >= 0")
+    with np.errstate(over="ignore"):                   # an overflow is what the checks below look for
+        r32 = rate.astype(np.float32)
+        worst = decay_penalty(t_ref, r32, [np.asarray(times).min()])[:, 0] if len(times) else np.zeros(B)
+    if B and not np.isfinite(r32).all():
+        b = int(np.argmax(~np.isfinite(r32)))
+        raise ValueError(f"session {b}: decay rate {float(rate[b])} overflows float32")
+    if B and not np.isfinite(worst).all():
+        b = int(np.argmax(~np.isfinite(worst)))
+        raise ValueError(f"session {b}: decay rate {float(rate[b])} gives the penalty {worst[b]} for its oldest "
+                         "item, not finite in float32")
+    out = np.empty(2 * B, dtype=np.int32)
+    out[:B], out[B:] = t_ref, r32.view(np.int32)
+    return out
+
+
+def session_request_times(keys, session_time_dict):
+    """Request times t_req of a batch's sessions (keys in batch order) in epoch minutes: the click_t of the session's
+    last input click (session_time_dict[key][-2], the click the sampler takes the request context from).  int64."""
+    return epoch_minutes([session_time_dict[k][-2]["click_t"] for k in keys])
+
+
 def session_windows(keys, session_time_dict, max_age_min):
     """Publish-time windows of a batch's sessions (keys in batch order) for recommend(window=...): [t_req - max_age_min,
-    t_req] in epoch minutes, t_req = the click_t of the session's last input click (session_time_dict[key][-2], the
-    click the sampler takes the request context from).  Returns int64 arrays (lo, hi)."""
-    hi = epoch_minutes([session_time_dict[k][-2]["click_t"] for k in keys])
+    t_req] in epoch minutes, t_req = session_request_times.  Returns int64 arrays (lo, hi)."""
+    hi = session_request_times(keys, session_time_dict)
     return hi - int(max_age_min), hi
 
 

@@ -5,6 +5,7 @@ with and without the session's own clicks excluded.
     python tools/recommend_probe.py [--shapes globo,mind]
     python tools/recommend_probe.py --window [--shapes globo,mind]
     python tools/recommend_probe.py --category [--shapes globo,mind]
+    python tools/recommend_probe.py --decay [--shapes globo,mind]
 
 recommend_split across ranks is checked by tools/split_check.py.
 
@@ -39,6 +40,16 @@ categories) / tcar_recommend_category), item codes drawn uniformly from G catego
                                              events over 32 batches); ratio = with / without
   rescored_mean / rescored_max               items re-scored exactly per query
   rebuild_us                                 one rebuild of iext_cat from ps.iext (CUDA events, mean of 10)
+
+--decay: the freshness decay (recommend(decay=...) / tcar_score_fwd_decay / tcar_recommend_decay), item times uniform
+over ten days in minutes and every session's t_ref at their end, half-lives of 6, 24 and 48 h, K in {20, 100}, B = 512,
+T = 1, no exclusions.  One JSON line per shape, half-life and K:
+  gemm_mode1_us_cold / gemm_decay_us_cold    score_fwd_pair_kernel<1> / <3> alone (torch.profiler), the L2
+                                             overwritten before each call; gemm_ratio = decay / mode 1
+  recommend_us / recommend_decay_us          Seq2SeqAttNN.recommend without / with the decay per batch (CUDA events
+                                             over 32 batches); ratio = decay / none
+  rescored_mean / rescored_max               items re-scored exactly per query with the decay (rescored_plain_mean:
+                                             without; rescored_ratio = with / without)
 """
 import argparse
 import json
@@ -47,7 +58,7 @@ import numpy as np
 import torch
 
 from probe_common import B, gpu_info, make_model
-from tcar_b200 import _native as nv, synth
+from tcar_b200 import _native as nv, synth, util as nv_util
 
 SHAPES = {"globo": 364047, "mind": 103630}
 
@@ -216,6 +227,47 @@ def events_us(fn, n):
     return t0.elapsed_time(t1) / n * 1e3
 
 
+def decay_workloads(model, mwdhm, shape, info, flush):
+    """--decay: item times uniform over ten days in minutes, every session's t_ref at their end, half-lives of 6, 24
+    and 48 h (rate = ln 2 / (60 H) per minute)."""
+    N, ps, p = model.N, model.ps, nv.ptr
+    rs = np.random.RandomState(5)
+    model.set_item_times(rs.randint(0, 14400, N))
+    bts = []
+    for i in range(4):
+        packed = synth.make_index_batch(N, B, 1, 0, mwdhm, seed=100 + i)
+        bts.append(model.to_device(torch.from_numpy(packed).pin_memory(), B, 1, 0))
+    t_ref = np.full(B, 14400)
+    for hl in (6, 24, 48):
+        rate = np.log(2) / (60 * hl)
+        model.recommend(bts[0], 20)                         # leaves bts[0]'s session vectors in place
+        ws = model._score_buffers(ps.n_pad, False)
+        dv = torch.from_numpy(nv_util.check_decay((t_ref, rate), B, [0])).cuda()
+        calls = (("tcar_score_fwd", p(model.Q), p(ps.iext), p(model.c_ref), None, p(ws["part"]), p(ws["cmax"]),
+                  p(ws["tmax"]), B, N, ps.n_pad, 1, nv.CLUSTER_PAIR),
+                 ("tcar_score_fwd_decay", p(model.Q), p(ps.iext), p(ws["cmax"]), p(ws["tmax"]), p(model._item_time),
+                  p(dv), p(dv[B:]), None, None, B, N, ps.n_pad))
+        g1, g3 = profiled(calls, ("score_fwd_pair_kernel<1>", "score_fwd_pair_kernel<3>"), flush)
+        for K in (20, 100):
+            resc, resc0 = [], []
+            for bt in bts:
+                model.recommend(bt, K)
+                resc0.append(model.rec_rescored[:B].cpu().numpy())
+                model.recommend(bt, K, decay=(t_ref, rate))
+                resc.append(model.rec_rescored[:B].cpu().numpy())
+            resc, resc0 = np.concatenate(resc), np.concatenate(resc0)
+            t_plain = events_us(lambda i: model.recommend(bts[i % 4], K), 32)
+            t_decay = events_us(lambda i: model.recommend(bts[i % 4], K, decay=(t_ref, rate)), 32)
+            res = dict(info, workload=f"{shape} N={N} B={B} T=1 K={K} half_life={hl}h", N=N, B=B, T=1, K=K,
+                       half_life_h=hl, gemm_mode1_us_cold=round(g1, 2), gemm_decay_us_cold=round(g3, 2),
+                       gemm_ratio=round(g3 / g1, 3), recommend_us=round(t_plain, 1),
+                       recommend_decay_us=round(t_decay, 1), ratio=round(t_decay / t_plain, 3),
+                       rescored_mean=round(float(resc.mean()), 1), rescored_max=int(resc.max()),
+                       rescored_plain_mean=round(float(resc0.mean()), 1),
+                       rescored_ratio=round(float(resc.mean() / resc0.mean()), 3))
+            print("recommend_probe_decay " + json.dumps(res), flush=True)
+
+
 def category_workloads(model, mwdhm, shape, G, info, flush):
     N, ps, p = model.N, model.ps, nv.ptr
     rs = np.random.RandomState(G)
@@ -286,6 +338,7 @@ def main():
     ap.add_argument("--shapes", default="globo,mind")
     ap.add_argument("--window", action="store_true", help="publish-time windows (see the module docstring)")
     ap.add_argument("--category", action="store_true", help="caps and allowed categories (see the module docstring)")
+    ap.add_argument("--decay", action="store_true", help="freshness decay (see the module docstring)")
     a = ap.parse_args()
     torch.cuda.set_device(0)
     info = gpu_info()
@@ -295,6 +348,11 @@ def main():
         if a.category:
             for G in ((461,) if shape == "globo" else (17, 264)):
                 category_workloads(model, mwdhm, shape, G, info, flush)
+            del model
+            torch.cuda.empty_cache()
+            continue
+        if a.decay:
+            decay_workloads(model, mwdhm, shape, info, flush)
             del model
             torch.cuda.empty_cache()
             continue

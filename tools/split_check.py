@@ -1,7 +1,7 @@
 """Run under torchrun: the split walkers of Seq2SeqAttNN -- test() (catalog-sharded eval_round, one round per `world`
 batches), test_impressions() and recommend_split() (batch i on rank i mod world; once more with 24 h publish-time
-windows, once more with at most 2 articles per category) -- on one synthetic split at world N equal the same walkers at
-world 1.
+windows, once more with at most 2 articles per category, once more with a 6 h freshness half-life inside 48 h
+windows) -- on one synthetic split at world N equal the same walkers at world 1.
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29513 \\
         tools/split_check.py
@@ -44,8 +44,8 @@ def categories(item_dict):
 
 def run_walkers(model, split, impressions, item_dict):
     """The walkers on the same batches (Sampler shuffles len_dict in place and draws from `random`); recommend_split
-    also with 24 h publish-time windows (written to recommend_1*.txt) and with at most 2 articles per category
-    (recommend_2*.txt)."""
+    also with 24 h publish-time windows (written to recommend_1*.txt), with at most 2 articles per category
+    (recommend_2*.txt) and with a 6 h half-life inside 48 h windows (recommend_3*.txt)."""
     def fresh():
         random.seed(7)
         return (copy.deepcopy(split[0]), *split[1:])
@@ -55,7 +55,11 @@ def run_walkers(model, split, impressions, item_dict):
            "recommend_window": model.recommend_split(None, fresh(), item_dict,
                                                      {"recommend_k": K, "recommend_exclude_clicked": True,
                                                       "recommend_max_age_h": 24.0, "publish_time": publish_times(N),
-                                                      "foldnum": 1})}
+                                                      "foldnum": 1}),
+           "recommend_decay": model.recommend_split(None, fresh(), item_dict,
+                                                    {"recommend_k": K, "recommend_exclude_clicked": True,
+                                                     "recommend_half_life_h": 6.0, "recommend_max_age_h": 48.0,
+                                                     "publish_time": publish_times(N), "foldnum": 3})}
     model.reverse_item = {cnt - 1: art for art, cnt in item_dict.items()}
     model.category_id = categories(item_dict)
     out["recommend_capped"] = model.recommend_split(None, fresh(), item_dict,
@@ -99,6 +103,7 @@ def main():
     lines_n, lines_1 = lines(0)
     win_n, win_1 = lines(1)
     cap_n, cap_1 = lines(2)
+    dec_n, dec_1 = lines(3)
     equal = {"test": close(a["test"], b["test"], exact=("coverage",), rel=("loss",)),
              "impressions": close(a["impressions"], b["impressions"], exact=("sessions", "skipped")),
              "recommend": close(a["recommend"], b["recommend"], exact=("sessions",)),
@@ -109,7 +114,11 @@ def main():
              len(win_1) == b["recommend_window"]["sessions"],
              "recommend_capped": close(a["recommend_capped"], b["recommend_capped"], exact=("sessions",)),
              "recommend_capped_files": sorted(cap_n) == sorted(cap_1) and
-             len(cap_1) == b["recommend_capped"]["sessions"]}
+             len(cap_1) == b["recommend_capped"]["sessions"],
+             "recommend_decay": close(a["recommend_decay"], b["recommend_decay"],
+                                      exact=("sessions", "label_outside")),
+             "recommend_decay_files": sorted(dec_n) == sorted(dec_1) and
+             len(dec_1) == b["recommend_decay"]["sessions"]}
     ok = all(equal.values())
     print(f"rank {rank} split_check " + json.dumps(dict(gpu_info(), world=world, gpus=gpus, backend=dist.get_backend(),
                                                         sessions=SESSIONS, K=K, exclude_clicked=True, world_n=a,
